@@ -4,6 +4,7 @@ kernel's HBM roofline and the reference's CPU path timed beside it.
 
     python bench.py --gpus N --steps K --warmup W            # this repo (one rank per GPU)
     python bench.py --impl reference --gpus N --steps K ...  # reference CPU path (rank 0 only)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's logits to DIR
 
 A step = one forward of the term-quantised ResNet-18 over one synthetic batch of 256 images
 per GPU (BASELINE.json configs[1]; reference setting evaluate_group_size.py:71-74: 9-bit
@@ -523,10 +524,21 @@ def run_b200(args):
             line["other_configs"] = bench_extra.other_configs(dev)
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_reference_images_per_sec(sample_batch=args.cpu_batch, steps=1)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": out})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
     return line
+
+
+def dump_outputs(directory, arrays):
+    """Writes each tensor as DIR/<name>.npy (float32) so that two builds run with the same arguments, and hence the
+    same seeded inputs, can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------
@@ -616,7 +628,14 @@ def main():
     ap.add_argument("--conv-engine", default="auto", choices=["auto", "f16", "i8"],
                     help="how the exact accumulator is obtained per layer (conv_codes.plan_weight): auto = kind::f16 where "
                          "proven from the weights, kind::i8 planes otherwise")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the logits of the last one (the gathered logits of the whole "
+                         "job, float32) to DIR/logits.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path; --impl reference times a CPU sample instead")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     # stdout carries ONE JSON line: anything a library prints to file descriptor 1 meanwhile (NCCL's version banner,
