@@ -264,6 +264,26 @@ int tq_stem_conv7x7s2_pool(const void *x, int x_dtype, void *x2_scratch, const v
                            void *stream);
 
 /*
+ * The stem in two passes that split the 3x3/s2/p1 max-pool by axis, so that only half of the conv map crosses HBM:
+ *   tq_stem_conv7x7s2_rowmax (x_dtype TQ_F32, TQ_BF16 or TQ_F16) / tq_stem_conv7x7s2_u8_rowmax (uint8 images as in
+ *   tq_stem_conv7x7s2_u8) write out = fp32 NHWC [N, H/2, Wp, Cout] (Wp = (W/2 - 1)/2 + 1), the RAW conv sums maxed
+ *   over conv columns 2q-1, 2q, 2q+1 of each conv row (columns outside the map excluded);
+ *   tq_bn_relu_maxpool_encode_rowmax takes that tensor as x [N, H, W, C] (H = conv rows, W = pooled columns,
+ *   C % 4 == 0) and writes out fp32 NHWC [N, (H - 1)/2 + 1, W, C] = relu(fma(max over rows 2p-1, 2p, 2p+1, bn_a,
+ *   bn_b)) and its fp16 codes as tq_bn_relu_maxpool_encode does.
+ * Together: the same values as tq_stem_conv7x7s2_dt followed by tq_bn_relu_maxpool_encode.
+ * CONTRACT: as for tq_stem_conv7x7s2_pool, the max is taken before the affine, so bn_a >= 0: the caller folds
+ * sign(bn_a) into the channel's weights and passes |bn_a| (conv_codes.stem_pool_operands).
+ */
+int tq_stem_conv7x7s2_rowmax(const void *x, int x_dtype, void *x2_scratch, const void *w2, float *out,
+                             int N, int H, int W, int Cout, void *stream);
+int tq_stem_conv7x7s2_u8_rowmax(const void *x_u8, const float *mean3, const float *std3, void *x2_scratch,
+                                const void *w2, float *out, int N, int H, int W, int Cout, void *stream);
+int tq_bn_relu_maxpool_encode_rowmax(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                     void *out_codes, int N, int H, int W, int C, int relu,
+                                     float next_sf, int next_bits, int next_terms, void *stream);
+
+/*
  * Depthwise 3x3 conv (pad 1, stride 1 or 2) on term codes, the memory-bound layer of the depthwise CNNs
  * (BASELINE.json configs[3]; wrapped by the reference with the (16, 1, 16) weight setting, cnn_models/__init__.py:52-65,
  * and run as TR encode -> cuDNN fp32 conv -> BatchNorm -> ReLU6, tr_layer.py:124-126):

@@ -42,6 +42,9 @@ SYMBOLS = {
     "tq_stem_conv7x7s2_dt": (_i, [_p, _i, _p, _p, _p, _i, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2_u8": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2_pool": (_i, [_p, _i, _p, _p, _p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _i, _i, _p]),
+    "tq_stem_conv7x7s2_rowmax": (_i, [_p, _i, _p, _p, _p, _i, _i, _i, _i, _p]),
+    "tq_stem_conv7x7s2_u8_rowmax": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p]),
+    "tq_bn_relu_maxpool_encode_rowmax": (_i, [_p] * 5 + [_i] * 5 + [_f, _i, _i, _p]),
     "tq_selftest_division": (_i, [C.c_uint64, C.c_uint32, _p, _p]),
 }
 

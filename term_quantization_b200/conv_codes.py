@@ -354,18 +354,21 @@ def bn_act_encode(x_nhwc, bn=None, relu=False, want_f32=False, next_quant=None, 
     return out, codes
 
 
-def bn_relu_maxpool_encode(x_nhwc, bn, relu=True, next_quant=None):
+def bn_relu_maxpool_encode(x_nhwc, bn, relu=True, next_quant=None, rowmax=False):
     """maxpool3x3/s2/p1(relu(fma(x, a, b))) on an fp32 [N, H, W, C] tensor, plus the fp16 term
-    codes of the result for the first wrapped conv.  Returns (out [N, Ho, Wo, C], codes or None)."""
+    codes of the result for the first wrapped conv.  Returns (out [N, Ho, Wo, C], codes or None).
+    rowmax=True: x is [N, H, Wo, C], the row maxima stem_conv7x7s2(..., rowmax=True) writes (the horizontal half of the
+    pool already taken, bn from stem_pool_operands); only the vertical window is left (tq_bn_relu_maxpool_encode_rowmax)."""
     if x_nhwc.dtype != torch.float32 or not x_nhwc.is_contiguous() or not x_nhwc.is_cuda:
         raise RuntimeError("bn_relu_maxpool_encode expects a contiguous fp32 CUDA [N, H, W, C] tensor")
     N, H, W, C = x_nhwc.shape
-    Ho, Wo = (H - 1) // 2 + 1, (W - 1) // 2 + 1
+    Ho, Wo = (H - 1) // 2 + 1, (W if rowmax else (W - 1) // 2 + 1)
     out = torch.empty((N, Ho, Wo, C), dtype=torch.float32, device=x_nhwc.device)
     codes = torch.empty((N, Ho, Wo, C), dtype=torch.float16, device=x_nhwc.device) if next_quant else None
     sf, bits, terms = next_quant if next_quant else (1.0, 1, 0)
+    fn = _lib.lib().tq_bn_relu_maxpool_encode_rowmax if rowmax else _lib.lib().tq_bn_relu_maxpool_encode
     with torch.cuda.device(x_nhwc.device):
-        rc = _lib.lib().tq_bn_relu_maxpool_encode(
+        rc = fn(
             x_nhwc.data_ptr(), bn[0].data_ptr(), bn[1].data_ptr(), out.data_ptr(),
             codes.data_ptr() if codes is not None else None, N, H, W, C, int(bool(relu)),
             float(sf), int(bits), int(terms), torch.cuda.current_stream(x_nhwc.device).cuda_stream)
@@ -399,8 +402,16 @@ def pack_stem_weight(w, channel_sign=None):
 _STEM_DTYPES = {torch.float32: _lib.TQ_F32, torch.bfloat16: _lib.TQ_BF16, torch.float16: _lib.TQ_F16}
 
 
-def stem_conv7x7s2(x_nhwc, w2, scratch=None, cout=None):
-    """fp32 / bf16 / fp16 [N, H, W, 3] -> fp32 [N, H/2, W/2, Cout] (7x7 / stride 2 / pad 3, no bias)."""
+def _stem_out_w(W, rowmax):
+    """Columns of the stem conv's output: W/2 conv columns, or the (W/2 - 1) // 2 + 1 row maxima."""
+    return (W // 2 - 1) // 2 + 1 if rowmax else W // 2
+
+
+def stem_conv7x7s2(x_nhwc, w2, scratch=None, cout=None, rowmax=False):
+    """fp32 / bf16 / fp16 [N, H, W, 3] -> fp32 [N, H/2, W/2, Cout] (7x7 / stride 2 / pad 3, no bias).
+    rowmax=True: fp32 [N, H/2, Wp, Cout] (Wp = (W/2 - 1) // 2 + 1), the max of conv columns 2q-1, 2q, 2q+1 of each conv
+    row -- the horizontal half of the stem's 3x3/s2/p1 max-pool (tq_stem_conv7x7s2_rowmax), for
+    bn_relu_maxpool_encode(..., rowmax=True); `w2` then comes from stem_pool_operands (the pool runs before the affine)."""
     if x_nhwc.dtype not in _STEM_DTYPES or not x_nhwc.is_contiguous() or x_nhwc.shape[-1] != 3:
         raise RuntimeError("stem_conv7x7s2 expects a contiguous fp32 / bf16 / fp16 [N, H, W, 3] tensor")
     N, H, W, _ = x_nhwc.shape
@@ -408,18 +419,20 @@ def stem_conv7x7s2(x_nhwc, w2, scratch=None, cout=None):
     need = (2 if x_nhwc.dtype == torch.float32 else 1) * N * (H // 2 + 3) * (W // 2 + 3) * 16
     if scratch is None or scratch.numel() < need:
         scratch = torch.empty(need, dtype=torch.float16, device=x_nhwc.device)
-    out = torch.empty((N, H // 2, W // 2, Cout), dtype=torch.float32, device=x_nhwc.device)
+    out = torch.empty((N, H // 2, _stem_out_w(W, rowmax), Cout), dtype=torch.float32, device=x_nhwc.device)
+    fn = _lib.lib().tq_stem_conv7x7s2_rowmax if rowmax else _lib.lib().tq_stem_conv7x7s2_dt
     with torch.cuda.device(x_nhwc.device):
-        rc = _lib.lib().tq_stem_conv7x7s2_dt(x_nhwc.data_ptr(), _STEM_DTYPES[x_nhwc.dtype], scratch.data_ptr(),
+        rc = fn(x_nhwc.data_ptr(), _STEM_DTYPES[x_nhwc.dtype], scratch.data_ptr(),
                                              w2.data_ptr(), out.data_ptr(), N, H, W, Cout,
                                              torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
     return out, scratch
 
 
-def stem_conv7x7s2_u8(x_u8_nhwc, mean, std, w2, scratch=None, cout=None):
+def stem_conv7x7s2_u8(x_u8_nhwc, mean, std, w2, scratch=None, cout=None, rowmax=False):
     """uint8 [N, H, W, 3] images -> fp32 [N, H/2, W/2, Cout]: ToTensor + Normalize (rounded to bf16, exactly what
-    inference.normalize_u8 produces) folded into the stem conv's fold pass (tq_stem_conv7x7s2_u8)."""
+    inference.normalize_u8 produces) folded into the stem conv's fold pass (tq_stem_conv7x7s2_u8).
+    rowmax: as for stem_conv7x7s2 (tq_stem_conv7x7s2_u8_rowmax)."""
     import ctypes
     if x_u8_nhwc.dtype != torch.uint8 or not x_u8_nhwc.is_contiguous() or not x_u8_nhwc.is_cuda or x_u8_nhwc.shape[-1] != 3:
         raise RuntimeError("stem_conv7x7s2_u8 expects a contiguous uint8 CUDA [N, H, W, 3] tensor")
@@ -428,11 +441,12 @@ def stem_conv7x7s2_u8(x_u8_nhwc, mean, std, w2, scratch=None, cout=None):
     need = N * (H // 2 + 3) * (W // 2 + 3) * 16
     if scratch is None or scratch.numel() < need:
         scratch = torch.empty(need, dtype=torch.float16, device=x_u8_nhwc.device)
-    out = torch.empty((N, H // 2, W // 2, Cout), dtype=torch.float32, device=x_u8_nhwc.device)
+    out = torch.empty((N, H // 2, _stem_out_w(W, rowmax), Cout), dtype=torch.float32, device=x_u8_nhwc.device)
     m = (ctypes.c_float * 3)(*mean)
     s = (ctypes.c_float * 3)(*std)
+    fn = _lib.lib().tq_stem_conv7x7s2_u8_rowmax if rowmax else _lib.lib().tq_stem_conv7x7s2_u8
     with torch.cuda.device(x_u8_nhwc.device):
-        rc = _lib.lib().tq_stem_conv7x7s2_u8(x_u8_nhwc.data_ptr(), ctypes.cast(m, ctypes.c_void_p), ctypes.cast(s, ctypes.c_void_p),
+        rc = fn(x_u8_nhwc.data_ptr(), ctypes.cast(m, ctypes.c_void_p), ctypes.cast(s, ctypes.c_void_p),
                                              scratch.data_ptr(), w2.data_ptr(), out.data_ptr(), N, H, W, Cout,
                                              torch.cuda.current_stream(x_u8_nhwc.device).cuda_stream)
     _lib.check(rc)

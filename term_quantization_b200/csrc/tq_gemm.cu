@@ -1064,6 +1064,50 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                 TR_SINCE(1, tl0);
                 TR_T0(tq0);
                 if constexpr (MODE == 2) {
+                    if (g.pool == 2) {
+                        // ---- horizontal half of the 3x3 / stride 2 / pad 1 max-pool (two-pass stem) ----
+                        // The tile is 4 conv rows x 32 conv columns (31 used, consecutive tiles overlapping by one
+                        // column): warp ew holds conv row ew, lane x its column x.  Output q (lane 2 ql) is the max of
+                        // the RAW conv sums of lanes 2 ql, 2 ql + 1, 2 ql + 2 (conv columns 2q-1, 2q, 2q+1; a column outside
+                        // the conv map is left out), taken with two shuffles per value: no staging of the conv values, so
+                        // the epilogue adds almost nothing to the shared-memory traffic of the MMAs.  The weights carry
+                        // sign(bn_a) (see the pooled mode below), so tq_bn_relu_maxpool_encode_rowmax takes the vertical
+                        // max and applies the affine after it.
+                        const int Q = g.pool_q, ql = lane >> 1, q = tw * Q + ql;
+                        const bool left = q > 0, right = 2 * q + 1 < g.Wo;
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) {
+                            const float c = __shfl_down_sync(0xFFFFFFFFu, t[j], 1);
+                            const float r = __shfl_down_sync(0xFFFFFFFFu, t[j], 2);
+                            const float m = right ? fmaxf(c, r) : c;
+                            t[j] = left ? fmaxf(t[j], m) : m;
+                        }
+                        TR_SINCE(2, tq0);
+                        TR_T0(tq2);
+                        // the row-max staging tile ([4 * Q][32] fp32) is free once this group's previous TMA store has read it
+                        if (store_thread) bulk_wait_read0();
+                        epi_bar_sync(1 + grp);
+                        TR_SINCE(4, tq2);
+                        TR_T0(tq3);
+                        if (!(lane & 1) && ql < Q) {
+                            const int o = ew * Q + ql;
+                            uint8_t *orow = st_f32 + o * 128;
+                            const uint32_t sw = (uint32_t)(o & 7);
+#pragma unroll
+                            for (int j = 0; j < 32; j += 4)
+                                *reinterpret_cast<float4 *>(orow + (((uint32_t)(j >> 2) ^ sw) << 4)) =
+                                    make_float4(t[j], t[j + 1], t[j + 2], t[j + 3]);
+                        }
+                        TR_SINCE(5, tq3);
+                        fence_proxy_async();
+                        epi_bar_sync(1 + grp);
+                        if (store_thread) {
+                            tma_store_4d(&tmC, st_f32, c0, tw * Q, th * g.hbox, n0);
+                            bulk_commit();
+                        }
+                        TR_SINCE(6, tq0);
+                        continue;
+                    }
                     if (g.pool) {
                         // ---- fused BatchNorm + ReLU + 3x3 / stride 2 / pad 1 max-pool + next-layer encode (stem) ----
                         // The tile is the (2P+1) x (2Q+1) box of conv pixels under P x Q pooled pixels.  The RAW conv
@@ -1306,7 +1350,7 @@ static int plan_smem(ConvGeom &g, int block_n)
     // epilogue staging per group: fp32 tile only if an fp32 tile is written or a residual is read, code tile only
     // if codes are written -- what is not needed goes to the stage ring
     g.epi_codes_off = (g.write_f32 || g.residual) ? GM_EPI_F32_BYTES : 0;
-    g.epi_group_bytes = g.epi_codes_off + ((g.write_codes || g.pool) ? GM_EPI_CODE_BYTES : 0);
+    g.epi_group_bytes = g.epi_codes_off + ((g.write_codes || g.pool == 1) ? GM_EPI_CODE_BYTES : 0);
     const int epi_bytes = GM_EPI_GROUPS * g.epi_group_bytes;
     const int fixed = g.ring_off + epi_bytes + (2 << GM_LUT_MAX_BITS) * 2 + 1024 /* barriers */ + 1024 /* align */;
     int stages = (GM_SMEM_BUDGET - fixed) / g.stage_bytes;
@@ -1887,7 +1931,8 @@ stem_prepare_kernel(const Tin *__restrict__ x, __half *__restrict__ x2, int N, i
 constexpr int STEM_U8 = 100;
 
 // pool = 0: out = conv (fp32 [N, H/2, W/2, Cout]).  pool = 1: out = maxpool3x3s2p1(relu?(fma(conv, bn_a, bn_b)))
-// (fp32 [N, Hp, Wp, Cout]) and, if out_codes, its fp16 term codes for the next layer's quantiser.
+// (fp32 [N, Hp, Wp, Cout]) and, if out_codes, its fp16 term codes for the next layer's quantiser.  pool = 2: out = the
+// max of conv columns 2q-1, 2q, 2q+1 of every conv row (fp32 [N, H/2, Wp, Cout]), the horizontal half of the pool.
 static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w2, float *out, void *out_codes,
                      const float *bn_a, const float *bn_b, int relu, int pool, float next_sf, int next_bits,
                      int next_terms, int N, int H, int W, int Cout, void *stream, const float *mean3 = nullptr,
@@ -1940,6 +1985,15 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
     if (!pool) {
         if (!pick_box_halo(g)) return fail(TQ_ERR_UNSUPPORTED, "stem conv: no tile shape");
         g.step_w = g.wbox; g.step_h = g.hbox;
+    } else if (pool == 2) {
+        // row-max tile: 4 conv rows x 32 conv columns (one warp per row, see the epilogue) -> 4 x Q row maxima, Q <= 15
+        Wp = (Wo - 1) / 2 + 1;
+        g.pool = 2;
+        g.pool_q = Wp < 15 ? Wp : 15;
+        g.wbox = 32; g.hbox = Ho < 4 ? Ho : 4; g.nbox = 1;
+        g.step_w = 2 * g.pool_q; g.step_h = g.hbox; g.off_w = -1; g.off_h = 0;
+        g.tiles_w = (Wp + g.pool_q - 1) / g.pool_q; g.tiles_h = (Ho + g.hbox - 1) / g.hbox; g.tiles_n = N;
+        g.m_tiles = g.tiles_w * g.tiles_h * g.tiles_n;
     } else {
         // pooled tile P x Q over the (2P+1) x (2Q+1) conv pixels it needs (<= 128 accumulator rows): fewest tiles
         Hp = (Ho + 2 - 3) / 2 + 1; Wp = (Wo + 2 - 3) / 2 + 1;
@@ -2009,6 +2063,11 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
         cuuint32_t box[4] = {32, (cuuint32_t)g.wbox, (cuuint32_t)g.hbox, (cuuint32_t)g.nbox};
         cuuint32_t one[4] = {1, 1, 1, 1};
         if ((rc = encode_map(enc, &tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, out, 4, odims, box, one, "stem output")) != TQ_OK) return rc;
+    } else if (pool == 2) {
+        cuuint64_t odims[4] = {(cuuint64_t)Cout, (cuuint64_t)Wp, (cuuint64_t)Ho, (cuuint64_t)N};
+        cuuint32_t box[4] = {32, (cuuint32_t)g.pool_q, (cuuint32_t)g.hbox, 1};
+        cuuint32_t one[4] = {1, 1, 1, 1};
+        if ((rc = encode_map(enc, &tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, out, 4, odims, box, one, "stem row maxima")) != TQ_OK) return rc;
     } else {
         cuuint64_t odims[4] = {(cuuint64_t)Cout, (cuuint64_t)Wp, (cuuint64_t)Hp, (cuuint64_t)N};
         cuuint32_t box[4] = {32, (cuuint32_t)g.pool_q, (cuuint32_t)g.pool_p, 1};
@@ -2047,6 +2106,19 @@ extern "C" int tq_stem_conv7x7s2_u8(const void *x_u8, const float *mean3, const 
                                     float *out, int N, int H, int W, int Cout, void *stream)
 {
     return stem_impl(x_u8, STEM_U8, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 0, 1.0f, 1, 0, N, H, W, Cout, stream,
+                     mean3, std3);
+}
+
+extern "C" int tq_stem_conv7x7s2_rowmax(const void *x, int x_dtype, void *x2_scratch, const void *w2, float *out,
+                                        int N, int H, int W, int Cout, void *stream)
+{
+    return stem_impl(x, x_dtype, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 2, 1.0f, 1, 0, N, H, W, Cout, stream);
+}
+
+extern "C" int tq_stem_conv7x7s2_u8_rowmax(const void *x_u8, const float *mean3, const float *std3, void *x2_scratch,
+                                           const void *w2, float *out, int N, int H, int W, int Cout, void *stream)
+{
+    return stem_impl(x_u8, STEM_U8, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 2, 1.0f, 1, 0, N, H, W, Cout, stream,
                      mean3, std3);
 }
 

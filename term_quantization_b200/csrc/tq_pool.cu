@@ -85,16 +85,26 @@ bn_relu_maxpool3x3s2_kernel(const float *__restrict__ x, const float *__restrict
 // PC = 7: 1.2 times) instead of the 2.25 times of the kernel above, whose row overlap between CTAs is served by L2 (8.4 TB/s
 // through L2 for 4.4 TB/s of algorithmic bytes).  A first tiled version with ordinary loads + barriers between the load and
 // the pooling phase was 2x SLOWER than the simple kernel (0.56 vs 0.26 ms): no overlap, little memory parallelism.
-constexpr int PT_PR = 4, PT_PC = 7, PT_CB = 64, PT_IH = 2 * PT_PR + 1, PT_IW = 2 * PT_PC + 1;
-constexpr int PT_STAGE_BYTES = PT_IH * PT_IW * PT_CB * 4;
+// KW: horizontal window (stride 2, pad 1 for KW = 3; stride 1, no padding for KW = 1).  KW = 1 pools the row maxima the
+// stem conv writes (tq_stem_conv7x7s2_rowmax): only the vertical 3 / 2 / 1 window is left, on half the bytes.
+constexpr int PT_PR = 4, PT_CB = 64, PT_IH = 2 * PT_PR + 1;
 constexpr int PT_STAGES = 3;                    // boxes in flight or in use per CTA (3 x 34.6 KB: two CTAs per SM)
-constexpr int PT_THREADS = PT_PR * PT_PC * (PT_CB / 4);   // one (pooled pixel, 4 channels) item per thread and tile: 448
+constexpr int PT_THREADS = PT_PR * 7 * (PT_CB / 4);       // one (pooled pixel, 4 channels) item per thread and tile (KW = 3): 448
+template <int KW> struct PoolTile {
+    static constexpr int SW = KW == 3 ? 2 : 1, PAD = KW / 2;
+    static constexpr int PC = KW == 3 ? 7 : 14;             // pooled columns per tile: a ~34 KB input box either way
+    static constexpr int IW = SW * (PC - 1) + KW;
+    static constexpr int STAGE_BYTES = PT_IH * IW * PT_CB * 4;
+};
 
+template <int KW>
 __global__ void __launch_bounds__(PT_THREADS, 2)
 bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, const float *__restrict__ bn_a,
                                   const float *__restrict__ bn_b, float *__restrict__ out,
                                   __half *__restrict__ codes, PoolParams p)
 {
+    using T = PoolTile<KW>;
+    constexpr int PT_PC = T::PC, PT_IW = T::IW, PT_STAGE_BYTES = T::STAGE_BYTES;
     extern __shared__ __align__(128) uint8_t pool_smem[];
     uint8_t *base = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(pool_smem) + 127) & ~uintptr_t(127));
     __half *lut = reinterpret_cast<__half *>(base + PT_STAGES * PT_STAGE_BYTES);
@@ -113,7 +123,7 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
     }
     __syncthreads();
     const Quant nq = make_quant(p.write_codes ? p.next_sf : 1.0f, (float)((1u << p.next_bits) - 1u));
-    const int cblocks = p.C / PT_CB, tiles_w = (p.Wo + PT_PC - 1) / PT_PC, tiles_h = (p.Ho + PT_PR - 1) / PT_PR;
+    const int cblocks = (p.C + PT_CB - 1) / PT_CB, tiles_w = (p.Wo + PT_PC - 1) / PT_PC, tiles_h = (p.Ho + PT_PR - 1) / PT_PR;
     const int64_t total = (int64_t)p.N * tiles_h * tiles_w * cblocks;
     const int C4 = p.C >> 2;
     constexpr int c4n = PT_CB / 4;
@@ -125,7 +135,7 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)PT_STAGE_BYTES) : "memory");
         asm volatile(
             "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-            ::"r"(s32(base + stage * PT_STAGE_BYTES)), "l"(&tmIn), "r"(bar), "r"(cb * PT_CB), "r"(tw * PT_PC * 2 - 1),
+            ::"r"(s32(base + stage * PT_STAGE_BYTES)), "l"(&tmIn), "r"(bar), "r"(cb * PT_CB), "r"(tw * PT_PC * T::SW - T::PAD),
               "r"(th * PT_PR * 2 - 1), "r"(n) : "memory");
     };
     int stage = 0;
@@ -153,13 +163,13 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
         const int cb = (int)(t % cblocks);
         const int64_t r = t / cblocks;
         const int tw = (int)(r % tiles_w), th = (int)((r / tiles_w) % tiles_h), n = (int)(r / ((int64_t)tiles_w * tiles_h));
-        const int h0 = th * PT_PR * 2 - 1, w0 = tw * PT_PC * 2 - 1;
+        const int h0 = th * PT_PR * 2 - 1, w0 = tw * PT_PC * T::SW - T::PAD;
         const float4 *tile = reinterpret_cast<const float4 *>(base + stage * PT_STAGE_BYTES);
         for (int o = threadIdx.x; o < PT_PR * PT_PC * c4n; o += blockDim.x) {
             const int c4 = o % c4n, pw = (o / c4n) % PT_PC, ph = o / (c4n * PT_PC);
             const int ho = th * PT_PR + ph, wo = tw * PT_PC + pw;
-            if (ho >= p.Ho || wo >= p.Wo) continue;
             const int cg = cb * c4n + c4;
+            if (ho >= p.Ho || wo >= p.Wo || cg >= C4) continue;
             const float4 a = __ldg(reinterpret_cast<const float4 *>(bn_a) + cg);
             const float4 b = __ldg(reinterpret_cast<const float4 *>(bn_b) + cg);
             const float ninf = -INFINITY;
@@ -169,10 +179,10 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
                 const int h = h0 + 2 * ph + dy;
                 if (h < 0 || h >= p.H) continue;
 #pragma unroll
-                for (int dx = 0; dx < 3; ++dx) {
-                    const int w = w0 + 2 * pw + dx;
+                for (int dx = 0; dx < KW; ++dx) {
+                    const int w = w0 + T::SW * pw + dx;
                     if (w < 0 || w >= p.W) continue;
-                    const float4 v = tile[((2 * ph + dy) * PT_IW + 2 * pw + dx) * c4n + c4];
+                    const float4 v = tile[((2 * ph + dy) * PT_IW + T::SW * pw + dx) * c4n + c4];
                     m.x = fmaxf(m.x, __fmaf_rn(v.x, a.x, b.x));
                     m.y = fmaxf(m.y, __fmaf_rn(v.y, a.y, b.y));
                     m.z = fmaxf(m.z, __fmaf_rn(v.z, a.z, b.z));
@@ -203,18 +213,20 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
 
 using namespace tq;
 
-extern "C" int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, const float *bn_b, float *out,
-                                         void *out_codes, int N, int H, int W, int C, int relu,
-                                         float next_sf, int next_bits, int next_terms, void *stream)
+namespace {
+
+// the checks and parameters both entry points share; Ho = pooled rows, Wo = pooled columns
+int pool_params(PoolParams &p, const float *x, const float *bn_a, const float *bn_b, float *out, void *out_codes, int N,
+                int H, int W, int C, int Wo, int relu, float next_sf, int next_bits, int next_terms)
 {
     if (!x || !bn_a || !bn_b || !out) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1 || C < 4 || C % 4) return fail(TQ_ERR_INVALID, "bad shape (C must be a multiple of 4)");
     if ((((uintptr_t)x | (uintptr_t)bn_a | (uintptr_t)bn_b | (uintptr_t)out | (uintptr_t)out_codes) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
-    PoolParams p{};
+    p = PoolParams{};
     p.N = N; p.H = H; p.W = W; p.C = C;
     p.Ho = (H + 2 - 3) / 2 + 1;
-    p.Wo = (W + 2 - 3) / 2 + 1;
+    p.Wo = Wo;
     p.relu = relu ? 1 : 0;
     p.write_codes = out_codes ? 1 : 0;
     p.next_sf = out_codes ? next_sf : 1.0f;
@@ -226,37 +238,56 @@ extern "C" int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, cons
         if (next_bits < 1 || next_bits > 11 || next_terms < 0) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..11 bits");
     }
     p.next_fastdiv = (p.next_sf >= 9.313225746154785e-10f && p.next_sf <= 1073741824.0f) ? 1 : 0;
+    return TQ_OK;
+}
+
+template <int KW>
+int launch_tiled(EncodeTiledFn enc, const float *x, const float *bn_a, const float *bn_b, float *out, void *out_codes,
+                 const PoolParams &p, void *stream)
+{
+    using T = PoolTile<KW>;
+    const int N = p.N, H = p.H, W = p.W, C = p.C;
+    CUtensorMap tm;
+    cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+    cuuint64_t strides[3] = {(cuuint64_t)C * 4, (cuuint64_t)W * C * 4, (cuuint64_t)H * W * C * 4};
+    cuuint32_t box[4] = {(cuuint32_t)PT_CB, (cuuint32_t)T::IW, (cuuint32_t)PT_IH, 1};
+    cuuint32_t one[4] = {1, 1, 1, 1};
+    CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float *>(x), dims, strides, box, one,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled(pool input) failed: %d", (int)r);
+    const size_t smem_t = PT_STAGES * (size_t)T::STAGE_BYTES + (((size_t)(2u << p.next_bits) * 2 + 15) & ~(size_t)15) + 64 + 128;
+    static bool attr_done[64] = {false};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev >= 0 && dev < 64 && !attr_done[dev]) {
+        if (cudaFuncSetAttribute(bn_relu_maxpool3x3s2_tiled_kernel<KW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024) != cudaSuccess)
+            return check_launch("cudaFuncSetAttribute(bn_relu_maxpool3x3s2_tiled_kernel)");
+        attr_done[dev] = true;
+    }
+    const int64_t tiles = (int64_t)N * ((p.Ho + PT_PR - 1) / PT_PR) * ((p.Wo + T::PC - 1) / T::PC) * ((C + PT_CB - 1) / PT_CB);
+    const int64_t capt = (int64_t)num_sms() * 2;
+    bn_relu_maxpool3x3s2_tiled_kernel<KW><<<(int)(tiles < capt ? tiles : capt), PT_THREADS, smem_t, (cudaStream_t)stream>>>(
+        tm, bn_a, bn_b, out, (__half *)out_codes, p);
+    count_launch();
+    return check_launch("bn_relu_maxpool3x3s2_tiled_kernel");
+}
+
+}  // namespace
+
+extern "C" int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                         void *out_codes, int N, int H, int W, int C, int relu,
+                                         float next_sf, int next_bits, int next_terms, void *stream)
+{
+    PoolParams p;
+    int rc = pool_params(p, x, bn_a, bn_b, out, out_codes, N, H, W, C, (W + 2 - 3) / 2 + 1, relu, next_sf, next_bits, next_terms);
+    if (rc != TQ_OK) return rc;
     // tiled TMA variant for 64-channel blocks on maps of at least one 4 x 14 tile; TQ_POOL_TILED=0 keeps the
     // one-thread-per-output kernel
     static const int tiled_env = getenv("TQ_POOL_TILED") ? atoi(getenv("TQ_POOL_TILED")) : 1;
-    if (tiled_env && C % PT_CB == 0 && p.Ho >= PT_PR && p.Wo >= PT_PC) {
+    if (tiled_env && C % PT_CB == 0 && p.Ho >= PT_PR && p.Wo >= PoolTile<3>::PC) {
         EncodeTiledFn enc = encode_tiled();
-        if (enc) {
-            CUtensorMap tm;
-            cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-            cuuint64_t strides[3] = {(cuuint64_t)C * 4, (cuuint64_t)W * C * 4, (cuuint64_t)H * W * C * 4};
-            cuuint32_t box[4] = {(cuuint32_t)PT_CB, (cuuint32_t)PT_IW, (cuuint32_t)PT_IH, 1};
-            cuuint32_t one[4] = {1, 1, 1, 1};
-            CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float *>(x), dims, strides, box, one,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled(pool input) failed: %d", (int)r);
-            const size_t smem_t = PT_STAGES * (size_t)PT_STAGE_BYTES + (((size_t)(2u << p.next_bits) * 2 + 15) & ~(size_t)15) + 64 + 128;
-            static bool attr_done[64] = {false};
-            int dev = 0;
-            cudaGetDevice(&dev);
-            if (dev >= 0 && dev < 64 && !attr_done[dev]) {
-                if (cudaFuncSetAttribute(bn_relu_maxpool3x3s2_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024) != cudaSuccess)
-                    return check_launch("cudaFuncSetAttribute(bn_relu_maxpool3x3s2_tiled_kernel)");
-                attr_done[dev] = true;
-            }
-            const int64_t tiles = (int64_t)N * ((p.Ho + PT_PR - 1) / PT_PR) * ((p.Wo + PT_PC - 1) / PT_PC) * (C / PT_CB);
-            const int64_t capt = (int64_t)num_sms() * 2;
-            bn_relu_maxpool3x3s2_tiled_kernel<<<(int)(tiles < capt ? tiles : capt), PT_THREADS, smem_t, (cudaStream_t)stream>>>(
-                tm, bn_a, bn_b, out, (__half *)out_codes, p);
-            count_launch();
-            return check_launch("bn_relu_maxpool3x3s2_tiled_kernel");
-        }
+        if (enc) return launch_tiled<3>(enc, x, bn_a, bn_b, out, out_codes, p, stream);
     }
     const int64_t total = (int64_t)N * p.Ho * p.Wo * (C / 4);
     int64_t blocks = (total + 255) / 256;
@@ -267,6 +298,19 @@ extern "C" int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, cons
         x, bn_a, bn_b, out, (__half *)out_codes, p);
     count_launch();
     return check_launch("bn_relu_maxpool3x3s2_kernel");
+}
+
+extern "C" int tq_bn_relu_maxpool_encode_rowmax(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                                void *out_codes, int N, int H, int W, int C, int relu,
+                                                float next_sf, int next_bits, int next_terms, void *stream)
+{
+    // x: [N, H, W, C] row maxima (W = pooled columns); the vertical 3 / 2 / 1 window is all that is left
+    PoolParams p;
+    int rc = pool_params(p, x, bn_a, bn_b, out, out_codes, N, H, W, C, W, relu, next_sf, next_bits, next_terms);
+    if (rc != TQ_OK) return rc;
+    EncodeTiledFn enc = encode_tiled();
+    if (!enc) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
+    return launch_tiled<1>(enc, x, bn_a, bn_b, out, out_codes, p, stream);
 }
 
 

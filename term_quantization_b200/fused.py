@@ -8,8 +8,8 @@ the residual add and the ReLU, and emits the fp16 term codes the *next* conv con
 fp32 activations are materialised only where the graph needs them (block outputs, which feed
 the next residual add).  The stem (first conv, never wrapped: cnn_models/__init__.py:34-36) stays
 unquantised fp32 arithmetic but also runs on the tensor cores (hi/lo fp16 operand pairs, fp32
-accumulate: conv_codes.stem_conv7x7s2; `stem="cudnn"` keeps cuDNN's fp32 conv); its BatchNorm + ReLU +
-max-pool + first encode are one pass.  Global average pool and the classifier stay on PyTorch.
+accumulate: conv_codes.stem_conv7x7s2; `stem="cudnn"` keeps cuDNN's fp32 conv); the row half of its max-pool
+runs in the conv's epilogue, BatchNorm + ReLU + the column half + first encode in one pass.  Global average pool and the classifier stay on PyTorch.
 
 Numerics: every conv's accumulator is the exact int32 accumulator of the integer contraction -- by a static proof
 from the weight codes (kind::f16 MMAs with K-chunk accumulators) or on the kind::i8 plane engine
@@ -82,8 +82,8 @@ class FusedResNet(nn.Module):
 
     def __init__(self, model, stem="tcgen05", engine="auto"):
         """engine: how each conv's exact accumulator is obtained ('auto' | 'f16' | 'i8', conv_codes.plan_weight).
-        stem: 'tcgen05' (stem conv on the tensor cores, then the fused BN+ReLU+max-pool+encode pass: 0.26 + 0.26 ms at
-        batch 256), 'tcgen05_pool' (the whole stem -- conv, BatchNorm, ReLU, max-pool, first encode -- in ONE
+        stem: 'tcgen05' (stem conv on the tensor cores with the horizontal half of the max-pool in its epilogue, then the
+        vertical half + BN + ReLU + first encode in one pass: the conv map crosses HBM at half size), 'tcgen05_pool' (the whole stem -- conv, BatchNorm, ReLU, max-pool, first encode -- in ONE
         tensor-core kernel, pooling in the conv epilogue: the 822 MB conv output never reaches HBM; bit-identical, but its
         pooled epilogue makes it 0.53 ms), or 'cudnn' (cuDNN's fp32 conv)."""
         super().__init__()
@@ -114,9 +114,9 @@ class FusedResNet(nn.Module):
         if (stem != "cudnn" and self.fuse_stem and tuple(c1.weight.shape[1:]) == (3, 7, 7) and c1.stride == (2, 2)
                 and c1.padding == (3, 3) and c1.dilation == (1, 1) and c1.groups == 1 and c1.bias is None
                 and c1.out_channels <= 64):
-            self.stem_w = conv_codes.pack_stem_weight(c1.weight)
-            if stem == "tcgen05_pool":
-                self.stem_w_pool, self.stem_bn_pool = conv_codes.stem_pool_operands(c1.weight, self.stem_bn)
+            # both tensor-core stems pool the raw conv sums and apply the BatchNorm affine after: sign(slope) goes into
+            # the weights, |slope| into stem_bn_pool (conv_codes.stem_pool_operands)
+            self.stem_w, self.stem_bn_pool = conv_codes.stem_pool_operands(c1.weight, self.stem_bn)
         self._stem_scratch = None
 
     @staticmethod
@@ -164,8 +164,8 @@ class FusedResNet(nn.Module):
             # uint8 NHWC batch: normalisation inside the fold pass of the two-launch tensor-core stem (forward_u8 checked)
             q0 = self.blocks[0][0].quant
             y, self._stem_scratch = conv_codes.stem_conv7x7s2_u8(x, u8_norm[0], u8_norm[1], self.stem_w, self._stem_scratch,
-                                                                 cout=m.conv1.out_channels)
-            cur, c0 = conv_codes.bn_relu_maxpool_encode(y, self.stem_bn, relu=True, next_quant=q0)
+                                                                 cout=m.conv1.out_channels, rowmax=True)
+            cur, c0 = conv_codes.bn_relu_maxpool_encode(y, self.stem_bn_pool, relu=True, next_quant=q0, rowmax=True)
             codes = {q0: c0}
         elif self.fuse_stem:
             x = x.contiguous(memory_format=torch.channels_last)
@@ -176,12 +176,13 @@ class FusedResNet(nn.Module):
                 if self.stem_mode == "tcgen05_pool":
                     # conv + bn1 + relu + maxpool + first encode: one tensor-core kernel
                     cur, c0, self._stem_scratch = conv_codes.stem_conv_pool(
-                        x.permute(0, 2, 3, 1), self.stem_w_pool, self.stem_bn_pool, relu=True, next_quant=q0,
+                        x.permute(0, 2, 3, 1), self.stem_w, self.stem_bn_pool, relu=True, next_quant=q0,
                         scratch=self._stem_scratch)
                 else:
-                    y, self._stem_scratch = conv_codes.stem_conv7x7s2(x.permute(0, 2, 3, 1), self.stem_w,
-                                                                      self._stem_scratch, cout=m.conv1.out_channels)
-                    cur, c0 = conv_codes.bn_relu_maxpool_encode(y, self.stem_bn, relu=True, next_quant=q0)
+                    # conv + row max of the pool window, then column max + bn1 + relu + first encode
+                    y, self._stem_scratch = conv_codes.stem_conv7x7s2(x.permute(0, 2, 3, 1), self.stem_w, self._stem_scratch,
+                                                                      cout=m.conv1.out_channels, rowmax=True)
+                    cur, c0 = conv_codes.bn_relu_maxpool_encode(y, self.stem_bn_pool, relu=True, next_quant=q0, rowmax=True)
             else:
                 y = m.conv1(x.float()).permute(0, 2, 3, 1)
                 cur, c0 = conv_codes.bn_relu_maxpool_encode(y, self.stem_bn, relu=True, next_quant=q0)
