@@ -10,7 +10,7 @@ accumulator.  That chain is reproducible on a CPU without any tolerance, which n
     t     = t + bias[co]               RN add                     (if the conv has a bias)
     t     = fmaf(t, bn_a[co], bn_b[co])  one rounding             (if a BatchNorm follows)
     t     = t + residual               RN add                     (block output)
-    t     = max(t, 0)                  (if a ReLU follows)
+    t     = fmaxf(t, 0)                (if a ReLU follows: NaN -> +0, -0 -> +0, see relu_f32())
     codes = tr(t; next_sf, bits, g=1, terms)   oracle.tr: the reference's quantise / HESE / truncate
 
 `run_resnet_chain` chains this over every BasicBlock of a ResNet exactly as fused.FusedResNet does.
@@ -53,9 +53,24 @@ def fused_conv(codes_nhwc, conv, residual=None, relu=False, next_quant=None):
     if residual is not None:
         t = t + np.asarray(residual, dtype=np.float32)
     if relu:
-        t = np.maximum(t, np.float32(0.0))
+        t = relu_f32(t)
     t = np.ascontiguousarray(t, dtype=np.float32)
     return t, (encode(t, next_quant) if next_quant is not None else None)
+
+
+def relu_f32(t):
+    """fmaxf(t, 0) as the fused epilogues compute it (DESIGN.md section 3): an IEEE maxNum drops a NaN operand, so
+    NaN -> +0 (where torch.relu keeps the NaN), and -0 -> +0."""
+    t = np.asarray(t, dtype=np.float32)
+    return np.where(t > 0, t, np.float32(0.0)).astype(np.float32)
+
+
+def maxpool_f32_nan_dropped(x_nhwc, k, stride, pad):
+    """The fused max-pools on an fp32 NHWC map: a running fmaxf from -inf, so a NaN is ignored and a window holding
+    only NaN (or nothing but padding) yields -inf, where torch's max_pool2d propagates the NaN."""
+    x = np.asarray(x_nhwc, dtype=np.float32)
+    x = np.where(np.isnan(x), np.float32(-np.inf), x)
+    return maxpool_nhwc(x, k, stride, pad).astype(np.float32)
 
 
 def run_resnet_chain(blocks, stem_out):
@@ -72,7 +87,7 @@ def run_resnet_chain(blocks, stem_out):
 
 def _act(t, relu):
     if relu:
-        t = np.maximum(t, np.float32(0.0))
+        t = relu_f32(t)
     if relu in ("relu6", 2):
         t = np.minimum(t, np.float32(6.0))
     return t

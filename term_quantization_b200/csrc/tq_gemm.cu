@@ -1954,6 +1954,11 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
     if (Cout < 4 || Cout % 4) return fail(TQ_ERR_UNSUPPORTED, "Cout must be a multiple of 4");
     if ((((uintptr_t)x2_scratch | (uintptr_t)w2 | (uintptr_t)out) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
+    // the pooled stem's quantiser is checked before the fold pass below is launched: a refused call enqueues nothing
+    if (pool == 1 && out_codes) {
+        if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
+        if (next_bits < 1 || next_bits > GM_LUT_MAX_BITS || next_terms < 0) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..%d bits", GM_LUT_MAX_BITS);
+    }
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
     cudaStream_t s = (cudaStream_t)stream;
@@ -2012,10 +2017,6 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
         if (g.pool_p * g.pool_q > 32) return fail(TQ_ERR_UNSUPPORTED, "pooled tile too large");
         g.bn_a = bn_a; g.bn_b = bn_b; g.relu = relu ? 1 : 0;
         g.write_codes = out_codes ? 1 : 0;
-        if (out_codes) {
-            if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
-            if (next_bits < 1 || next_bits > GM_LUT_MAX_BITS || next_terms < 0) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..%d bits", GM_LUT_MAX_BITS);
-        }
     }
     g.hw = g.wbox;
     const int block_n = Cout <= 64 ? 64 : 128;

@@ -176,3 +176,31 @@ def test_booth_encoding_pinned_to_verilog_truth_table():
     z = _enc_golden()
     for q, P, N in zip(z["booth_q"], z["booth_P"], z["booth_N"]):
         assert O.terms(int(q), O.ENC_BOOTH) == (int(P), int(N)), q
+
+
+@pytest.mark.parametrize("bits", range(1, 12))
+def test_fused_encoder_hard_values_hit_every_class(bits):
+    """The hard values of tests/test_fused_encoders_gpu.py really contain, for every (sf, bits) it uses, a tie that
+    rounds up, its lower neighbour rounding down, saturated codes of both signs, NaN (-> 0), zeros of both signs and
+    the smallest subnormal: the GPU comparisons cannot quietly turn trivial."""
+    from test_fused_encoders_gpu import ALL_SFS, hard_values, _oracle_codes
+    for sf in ALL_SFS:
+        x = hard_values(sf, bits)
+        sf32 = np.float32(sf)
+        q = np.array([O.quantize(v, sf32, bits) for v in x])
+        with np.errstate(over="ignore"):
+            r = np.abs(x) / sf32                                       # fp32 IEEE divide, as the kernels compute it
+        tie = np.flatnonzero(np.isfinite(r) & (r == np.floor(r) + np.float32(0.5)) & (r < 2 ** bits - 1))
+        assert tie.size, (sf, bits, "no exact tie below saturation")
+        ups = [i for i in tie if q[i] == int(r[i]) + 1]
+        assert ups, (sf, bits, "no tie rounds up")
+        lows = [i for i in ups if O.quantize(np.nextafter(x[i], np.float32(0)), sf32, bits) == int(r[i])
+                and np.nextafter(x[i], np.float32(0)) in x]
+        assert lows, (sf, bits, "no tie's lower neighbour (in the set) rounds down")
+        codes = _oracle_codes(x, sf, bits, bits)                       # budget not binding: saturation shows
+        sat = int(_oracle_codes(np.array([np.inf], np.float32), sf, bits, bits)[0])
+        assert sat > 0 and (codes == sat).any() and (codes == -sat).any(), (sf, bits, "saturated codes of both signs")
+        nan = np.isnan(x)
+        assert nan.any() and (codes[nan] == 0).all() and (_oracle_codes(x, sf, bits, 0) == 0).all()
+        assert (x == 0).sum() == 2 and np.signbit(x[x == 0]).sum() == 1                  # +0 and -0
+        assert (np.abs(x) == np.float32(2.0 ** -149)).sum() == 2
