@@ -119,17 +119,17 @@ def plan_weight(wgt, act_max, signed_act=False, engine="auto"):
     return WeightPlan("i8", 1, bound, act_max, signed_act, wgt, planes=planes, planes_w=pw, wgt_max=max(wmax, 1))
 
 
-_PLANS = {}
-
-
 def _cached_plan(wgt, act_max, signed_act, engine):
-    key = (wgt.data_ptr(), wgt._version, tuple(wgt.shape), int(act_max), bool(signed_act), engine)
-    plan = _PLANS.get(key)
-    if plan is None or plan.wgt is not wgt:
-        if len(_PLANS) > 256:
-            _PLANS.clear()
-        plan = _PLANS[key] = plan_weight(wgt, act_max, signed_act, engine)
-    return plan
+    """The plan of `wgt` for the raw ops called without plan=.  It is kept on the weight tensor itself, so it lives
+    exactly as long as the weight: a CUDA graph that captured a call keeps the weight alive and with it the int8 planes
+    the i8 engine reads.  An in-place change of the weight (a new _version) replaces the plan."""
+    plans = wgt.__dict__.setdefault("_tq_plans", {})
+    key = (int(act_max), bool(signed_act), engine)
+    stamp = (wgt.data_ptr(), wgt._version, tuple(wgt.shape))
+    hit = plans.get(key)
+    if hit is None or hit[0] != stamp:
+        hit = plans[key] = (stamp, plan_weight(wgt, act_max, signed_act, engine))
+    return hit[1]
 
 
 def _run_conv(act, plan, out, codes, bias, bn, residual, N, H, W, C, Cout, R, S, stride, pad, scale, relu, sf, bits,

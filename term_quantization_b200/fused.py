@@ -117,7 +117,8 @@ class FusedResNet(nn.Module):
             # both tensor-core stems pool the raw conv sums and apply the BatchNorm affine after: sign(slope) goes into
             # the weights, |slope| into stem_bn_pool (conv_codes.stem_pool_operands)
             self.stem_w, self.stem_bn_pool = conv_codes.stem_pool_operands(c1.weight, self.stem_bn)
-        self._stem_scratch = None
+        # (no stem scratch is kept here: each stem call allocates its folded image, so that under CUDA-graph capture it
+        # comes from that graph's private pool, and a later, larger call cannot free memory a captured graph still writes)
 
     @staticmethod
     def _encode(x_nhwc, quant):
@@ -163,8 +164,7 @@ class FusedResNet(nn.Module):
         if u8_norm is not None:
             # uint8 NHWC batch: normalisation inside the fold pass of the two-launch tensor-core stem (forward_u8 checked)
             q0 = self.blocks[0][0].quant
-            y, self._stem_scratch = conv_codes.stem_conv7x7s2_u8(x, u8_norm[0], u8_norm[1], self.stem_w, self._stem_scratch,
-                                                                 cout=m.conv1.out_channels, rowmax=True)
+            y, _ = conv_codes.stem_conv7x7s2_u8(x, u8_norm[0], u8_norm[1], self.stem_w, cout=m.conv1.out_channels, rowmax=True)
             cur, c0 = conv_codes.bn_relu_maxpool_encode(y, self.stem_bn_pool, relu=True, next_quant=q0, rowmax=True)
             codes = {q0: c0}
         elif self.fuse_stem:
@@ -175,13 +175,12 @@ class FusedResNet(nn.Module):
                     and (x.shape[2] // 2) * (x.shape[3] // 2) >= 128:
                 if self.stem_mode == "tcgen05_pool":
                     # conv + bn1 + relu + maxpool + first encode: one tensor-core kernel
-                    cur, c0, self._stem_scratch = conv_codes.stem_conv_pool(
-                        x.permute(0, 2, 3, 1), self.stem_w, self.stem_bn_pool, relu=True, next_quant=q0,
-                        scratch=self._stem_scratch)
+                    cur, c0, _ = conv_codes.stem_conv_pool(x.permute(0, 2, 3, 1), self.stem_w, self.stem_bn_pool, relu=True,
+                                                           next_quant=q0)
                 else:
                     # conv + row max of the pool window, then column max + bn1 + relu + first encode
-                    y, self._stem_scratch = conv_codes.stem_conv7x7s2(x.permute(0, 2, 3, 1), self.stem_w, self._stem_scratch,
-                                                                      cout=m.conv1.out_channels, rowmax=True)
+                    y, _ = conv_codes.stem_conv7x7s2(x.permute(0, 2, 3, 1), self.stem_w, cout=m.conv1.out_channels,
+                                                     rowmax=True)
                     cur, c0 = conv_codes.bn_relu_maxpool_encode(y, self.stem_bn_pool, relu=True, next_quant=q0, rowmax=True)
             else:
                 y = m.conv1(x.float()).permute(0, 2, 3, 1)

@@ -226,8 +226,10 @@ class ShardedInference:
 
     @torch.no_grad()
     def finish(self):
-        """Complete outstanding gathers.  Returns the gathered logits: of the last step ('step' / 'async') or of
-        every step since the last finish(), shape [steps, world * batch, classes] ('end')."""
+        """Complete outstanding gathers.  Returns the gathered logits of what is still outstanding: of the last step
+        ('async'), or of every step since the last finish(), shape [steps, world * batch, classes] ('end').  Returns
+        None when nothing is outstanding: with 'step', with world size 1 (every forward already returned its logits)
+        and when no step ran since the last finish()."""
         cur = torch.cuda.current_stream(self.device)
         if self.gather == "async" and self._side is not None:
             cur.wait_stream(self._side)
@@ -241,8 +243,13 @@ class ShardedInference:
     def stage(self, pinned):
         """Start the host->device copy of a pinned shard on the copy stream; returns the slot.
         `slots` device buffers rotate: stage shards i+1 (and i+2), then run(shard i), and the copies overlap the
-        compute; a slot is rewritten only after the forward that read it has been enqueued."""
+        compute; a slot is rewritten only after the forward that read it has been enqueued (staging more shards ahead
+        than there are slots raises)."""
         s = self._slot
+        if self._stage_evt[s] is not None and self._done_evt[s] is None:
+            # the shard staged in this slot has not run yet: rewriting it would make that run read this shard
+            raise RuntimeError(f"stage(): all {self.slots} slots hold shards that have not run; run() one first or "
+                               "use more slots")
         self._slot = (s + 1) % self.slots
         if self._stage[s] is None or self._stage[s].shape != pinned.shape or \
                 self._stage[s].stride() != pinned.stride():
@@ -257,6 +264,7 @@ class ShardedInference:
             evt = torch.cuda.Event()
             evt.record(self.copy_stream)
         self._stage_evt[s] = evt
+        self._done_evt[s] = None
         return s
 
     @torch.no_grad()
