@@ -56,7 +56,12 @@ extern "C" {
 
 /* term encodings.  The reference kernel implements HESE only
  * (kernels/tr_cuda_kernel.cu:29-55); BINARY (bit_utils.py:63-73) and radix-2
- * BOOTH (verilog/booth_encoder.v:57-78) are additions with the same selection rule. */
+ * BOOTH (verilog/booth_encoder.v:57-78) are additions with the same selection rule.
+ * For every encoding the truncated code of q in [0, 2^bits - 1] satisfies |code| <= 2^bits
+ * (BINARY: <= 2^bits - 1) and is non-decreasing in q (DESIGN.md section 3).  Every fused
+ * entry point below encodes with HESE; its _enc twin takes the encoding (`next_enc`,
+ * after the term budget) and returns TQ_ERR_INVALID for any other value before it
+ * launches anything. */
 #define TQ_ENC_HESE    0
 #define TQ_ENC_BINARY  1
 #define TQ_ENC_BOOTH   2
@@ -129,6 +134,10 @@ int tq_hist_accumulate(const void *x, int dtype, int64_t n,
 int tq_mse_profile(const float *hist, const float *x, int nbins,
                    const float *sfs, int nsf, int bits, int terms,
                    double *errs, int *argmin, void *stream);
+/* the same sweep with tr(x[b]) in the given TQ_ENC_* encoding */
+int tq_mse_profile_enc(const float *hist, const float *x, int nbins,
+                       const float *sfs, int nsf, int bits, int terms, int encoding,
+                       double *errs, int *argmin, void *stream);
 
 /*
  * *count += sum_i len(hese(int(w[i] / sf)))  (tr_layer.py:57-63, the per-element
@@ -136,6 +145,9 @@ int tq_mse_profile(const float *hist, const float *x, int nbins,
  */
 int tq_hese_term_count(const void *w, int dtype, int64_t n, float sf, unsigned flags,
                        unsigned long long *count, void *stream);
+/* the same count for any TQ_ENC_* encoding: *count += sum_i (number of terms of int(w[i] / sf)) */
+int tq_term_count(const void *w, int dtype, int64_t n, float sf, int encoding, unsigned flags,
+                  unsigned long long *count, void *stream);
 
 /*
  * Convolution on term codes with tcgen05 tensor cores (replaces the cuDNN fp32 conv under
@@ -170,7 +182,7 @@ int tq_conv2d_codes_f16(const void *act, const void *wgt, const float *bias, flo
  *     t = float(acc) * scale (+ bias[co]);  t = fma(t, bn_a[co], bn_b[co]);  t += residual[n,ho,wo,co];
  *     t = max(t, 0) if relu (relu = 2: ReLU6, t = min(max(t, 0), 6));  out_f32 = t;
  *     out_codes = term code of t under the consumer's quantiser
- *     (next_sf, next_bits <= 10, next_terms; g = 1, HESE) stored as fp16 NHWC.
+ *     (next_sf, next_bits <= 10, next_terms; g = 1, HESE; _enc: next_enc) stored as fp16 NHWC.
  * Every step is optional (NULL pointer / relu = 0); at least one of out_f32, out_codes is given.
  * Every step is one IEEE fp32 operation in this order, so the result is reproducible bit for bit on a CPU
  * (oracle/fused_emul.py).  Outputs are written with TMA stores from swizzled shared memory (fully coalesced,
@@ -181,6 +193,11 @@ int tq_conv2d_codes_fused(const void *act, const void *wgt, float *out_f32, void
                           int N, int H, int W, int C, int Cout, int R, int S, int stride, int pad,
                           float scale, int relu, float next_sf, int next_bits, int next_terms,
                           int acc_groups, void *stream);
+int tq_conv2d_codes_fused_enc(const void *act, const void *wgt, float *out_f32, void *out_codes,
+                              const float *bias, const float *bn_a, const float *bn_b, const float *residual,
+                              int N, int H, int W, int C, int Cout, int R, int S, int stride, int pad,
+                              float scale, int relu, float next_sf, int next_bits, int next_terms, int next_enc,
+                              int acc_groups, void *stream);
 
 /*
  * The same fused conv on SIGNED 8-BIT OPERAND PLANES with tcgen05.mma kind::i8 and int32 accumulators in
@@ -192,13 +209,18 @@ int tq_conv2d_codes_fused(const void *act, const void *wgt, float *out_f32, void
  * Plane pair (pa, pw) accumulates into TMEM accumulator pa + pw; the epilogue recombines them by Horner's rule
  * with the plane shift in int32 and continues exactly as tq_conv2d_codes_fused.  act_max / wgt_max are the caller's
  * bounds on |code| (2^bits by construction of the term codes); C * R * S * act_max * wgt_max < 2^31 is required.
- * tq_codes_to_planes() produces the planes from fp16 codes.
+ * tq_codes_to_planes() produces the planes from fp16 codes.  The output codes are HESE; _enc: next_enc.
  */
 int tq_conv2d_planes_i8(const void *act_planes, const void *wgt_planes, int planes_a, int planes_w,
                         float *out_f32, void *out_codes, const float *bias, const float *bn_a,
                         const float *bn_b, const float *residual, int N, int H, int W, int C, int Cout,
                         int R, int S, int stride, int pad, float scale, int relu, float next_sf,
                         int next_bits, int next_terms, int act_max, int wgt_max, void *stream);
+int tq_conv2d_planes_i8_enc(const void *act_planes, const void *wgt_planes, int planes_a, int planes_w,
+                            float *out_f32, void *out_codes, const float *bias, const float *bn_a,
+                            const float *bn_b, const float *residual, int N, int H, int W, int C, int Cout,
+                            int R, int S, int stride, int pad, float scale, int relu, float next_sf,
+                            int next_bits, int next_terms, int next_enc, int act_max, int wgt_max, void *stream);
 
 /* fp16 integer codes (n elements, n % 8 == 0) -> `planes` signed 8-bit planes of n bytes each, plane p at
  * planes_s8 + p * n.  planes = 1 stores the code itself; a value that does not fit sets *overflow (device int,
@@ -214,11 +236,14 @@ int tq_conv_weight_l1(const void *wgt_f16, int RS, int Cout, int C, long long *p
  * Fused tail of the unquantised stem (torchvision ResNet: bn1 -> relu -> maxpool(3, 2, 1), then
  * the first wrapped conv's LinearQuantize, tr_layer.py:96-99): x fp32 NHWC [N,H,W,C] ->
  * out fp32 NHWC [N,Ho,Wo,C] = maxpool3x3s2p1(relu(fma(x, bn_a, bn_b))) and, if out_codes != NULL,
- * the fp16 term codes of `out` under (next_sf, next_bits <= 11, next_terms).  C % 4 == 0.
+ * the fp16 term codes of `out` under (next_sf, next_bits <= 11, next_terms; HESE, _enc: next_enc).  C % 4 == 0.
  */
 int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, const float *bn_b, float *out,
                               void *out_codes, int N, int H, int W, int C, int relu,
                               float next_sf, int next_bits, int next_terms, void *stream);
+int tq_bn_relu_maxpool_encode_enc(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                  void *out_codes, int N, int H, int W, int C, int relu,
+                                  float next_sf, int next_bits, int next_terms, int next_enc, void *stream);
 
 /*
  * The unquantised stem conv of the CNNs (7x7, stride 2, pad 3, 3 input channels, no bias;
@@ -250,7 +275,7 @@ int tq_stem_conv7x7s2_u8(const void *x_u8, const float *mean3, const float *std3
 /*
  * The whole unquantised stem in one tensor-core kernel: conv 7x7/s2/p3 -> per-channel affine (BatchNorm) ->
  * ReLU (if relu) -> max-pool 3x3/s2/p1 -> fp32 NHWC [N, Hp, Wp, Cout] (Hp = (H/2 - 1)/2 + 1) and, if out_codes,
- * the fp16 term codes of that tensor for the first wrapped conv's quantiser (tr_layer.py:96-99).  Each tile
+ * the fp16 term codes of that tensor for the first wrapped conv's quantiser (tr_layer.py:96-99; HESE, _enc: next_enc).  Each tile
  * computes the (2P+1) x (2Q+1) conv pixels under P x Q pooled pixels, so the conv output (822 MB at batch 256)
  * never reaches HBM.  Same values as tq_stem_conv7x7s2_dt followed by tq_bn_relu_maxpool_encode.
  * CONTRACT: bn_a >= 0.  The pooling takes the window maximum of the raw conv sums and applies the affine once
@@ -262,6 +287,10 @@ int tq_stem_conv7x7s2_pool(const void *x, int x_dtype, void *x2_scratch, const v
                            const float *bn_a, const float *bn_b, int relu, float *out, void *out_codes,
                            int N, int H, int W, int Cout, float next_sf, int next_bits, int next_terms,
                            void *stream);
+int tq_stem_conv7x7s2_pool_enc(const void *x, int x_dtype, void *x2_scratch, const void *w2,
+                               const float *bn_a, const float *bn_b, int relu, float *out, void *out_codes,
+                               int N, int H, int W, int Cout, float next_sf, int next_bits, int next_terms,
+                               int next_enc, void *stream);
 
 /*
  * The stem in two passes that split the 3x3/s2/p1 max-pool by axis, so that only half of the conv map crosses HBM:
@@ -282,6 +311,9 @@ int tq_stem_conv7x7s2_u8_rowmax(const void *x_u8, const float *mean3, const floa
 int tq_bn_relu_maxpool_encode_rowmax(const float *x, const float *bn_a, const float *bn_b, float *out,
                                      void *out_codes, int N, int H, int W, int C, int relu,
                                      float next_sf, int next_bits, int next_terms, void *stream);
+int tq_bn_relu_maxpool_encode_rowmax_enc(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                         void *out_codes, int N, int H, int W, int C, int relu,
+                                         float next_sf, int next_bits, int next_terms, int next_enc, void *stream);
 
 /*
  * Depthwise 3x3 conv (pad 1, stride 1 or 2) on term codes, the memory-bound layer of the depthwise CNNs
@@ -289,7 +321,8 @@ int tq_bn_relu_maxpool_encode_rowmax(const float *x, const float *bn_a, const fl
  * and run as TR encode -> cuDNN fp32 conv -> BatchNorm -> ReLU6, tr_layer.py:124-126):
  *     acc[n,ho,wo,c] = sum_{r,s} act[n, ho*stride+r-1, wo*stride+s-1, c] * wgt[r*3+s, c]        (int32, exact)
  *     t = float(acc) * scale (+ bias[c]);  t = fma(t, bn_a[c], bn_b[c]);  relu: 0 none, 1 ReLU, 2 ReLU6;
- *     out_f32 = t and / or out_codes = fp16 term code of t under (next_sf, next_bits <= 11, next_terms), g = 1, HESE.
+ *     out_f32 = t and / or out_codes = fp16 term code of t under (next_sf, next_bits <= 11, next_terms), g = 1, HESE
+ *     (_enc: next_enc).
  * act fp16 NHWC [N,H,W,C] integer codes, wgt int32 [9][C] integer codes (|a| <= 2^11, |w| <= 2^16), C % 8 == 0.
  * act_unsigned != 0: the caller guarantees 0 <= act <= 1023 (the output of a ReLU under a quantiser of <= 9 bits), which
  * lets the kernel extract the integers without conversion instructions.  Input tiles (with their zero halo) are staged
@@ -299,28 +332,38 @@ int tq_depthwise3x3_codes(const void *act_codes, const int32_t *wgt_codes, float
                           const float *bias, const float *bn_a, const float *bn_b, int N, int H, int W, int C,
                           int stride, float scale, int relu, int act_unsigned, float next_sf, int next_bits,
                           int next_terms, void *stream);
+int tq_depthwise3x3_codes_enc(const void *act_codes, const int32_t *wgt_codes, float *out_f32, void *out_codes,
+                              const float *bias, const float *bn_a, const float *bn_b, int N, int H, int W, int C,
+                              int stride, float scale, int relu, int act_unsigned, float next_sf, int next_bits,
+                              int next_terms, int next_enc, void *stream);
 
 /*
  * Tail of an unwrapped conv (the first conv of every CNN, cnn_models/__init__.py:34-36) fused with the first wrapped
  * layer's LinearQuantize (tr_layer.py:96-99): x fp32 [npix][C] -> + bias (the conv's own bias, one fp32 add, when the
  * conv ran without it; may be NULL) -> fma(x, bn_a, bn_b) -> activation (relu as above) -> out_f32 and / or fp16 term
- * codes.  C % 4 == 0.
+ * codes (HESE; _enc: next_enc).  C % 4 == 0.
  */
 int tq_bn_act_encode(const float *x, const float *bias, const float *bn_a, const float *bn_b, float *out_f32,
                      void *out_codes, int64_t npix, int C, int relu, float next_sf, int next_bits, int next_terms,
                      void *stream);
+int tq_bn_act_encode_enc(const float *x, const float *bias, const float *bn_a, const float *bn_b, float *out_f32,
+                         void *out_codes, int64_t npix, int C, int relu, float next_sf, int next_bits, int next_terms,
+                         int next_enc, void *stream);
 
 /*
  * The unwrapped first conv of the VGG-style / depthwise CNNs (cnn_models/__init__.py:34-36: nn.Conv2d(3, Cout, 3, stride,
  * padding=1), Cout 32 or 64, stride 1 or 2) in fp32 on the CUDA cores, fused with what follows it: + bias, BatchNorm
  * affine, ReLU / ReLU6 and the first wrapped layer's LinearQuantize (tr_layer.py:96-99).  x fp32 NHWC [N][H][W][3],
  * wgt fp32 [3][3][3][Cout] (filter row, filter column, input channel, output channel); sums run in that order, one
- * fmaf per term, bias added after the sum.  out_f32 and / or fp16 term codes, NHWC.  An fp32 conv: it equals cuDNN's
- * up to the summation order, not bit for bit.
+ * fmaf per term, bias added after the sum.  out_f32 and / or fp16 term codes (HESE; _enc: next_enc), NHWC.  An fp32
+ * conv: it equals cuDNN's up to the summation order, not bit for bit.
  */
 int tq_first_conv3x3_fused(const float *x, const float *wgt, const float *bias, const float *bn_a, const float *bn_b,
                            float *out_f32, void *out_codes, int N, int H, int W, int Cout, int stride, int relu,
                            float next_sf, int next_bits, int next_terms, void *stream);
+int tq_first_conv3x3_fused_enc(const float *x, const float *wgt, const float *bias, const float *bn_a, const float *bn_b,
+                               float *out_f32, void *out_codes, int N, int H, int W, int Cout, int stride, int relu,
+                               float next_sf, int next_bits, int next_terms, int next_enc, void *stream);
 
 /*
  * nn.MaxPool2d(k, stride, pad) (floor mode, no dilation) on an fp16 NHWC tensor: the term codes between the convs of

@@ -14,6 +14,15 @@ TQ_OK, TQ_ERR_INVALID, TQ_ERR_UNSUPPORTED, TQ_ERR_CUDA = 0, 1, 2, 3
 TQ_F32, TQ_F64, TQ_BF16, TQ_F16 = 0, 1, 2, 3
 TQ_I8, TQ_I16, TQ_I32, TQ_U8, TQ_F16C = 0, 1, 2, 3, 4
 ENC_HESE, ENC_BINARY, ENC_BOOTH = 0, 1, 2
+ENCODINGS = {"hese": ENC_HESE, "binary": ENC_BINARY, "booth": ENC_BOOTH}
+
+
+def encoding_id(encoding):
+    """TQ_ENC_* value of a term encoding name; ValueError for anything else."""
+    if not isinstance(encoding, str) or encoding not in ENCODINGS:
+        raise ValueError(f"unknown term encoding {encoding!r}: expected one of {', '.join(ENCODINGS)}")
+    return ENCODINGS[encoding]
+
 FLAG_RELU, FLAG_RECIP_DIV, FLAG_EXACT_DIV = 1, 2, 4
 
 # every symbol include/tq_b200.h declares: (restype, argtypes)
@@ -26,25 +35,35 @@ SYMBOLS = {
     "tq_tr_encode_codes": (_i, [_p, _p, _i, _i, _i64, _i64, _i64, _f, _i, _i, _i, _i, _u, _p, _p]),
     "tq_hist_accumulate": (_i, [_p, _i, _i64, _p, _p, _i, _f, _f, _p]),
     "tq_mse_profile": (_i, [_p, _p, _i, _p, _i, _i, _i, _p, _p, _p]),
+    "tq_mse_profile_enc": (_i, [_p, _p, _i, _p, _i, _i, _i, _i, _p, _p, _p]),
     "tq_hese_term_count": (_i, [_p, _i, _i64, _f, _u, _p, _p]),
+    "tq_term_count": (_i, [_p, _i, _i64, _f, _i, _u, _p, _p]),
     "tq_conv2d_codes_f16": (_i, [_p, _p, _p, _p] + [_i] * 9 + [_f, _i, _p]),
     "tq_conv2d_codes_fused": (_i, [_p] * 8 + [_i] * 9 + [_f, _i, _f, _i, _i, _i, _p]),
+    "tq_conv2d_codes_fused_enc": (_i, [_p] * 8 + [_i] * 9 + [_f, _i, _f, _i, _i, _i, _i, _p]),
     "tq_conv2d_planes_i8": (_i, [_p, _p, _i, _i] + [_p] * 6 + [_i] * 9 + [_f, _i, _f, _i, _i, _i, _i, _p]),
+    "tq_conv2d_planes_i8_enc": (_i, [_p, _p, _i, _i] + [_p] * 6 + [_i] * 9 + [_f, _i, _f, _i, _i, _i, _i, _i, _p]),
     "tq_codes_to_planes": (_i, [_p, _p, _i64, _i, _p, _p]),
     "tq_conv_weight_l1": (_i, [_p, _i, _i, _i, _p, _p, _p]),
     "tq_depthwise3x3_codes": (_i, [_p] * 7 + [_i] * 5 + [_f, _i, _i, _f, _i, _i, _p]),
+    "tq_depthwise3x3_codes_enc": (_i, [_p] * 7 + [_i] * 5 + [_f, _i, _i, _f, _i, _i, _i, _p]),
     "tq_bn_act_encode": (_i, [_p] * 6 + [_i64, _i, _i, _f, _i, _i, _p]),
+    "tq_bn_act_encode_enc": (_i, [_p] * 6 + [_i64, _i, _i, _f, _i, _i, _i, _p]),
     "tq_maxpool2d_f16": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _p]),
     "tq_first_conv3x3_fused": (_i, [_p] * 7 + [_i, _i, _i, _i, _i, _i, _f, _i, _i, _p]),
+    "tq_first_conv3x3_fused_enc": (_i, [_p] * 7 + [_i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p]),
     "tq_u8_normalize_bf16": (_i, [_p, _p, _i64, _p, _p, _p]),
     "tq_bn_relu_maxpool_encode": (_i, [_p] * 5 + [_i] * 5 + [_f, _i, _i, _p]),
+    "tq_bn_relu_maxpool_encode_enc": (_i, [_p] * 5 + [_i] * 5 + [_f, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2_dt": (_i, [_p, _i, _p, _p, _p, _i, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2_u8": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2_pool": (_i, [_p, _i, _p, _p, _p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _i, _i, _p]),
+    "tq_stem_conv7x7s2_pool_enc": (_i, [_p, _i, _p, _p, _p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2_rowmax": (_i, [_p, _i, _p, _p, _p, _i, _i, _i, _i, _p]),
     "tq_stem_conv7x7s2_u8_rowmax": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p]),
     "tq_bn_relu_maxpool_encode_rowmax": (_i, [_p] * 5 + [_i] * 5 + [_f, _i, _i, _p]),
+    "tq_bn_relu_maxpool_encode_rowmax_enc": (_i, [_p] * 5 + [_i] * 5 + [_f, _i, _i, _i, _p]),
     "tq_selftest_division": (_i, [C.c_uint64, C.c_uint32, _p, _p]),
 }
 

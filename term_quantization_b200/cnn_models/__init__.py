@@ -13,6 +13,7 @@ from copy import deepcopy
 import torch.nn as nn
 from torchvision.models import alexnet, mobilenet_v2, resnet18, vgg16_bn  # noqa: F401
 
+from .. import _lib
 from ..tr_layer import TRConv2dLayer
 
 try:  # optional, exactly as optional as in the image
@@ -52,15 +53,17 @@ def _parent_of(model, name):
     return parent, keys[-1]
 
 
-def replace_conv_layers(model, tr_params, data_bits, data_terms):
-    """Swap every conv but the first for a TRConv2dLayer, in named_modules order."""
+def replace_conv_layers(model, tr_params, data_bits, data_terms, *, encoding='hese'):
+    """Swap every conv but the first for a TRConv2dLayer, in named_modules order; `encoding` is the term encoding
+    ('hese', 'binary' or 'booth') of every wrapped layer."""
+    _lib.encoding_id(encoding)
     for idx, (name, layer) in enumerate(_conv_layers(model)):
         if idx == 0:
             continue
         weight_bits, group_size, weight_terms = tr_params[idx]
         parent, key = _parent_of(model, name)
         parent._modules[key] = TRConv2dLayer(layer, data_bits, data_terms, weight_bits,
-                                             group_size, weight_terms)
+                                             group_size, weight_terms, encoding=encoding)
     return model
 
 
@@ -74,6 +77,7 @@ def static_conv_layer_settings(model, weight_bits, group_size, num_terms):
     return stats
 
 
-def convert_model(model, tr_params, data_bits, data_terms):
-    # the conversion rewrites weights in place, so work on a copy
-    return replace_conv_layers(deepcopy(model), tr_params, data_bits, data_terms)
+def convert_model(model, tr_params, data_bits, data_terms, *, encoding='hese'):
+    # the conversion rewrites weights in place, so work on a copy (refuse a bad encoding before copying)
+    _lib.encoding_id(encoding)
+    return replace_conv_layers(deepcopy(model), tr_params, data_bits, data_terms, encoding=encoding)

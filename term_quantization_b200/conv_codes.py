@@ -27,6 +27,27 @@ def pack_conv_weight(w, w_sf, weight_bits, group_size, num_terms):
 EXACT_LIMIT = 1 << 24
 
 
+def _quant_args(next_quant):
+    """(sf, bits, terms, TQ_ENC_*) of a consumer's quantiser given as (sf, bits, terms) -- HESE -- or
+    (sf, bits, terms, encoding name); None: no codes are written."""
+    if not next_quant:
+        return 1.0, 1, 0, _lib.ENC_HESE
+    if len(next_quant) not in (3, 4):
+        raise ValueError(f"next_quant must be (sf, bits, terms) or (sf, bits, terms, encoding), got {next_quant!r}")
+    enc = _lib.encoding_id(next_quant[3]) if len(next_quant) == 4 else _lib.ENC_HESE
+    return next_quant[0], next_quant[1], next_quant[2], enc
+
+
+def _entry(name, enc, at):
+    """The C entry point for a consumer quantiser in encoding `enc`, called with the arguments of `name`_enc: HESE goes
+    to the original entry point `name` (the encoding, argument `at`, dropped), any other encoding to the _enc twin."""
+    L = _lib.lib()
+    if enc != _lib.ENC_HESE:
+        return getattr(L, name + "_enc")
+    fn = getattr(L, name)
+    return lambda *args: fn(*args[:at], *args[at + 1:])
+
+
 def _relu_code(relu):
     """Activation of the fused epilogues: False / 0 none, True / 1 ReLU, 'relu6' / 2 ReLU6."""
     if relu in ("relu6", 2):
@@ -133,26 +154,25 @@ def _cached_plan(wgt, act_max, signed_act, engine):
 
 
 def _run_conv(act, plan, out, codes, bias, bn, residual, N, H, W, C, Cout, R, S, stride, pad, scale, relu, sf, bits,
-              terms, act_planes=None):
+              terms, enc, act_planes=None):
     ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
-    L = _lib.lib()
     stream = torch.cuda.current_stream(act.device).cuda_stream
     with torch.cuda.device(act.device):
         if plan.engine == "f16":
-            rc = L.tq_conv2d_codes_fused(
+            rc = _entry("tq_conv2d_codes_fused", enc, 22)(
                 act.data_ptr(), plan.wgt.data_ptr(), ptr(out), ptr(codes), ptr(bias),
                 ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None, ptr(residual),
                 N, H, W, C, Cout, R, S, stride, pad, float(scale), _relu_code(relu), float(sf), int(bits),
-                int(terms), int(plan.groups), stream)
+                int(terms), enc, int(plan.groups), stream)
         else:
             if act_planes is None:
                 pa = _planes_needed(plan.act_max)
                 act_planes, _ = codes_to_planes(act, pa)
-            rc = L.tq_conv2d_planes_i8(
+            rc = _entry("tq_conv2d_planes_i8", enc, 24)(
                 act_planes.data_ptr(), plan.planes.data_ptr(), act_planes.shape[0], plan.planes_w, ptr(out), ptr(codes),
                 ptr(bias), ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None, ptr(residual),
                 N, H, W, C, Cout, R, S, stride, pad, float(scale), _relu_code(relu), float(sf), int(bits), int(terms),
-                int(plan.act_max), int(plan.wgt_max), stream)
+                enc, int(plan.act_max), int(plan.wgt_max), stream)
     _lib.check(rc)
 
 
@@ -176,7 +196,8 @@ def conv2d_codes(act, wgt, bias, kernel_size, stride, pad, scale, out=None, *, a
         out = torch.empty((N, Ho, Wo, Cout), dtype=torch.float32, device=act.device)
     if plan is None:
         plan = _cached_plan(wgt, act_max, signed_act, engine)
-    _run_conv(act, plan, out, None, bias, None, None, N, H, W, C, Cout, R, S, stride, pad, scale, False, 1.0, 1, 0)
+    _run_conv(act, plan, out, None, bias, None, None, N, H, W, C, Cout, R, S, stride, pad, scale, False, 1.0, 1, 0,
+              _lib.ENC_HESE)
     return out
 
 
@@ -186,7 +207,8 @@ def conv2d_codes_fused(act, wgt, kernel_size, stride, pad, scale, *, bias=None, 
     """Conv on codes with the fused tail (see tq_conv2d_codes_fused in include/tq_b200.h).
 
     bn = (a, b) fp32 [Cout] per-channel affine applied as fma(t, a, b); residual fp32
-    [N, Ho, Wo, Cout]; next_quant = (sf, bits, terms) of the consumer's LinearQuantize.
+    [N, Ho, Wo, Cout]; next_quant = (sf, bits, terms) of the consumer's LinearQuantize (HESE), or
+    (sf, bits, terms, encoding) for a consumer with another term encoding.
     Returns (out_f32 or None, out_codes or None)."""
     N, H, W, C = act.shape
     R, S = kernel_size
@@ -200,10 +222,11 @@ def conv2d_codes_fused(act, wgt, kernel_size, stride, pad, scale, *, bias=None, 
     if residual is not None and (residual.shape != (N, Ho, Wo, Cout) or not residual.is_contiguous()
                                  or residual.dtype != torch.float32):
         raise RuntimeError("residual must be a contiguous fp32 [N, Ho, Wo, Cout] tensor")
-    sf, bits, terms = next_quant if next_quant else (1.0, 1, 0)
+    sf, bits, terms, enc = _quant_args(next_quant)
     if plan is None:
         plan = _cached_plan(wgt, act_max, signed_act, engine)
-    _run_conv(act, plan, out, codes, bias, bn, residual, N, H, W, C, Cout, R, S, stride, pad, scale, relu, sf, bits, terms)
+    _run_conv(act, plan, out, codes, bias, bn, residual, N, H, W, C, Cout, R, S, stride, pad, scale, relu, sf, bits, terms,
+              enc)
     return out, codes
 
 
@@ -272,13 +295,13 @@ def depthwise3x3_codes(act, wgt, stride, scale, *, bias=None, bn=None, relu=Fals
     Ho, Wo = (H - 1) // stride + 1, (W - 1) // stride + 1
     out = torch.empty((N, Ho, Wo, C), dtype=torch.float32, device=act.device) if want_f32 else None
     codes = torch.empty((N, Ho, Wo, C), dtype=torch.float16, device=act.device) if next_quant else None
-    sf, bits, terms = next_quant if next_quant else (1.0, 1, 0)
+    sf, bits, terms, enc = _quant_args(next_quant)
     ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
     with torch.cuda.device(act.device):
-        rc = _lib.lib().tq_depthwise3x3_codes(
+        rc = _entry("tq_depthwise3x3_codes", enc, 18)(
             act.data_ptr(), wgt.data_ptr(), ptr(out), ptr(codes), ptr(bias), ptr(bn[0]) if bn else None,
             ptr(bn[1]) if bn else None, N, H, W, C, stride, float(scale), _relu_code(relu), int(bool(act_unsigned)),
-            float(sf), int(bits), int(terms), torch.cuda.current_stream(act.device).cuda_stream)
+            float(sf), int(bits), int(terms), enc, torch.cuda.current_stream(act.device).cuda_stream)
     _lib.check(rc)
     return out, codes
 
@@ -303,15 +326,15 @@ def first_conv3x3_fused(x_nhwc, w_packed, stride=1, bias=None, bn=None, relu=Fal
     codes = torch.empty((N, Ho, Wo, Cout), dtype=torch.float16, device=x_nhwc.device) if next_quant else None
     if out is None and codes is None:
         raise RuntimeError("first_conv3x3_fused: nothing to compute (want_f32 or next_quant)")
-    sf, bits, terms = next_quant if next_quant else (1.0, 1, 0)
+    sf, bits, terms, enc = _quant_args(next_quant)
     ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
     for t in (bias, bn[0] if bn else None, bn[1] if bn else None):
         if t is not None and (t.dtype != torch.float32 or t.numel() != Cout or not t.is_contiguous() or t.device != x_nhwc.device):
             raise RuntimeError("first_conv3x3_fused: bias / bn must be contiguous fp32 [Cout] tensors on the input's device")
     with torch.cuda.device(x_nhwc.device):
-        rc = _lib.lib().tq_first_conv3x3_fused(
+        rc = _entry("tq_first_conv3x3_fused", enc, 16)(
             x_nhwc.data_ptr(), w_packed.data_ptr(), ptr(bias), ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None,
-            ptr(out), ptr(codes), N, H, W, Cout, int(stride), _relu_code(relu), float(sf), int(bits), int(terms),
+            ptr(out), ptr(codes), N, H, W, Cout, int(stride), _relu_code(relu), float(sf), int(bits), int(terms), enc,
             torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
     return out, codes
@@ -341,14 +364,14 @@ def bn_act_encode(x_nhwc, bn=None, relu=False, want_f32=False, next_quant=None, 
     C = x_nhwc.shape[-1]
     out = torch.empty_like(x_nhwc) if want_f32 else None
     codes = torch.empty(x_nhwc.shape, dtype=torch.float16, device=x_nhwc.device) if next_quant else None
-    sf, bits, terms = next_quant if next_quant else (1.0, 1, 0)
+    sf, bits, terms, enc = _quant_args(next_quant)
     ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
     with torch.cuda.device(x_nhwc.device):
         if bias is not None and (bias.dtype != torch.float32 or bias.numel() != C or not bias.is_contiguous() or bias.device != x_nhwc.device):
             raise RuntimeError("bn_act_encode: bias must be a contiguous fp32 [C] tensor on the input's device")
-        rc = _lib.lib().tq_bn_act_encode(
+        rc = _entry("tq_bn_act_encode", enc, 12)(
             x_nhwc.data_ptr(), ptr(bias), ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None, ptr(out), ptr(codes),
-            x_nhwc.numel() // C, C, _relu_code(relu), float(sf), int(bits), int(terms),
+            x_nhwc.numel() // C, C, _relu_code(relu), float(sf), int(bits), int(terms), enc,
             torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
     return out, codes
@@ -365,13 +388,13 @@ def bn_relu_maxpool_encode(x_nhwc, bn, relu=True, next_quant=None, rowmax=False)
     Ho, Wo = (H - 1) // 2 + 1, (W if rowmax else (W - 1) // 2 + 1)
     out = torch.empty((N, Ho, Wo, C), dtype=torch.float32, device=x_nhwc.device)
     codes = torch.empty((N, Ho, Wo, C), dtype=torch.float16, device=x_nhwc.device) if next_quant else None
-    sf, bits, terms = next_quant if next_quant else (1.0, 1, 0)
-    fn = _lib.lib().tq_bn_relu_maxpool_encode_rowmax if rowmax else _lib.lib().tq_bn_relu_maxpool_encode
+    sf, bits, terms, enc = _quant_args(next_quant)
+    fn = _entry("tq_bn_relu_maxpool_encode_rowmax" if rowmax else "tq_bn_relu_maxpool_encode", enc, 13)
     with torch.cuda.device(x_nhwc.device):
         rc = fn(
             x_nhwc.data_ptr(), bn[0].data_ptr(), bn[1].data_ptr(), out.data_ptr(),
             codes.data_ptr() if codes is not None else None, N, H, W, C, int(bool(relu)),
-            float(sf), int(bits), int(terms), torch.cuda.current_stream(x_nhwc.device).cuda_stream)
+            float(sf), int(bits), int(terms), enc, torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
     return out, codes
 
@@ -465,7 +488,7 @@ def stem_pool_operands(w, bn):
 def stem_conv_pool(x_nhwc, w2, bn, relu=True, next_quant=None, scratch=None):
     # (Cout = number of BatchNorm channels: the packed weight tile is always 128 rows)
     """The whole stem in one launch: maxpool3x3/s2/p1(relu(fma(conv7x7s2(x), a, b))) -> fp32
-    [N, Hp, Wp, Cout] plus the fp16 term codes of the result (next_quant = (sf, bits, terms)).
+    [N, Hp, Wp, Cout] plus the fp16 term codes of the result (next_quant = (sf, bits, terms[, encoding])).
     Same values as stem_conv7x7s2 followed by bn_relu_maxpool_encode; the conv output never reaches HBM.
     `w2`, `bn` must come from stem_pool_operands (sign of the slope folded into the weights, bn[0] >= 0).
     Returns (out, codes or None, scratch)."""
@@ -479,12 +502,12 @@ def stem_conv_pool(x_nhwc, w2, bn, relu=True, next_quant=None, scratch=None):
     Hp, Wp = (H // 2 - 1) // 2 + 1, (W // 2 - 1) // 2 + 1
     out = torch.empty((N, Hp, Wp, Cout), dtype=torch.float32, device=x_nhwc.device)
     codes = torch.empty((N, Hp, Wp, Cout), dtype=torch.float16, device=x_nhwc.device) if next_quant else None
-    sf, bits, terms = next_quant if next_quant else (1.0, 1, 0)
+    sf, bits, terms, enc = _quant_args(next_quant)
     with torch.cuda.device(x_nhwc.device):
-        rc = _lib.lib().tq_stem_conv7x7s2_pool(
+        rc = _entry("tq_stem_conv7x7s2_pool", enc, 16)(
             x_nhwc.data_ptr(), _STEM_DTYPES[x_nhwc.dtype], scratch.data_ptr(), w2.data_ptr(),
             bn[0].data_ptr(), bn[1].data_ptr(), int(bool(relu)), out.data_ptr(),
-            codes.data_ptr() if codes is not None else None, N, H, W, Cout, float(sf), int(bits), int(terms),
+            codes.data_ptr() if codes is not None else None, N, H, W, Cout, float(sf), int(bits), int(terms), enc,
             torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
     return out, codes, scratch

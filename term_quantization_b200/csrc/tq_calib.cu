@@ -71,7 +71,7 @@ constexpr int MSE_THREADS = 256;
 
 __global__ void __launch_bounds__(MSE_THREADS)
 mse_profile_kernel(const float *__restrict__ hist, const float *__restrict__ x, int nbins,
-                   const float *__restrict__ sfs, int bits, int terms, double *__restrict__ errs)
+                   const float *__restrict__ sfs, int bits, int terms, int enc, double *__restrict__ errs)
 {
     const int s = blockIdx.x;
     const float sf = sfs[s];
@@ -81,7 +81,7 @@ mse_profile_kernel(const float *__restrict__ hist, const float *__restrict__ x, 
         const float xv = x[b];
         uint32_t neg;
         const uint32_t q = quantize_any<float, false>(xv, k, false, neg);
-        int code = elem_code(q, TQ_ENC_HESE, terms);
+        int code = elem_code(q, enc, terms);
         code = neg ? -code : code;
         const float xh = __fmul_rn((float)code, sf);
         const float d = __fsub_rn(xv, xh);                 // (x - xh)
@@ -129,10 +129,10 @@ argmin_kernel(const double *__restrict__ errs, int nsf, int *__restrict__ argmin
     if (threadIdx.x == 0) *argmin = bi[0];
 }
 
-// ---- HESE term count ---------------------------------------------------------------------------
+// ---- term count ---------------------------------------------------------------------------------
 template <typename Tin>
 __global__ void __launch_bounds__(256)
-hese_count_kernel(const Tin *__restrict__ w, int64_t n, float sf, float inv_sf, int recip,
+term_count_kernel(const Tin *__restrict__ w, int64_t n, float sf, float inv_sf, int recip, int enc,
                   unsigned long long *__restrict__ count)
 {
     unsigned long long local = 0;
@@ -142,7 +142,7 @@ hese_count_kernel(const Tin *__restrict__ w, int64_t n, float sf, float inv_sf, 
         const int k = __float2int_rz(r);                      // .int(): toward zero
         const uint32_t m = (uint32_t)(k < 0 ? -(long long)k : (long long)k);
         uint32_t T, N;
-        term_masks(m, TQ_ENC_HESE, T, N);
+        term_masks(m, enc, T, N);
         local += (unsigned)__popc(T);
     }
     for (int o = 16; o > 0; o >>= 1) local += __shfl_xor_sync(0xFFFFFFFFu, local, o);
@@ -236,11 +236,19 @@ extern "C" int tq_mse_profile(const float *hist, const float *x, int nbins, cons
                               int nsf, int bits, int terms, double *errs, int *argmin,
                               void *stream)
 {
+    return tq_mse_profile_enc(hist, x, nbins, sfs, nsf, bits, terms, TQ_ENC_HESE, errs, argmin, stream);
+}
+
+extern "C" int tq_mse_profile_enc(const float *hist, const float *x, int nbins, const float *sfs,
+                                  int nsf, int bits, int terms, int encoding, double *errs, int *argmin,
+                                  void *stream)
+{
+    if (check_encoding(encoding) != TQ_OK) return TQ_ERR_INVALID;
     if (!hist || !x || !sfs || !errs || !argmin) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (nbins < 1 || nsf < 1) return fail(TQ_ERR_INVALID, "empty sweep");
     if (bits < 1 || bits > TQ_MAX_BITS || terms < 0) return fail(TQ_ERR_INVALID, "bad bits/terms");
     cudaStream_t s = (cudaStream_t)stream;
-    mse_profile_kernel<<<nsf, MSE_THREADS, 0, s>>>(hist, x, nbins, sfs, bits, terms, errs);
+    mse_profile_kernel<<<nsf, MSE_THREADS, 0, s>>>(hist, x, nbins, sfs, bits, terms, encoding, errs);
     count_launch();
     int rc = check_launch("mse_profile_kernel");
     if (rc != TQ_OK) return rc;
@@ -252,6 +260,13 @@ extern "C" int tq_mse_profile(const float *hist, const float *x, int nbins, cons
 extern "C" int tq_hese_term_count(const void *w, int dtype, int64_t n, float sf, unsigned flags,
                                   unsigned long long *count, void *stream)
 {
+    return tq_term_count(w, dtype, n, sf, TQ_ENC_HESE, flags, count, stream);
+}
+
+extern "C" int tq_term_count(const void *w, int dtype, int64_t n, float sf, int encoding, unsigned flags,
+                             unsigned long long *count, void *stream)
+{
+    if (check_encoding(encoding) != TQ_OK) return TQ_ERR_INVALID;
     if (!count || (!w && n)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (!(sf > 0.0f)) return fail(TQ_ERR_INVALID, "sf must be positive");
     if (n <= 0) return TQ_OK;
@@ -261,15 +276,15 @@ extern "C" int tq_hese_term_count(const void *w, int dtype, int64_t n, float sf,
     const int grid = grid_cap(n, 256, 8);
     switch (dtype) {
         case TQ_F32:
-            hese_count_kernel<float><<<grid, 256, 0, s>>>((const float *)w, n, sf, inv, recip, count);
+            term_count_kernel<float><<<grid, 256, 0, s>>>((const float *)w, n, sf, inv, recip, encoding, count);
             break;
         case TQ_BF16:
-            hese_count_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>((const __nv_bfloat16 *)w, n, sf, inv, recip, count);
+            term_count_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>((const __nv_bfloat16 *)w, n, sf, inv, recip, encoding, count);
             break;
         default: return fail(TQ_ERR_UNSUPPORTED, "term count supports f32/bf16 inputs");
     }
     count_launch();
-    return check_launch("hese_count_kernel");
+    return check_launch("term_count_kernel");
 }
 
 extern "C" int tq_selftest_division(uint64_t n, uint32_t seed, unsigned long long *mismatch,

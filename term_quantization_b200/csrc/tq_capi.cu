@@ -27,6 +27,13 @@ int check_launch(const char *what)
     return TQ_OK;
 }
 
+int check_encoding(int enc)
+{
+    if (enc != TQ_ENC_HESE && enc != TQ_ENC_BINARY && enc != TQ_ENC_BOOTH)
+        return fail(TQ_ERR_INVALID, "unknown term encoding %d (TQ_ENC_HESE, TQ_ENC_BINARY or TQ_ENC_BOOTH)", enc);
+    return TQ_OK;
+}
+
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
 int num_sms()

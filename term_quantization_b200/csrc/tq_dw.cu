@@ -38,7 +38,7 @@ struct DwParams {
     int relu;                   // 0 none, 1 ReLU, 2 ReLU6
     int write_f32, write_codes;
     float next_sf;
-    int next_bits, next_terms, next_fastdiv;
+    int next_bits, next_terms, next_enc, next_fastdiv;
 };
 
 // activation shared by the epilogues of this file
@@ -82,7 +82,7 @@ depthwise3x3_codes_kernel(const __grid_constant__ CUtensorMap tmIn, const int32_
     for (int i = threadIdx.x; i < 9 * p.C; i += blockDim.x) sw[i] = wgt[i];
     if (p.write_codes) {
         for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), TQ_ENC_HESE, p.next_terms);
+            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
             lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
         }
     }
@@ -240,7 +240,7 @@ bn_act_encode_kernel(const float *__restrict__ x, float *__restrict__ out_f32, _
     __half *lut = reinterpret_cast<__half *>(dw_smem);
     if (p.write_codes) {
         for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), TQ_ENC_HESE, p.next_terms);
+            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
             lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
         }
         __syncthreads();
@@ -328,7 +328,7 @@ struct FirstConvParams {
     const float *bias, *bn_a, *bn_b;
     int relu, write_f32, write_codes;
     float next_sf;
-    int next_bits, next_terms, next_fastdiv;
+    int next_bits, next_terms, next_enc, next_fastdiv;
 };
 
 template <int COUT, int STRIDE, bool FAST>
@@ -347,7 +347,7 @@ first_conv3x3_kernel(const float *__restrict__ x, const float *__restrict__ wgt,
     for (int i = threadIdx.x; i < 27 * COUT; i += 256) sw[i] = wgt[i];
     if (p.write_codes) {
         for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += 256) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), TQ_ENC_HESE, p.next_terms);
+            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
             lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
         }
     }
@@ -434,12 +434,13 @@ first_conv3x3_kernel(const float *__restrict__ x, const float *__restrict__ wgt,
     }
 }
 
-static int fill_quant(DwParams &p, void *out_codes, float next_sf, int next_bits, int next_terms)
+static int fill_quant(DwParams &p, void *out_codes, float next_sf, int next_bits, int next_terms, int next_enc)
 {
     p.write_codes = out_codes ? 1 : 0;
     p.next_sf = out_codes ? next_sf : 1.0f;
     p.next_bits = out_codes ? next_bits : 1;
     p.next_terms = next_terms;
+    p.next_enc = next_enc;
     if (out_codes) {
         if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
         // codes are stored as fp16: |code| <= 2^bits must stay exactly representable
@@ -458,6 +459,16 @@ extern "C" int tq_depthwise3x3_codes(const void *act_codes, const int32_t *wgt_c
                                      int stride, float scale, int relu, int act_unsigned, float next_sf, int next_bits,
                                      int next_terms, void *stream)
 {
+    return tq_depthwise3x3_codes_enc(act_codes, wgt_codes, out_f32, out_codes, bias, bn_a, bn_b, N, H, W, C, stride, scale,
+                                     relu, act_unsigned, next_sf, next_bits, next_terms, TQ_ENC_HESE, stream);
+}
+
+extern "C" int tq_depthwise3x3_codes_enc(const void *act_codes, const int32_t *wgt_codes, float *out_f32, void *out_codes,
+                                         const float *bias, const float *bn_a, const float *bn_b, int N, int H, int W, int C,
+                                         int stride, float scale, int relu, int act_unsigned, float next_sf, int next_bits,
+                                         int next_terms, int next_enc, void *stream)
+{
+    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
     if (!act_codes || !wgt_codes || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1 || C < 8 || C % 8) return fail(TQ_ERR_INVALID, "bad shape (C must be a multiple of 8)");
     if (stride != 1 && stride != 2) return fail(TQ_ERR_UNSUPPORTED, "depthwise 3x3: stride 1 or 2");
@@ -473,7 +484,7 @@ extern "C" int tq_depthwise3x3_codes(const void *act_codes, const int32_t *wgt_c
     p.Wo = (W + 2 - 3) / stride + 1;
     p.scale = scale; p.bias = bias; p.bn_a = bn_a; p.bn_b = bn_b; p.relu = relu;
     p.write_f32 = out_f32 ? 1 : 0;
-    int rc = fill_quant(p, out_codes, next_sf, next_bits, next_terms);
+    int rc = fill_quant(p, out_codes, next_sf, next_bits, next_terms, next_enc);
     if (rc != TQ_OK) return rc;
     // tile: TW a multiple of DW_PIX; small maps take small tiles (a 7x7 map in a 8x16 tile would idle 62 % of the lanes)
     DwTile tl{};
@@ -542,6 +553,15 @@ extern "C" int tq_bn_act_encode(const float *x, const float *bias, const float *
                                 void *out_codes, int64_t npix, int C, int relu, float next_sf, int next_bits, int next_terms,
                                 void *stream)
 {
+    return tq_bn_act_encode_enc(x, bias, bn_a, bn_b, out_f32, out_codes, npix, C, relu, next_sf, next_bits, next_terms,
+                                TQ_ENC_HESE, stream);
+}
+
+extern "C" int tq_bn_act_encode_enc(const float *x, const float *bias, const float *bn_a, const float *bn_b, float *out_f32,
+                                    void *out_codes, int64_t npix, int C, int relu, float next_sf, int next_bits,
+                                    int next_terms, int next_enc, void *stream)
+{
+    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
     if (!x || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (npix < 0 || C < 4 || C % 4) return fail(TQ_ERR_INVALID, "bad shape (C must be a multiple of 4)");
     if ((bn_a == nullptr) != (bn_b == nullptr)) return fail(TQ_ERR_INVALID, "bn_a and bn_b go together");
@@ -551,7 +571,7 @@ extern "C" int tq_bn_act_encode(const float *x, const float *bias, const float *
     if (npix == 0) return TQ_OK;
     DwParams p{};
     p.C = C; p.bias = bias; p.bn_a = bn_a; p.bn_b = bn_b; p.relu = relu; p.write_f32 = out_f32 ? 1 : 0;
-    int rc = fill_quant(p, out_codes, next_sf, next_bits, next_terms);
+    int rc = fill_quant(p, out_codes, next_sf, next_bits, next_terms, next_enc);
     if (rc != TQ_OK) return rc;
     const int64_t n4 = npix * (C / 4);
     int64_t blocks = (n4 + 255) / 256;
@@ -604,6 +624,16 @@ extern "C" int tq_first_conv3x3_fused(const float *x, const float *wgt, const fl
                                       float *out_f32, void *out_codes, int N, int H, int W, int Cout, int stride, int relu,
                                       float next_sf, int next_bits, int next_terms, void *stream)
 {
+    return tq_first_conv3x3_fused_enc(x, wgt, bias, bn_a, bn_b, out_f32, out_codes, N, H, W, Cout, stride, relu, next_sf,
+                                      next_bits, next_terms, TQ_ENC_HESE, stream);
+}
+
+extern "C" int tq_first_conv3x3_fused_enc(const float *x, const float *wgt, const float *bias, const float *bn_a,
+                                          const float *bn_b, float *out_f32, void *out_codes, int N, int H, int W, int Cout,
+                                          int stride, int relu, float next_sf, int next_bits, int next_terms, int next_enc,
+                                          void *stream)
+{
+    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
     if (!x || !wgt || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1) return fail(TQ_ERR_INVALID, "bad shape");
     if (Cout != 32 && Cout != 64) return fail(TQ_ERR_UNSUPPORTED, "first conv: Cout must be 32 or 64, got %d", Cout);
@@ -617,9 +647,10 @@ extern "C" int tq_first_conv3x3_fused(const float *x, const float *wgt, const fl
     p.Ho = (H + 2 - 3) / stride + 1; p.Wo = (W + 2 - 3) / stride + 1;                // pad 1
     p.bias = bias; p.bn_a = bn_a; p.bn_b = bn_b; p.relu = relu; p.write_f32 = out_f32 ? 1 : 0;
     DwParams q{};
-    int rc = fill_quant(q, out_codes, next_sf, next_bits, next_terms);
+    int rc = fill_quant(q, out_codes, next_sf, next_bits, next_terms, next_enc);
     if (rc != TQ_OK) return rc;
-    p.write_codes = q.write_codes; p.next_sf = q.next_sf; p.next_bits = q.next_bits; p.next_terms = q.next_terms; p.next_fastdiv = q.next_fastdiv;
+    p.write_codes = q.write_codes; p.next_sf = q.next_sf; p.next_bits = q.next_bits; p.next_terms = q.next_terms;
+    p.next_enc = q.next_enc; p.next_fastdiv = q.next_fastdiv;
     cudaStream_t s = (cudaStream_t)stream;
     if (Cout == 64) return stride == 1 ? launch_first_conv<64, 1>(x, wgt, out_f32, out_codes, p, s) : launch_first_conv<64, 2>(x, wgt, out_f32, out_codes, p, s);
     return stride == 1 ? launch_first_conv<32, 1>(x, wgt, out_f32, out_codes, p, s) : launch_first_conv<32, 2>(x, wgt, out_f32, out_codes, p, s);

@@ -108,7 +108,7 @@ struct ConvGeom {
     const float *bias, *bn_a, *bn_b, *residual;
     int relu, relu6, write_f32, write_codes;    // relu6: additionally clamp at 6 (ReLU6 of the depthwise CNNs)
     float next_sf;
-    int next_bits, next_terms, next_fastdiv;
+    int next_bits, next_terms, next_enc, next_fastdiv;
 };
 
 // ---- PTX wrappers ---------------------------------------------------------------------------
@@ -488,7 +488,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     if (g.write_codes) {
         // (q, sign) -> fp16 term code of the consumer's quantiser, as in tr_elem_kernel
         for (uint32_t i = threadIdx.x; i < (2u << g.next_bits); i += GM_THREADS) {
-            int code = elem_code(i & ((1u << g.next_bits) - 1u), TQ_ENC_HESE, g.next_terms);
+            int code = elem_code(i & ((1u << g.next_bits) - 1u), g.next_enc, g.next_terms);
             lut[i] = __int2half_rn((i >> g.next_bits) ? -code : code);
         }
     }
@@ -1470,7 +1470,7 @@ static int launch_variant(ConvVariant v, const CUtensorMap &tmA, const CUtensorM
 // as long as the caller reuses the same buffers, and any other argument tuple simply plans again.
 struct ConvArgs {
     const void *act, *wgt, *out_f32, *out_codes, *bias, *bn_a, *bn_b, *residual;
-    int kind, N, H, W, C, Cout, R, S, stride, pad, relu, next_bits, next_terms, acc_groups, planes_a, planes_w, device;
+    int kind, N, H, W, C, Cout, R, S, stride, pad, relu, next_bits, next_terms, next_enc, acc_groups, planes_a, planes_w, device;
     float scale, next_sf;
 };
 struct ConvPlan {
@@ -1544,6 +1544,7 @@ static int plan_conv(const ConvArgs &a, ConvPlan &pl)
     g.next_sf = a.out_codes ? a.next_sf : 1.0f;
     g.next_bits = a.out_codes ? a.next_bits : 1;
     g.next_terms = a.next_terms;
+    g.next_enc = a.next_enc;
     g.next_fastdiv = (g.next_sf >= 9.313225746154785e-10f && g.next_sf <= 1073741824.0f) ? 1 : 0;
     // accumulator groups
     if (kind == 1) {
@@ -1691,8 +1692,10 @@ static int run_conv(ConvArgs &a, cudaStream_t s)
 
 static int check_conv_args(const void *act, const void *wgt, const void *out_f32, const void *out_codes, const void *bias,
                            const void *bn_a, const void *bn_b, const void *residual, int N, int H, int W, int C, int Cout,
-                           int R, int S, int stride, int pad, float next_sf, int next_bits, int next_terms, int c_align)
+                           int R, int S, int stride, int pad, float next_sf, int next_bits, int next_terms, int next_enc,
+                           int c_align)
 {
+    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
     if (!act || !wgt || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1 || C < 1 || Cout < 1 || R < 1 || S < 1 || stride < 1 || pad < 0)
         return fail(TQ_ERR_INVALID, "bad convolution geometry");
@@ -1724,8 +1727,18 @@ extern "C" int tq_conv2d_codes_fused(const void *act, const void *wgt, float *ou
                                      int stride, int pad, float scale, int relu, float next_sf, int next_bits,
                                      int next_terms, int acc_groups, void *stream)
 {
+    return tq_conv2d_codes_fused_enc(act, wgt, out_f32, out_codes, bias, bn_a, bn_b, residual, N, H, W, C, Cout, R, S, stride,
+                                     pad, scale, relu, next_sf, next_bits, next_terms, TQ_ENC_HESE, acc_groups, stream);
+}
+
+extern "C" int tq_conv2d_codes_fused_enc(const void *act, const void *wgt, float *out_f32, void *out_codes,
+                                         const float *bias, const float *bn_a, const float *bn_b,
+                                         const float *residual, int N, int H, int W, int C, int Cout, int R, int S,
+                                         int stride, int pad, float scale, int relu, float next_sf, int next_bits,
+                                         int next_terms, int next_enc, int acc_groups, void *stream)
+{
     int rc = check_conv_args(act, wgt, out_f32, out_codes, bias, bn_a, bn_b, residual, N, H, W, C, Cout, R, S, stride, pad,
-                             next_sf, next_bits, next_terms, 8);
+                             next_sf, next_bits, next_terms, next_enc, 8);
     if (rc != TQ_OK) return rc;
     ConvArgs a;
     memset(&a, 0, sizeof(a));                       // (padding bytes take part in the cache key)
@@ -1733,6 +1746,7 @@ extern "C" int tq_conv2d_codes_fused(const void *act, const void *wgt, float *ou
     a.residual = residual;
     a.kind = 0; a.N = N; a.H = H; a.W = W; a.C = C; a.Cout = Cout; a.R = R; a.S = S; a.stride = stride; a.pad = pad;
     a.relu = relu == 2 ? 2 : (relu ? 1 : 0); a.next_bits = out_codes ? next_bits : 1; a.next_terms = next_terms;
+    a.next_enc = next_enc;
     a.acc_groups = acc_groups < 1 ? 1 : acc_groups; a.planes_a = 1; a.planes_w = 1;
     a.scale = scale; a.next_sf = out_codes ? next_sf : 1.0f;
     return run_conv(a, (cudaStream_t)stream);
@@ -1753,8 +1767,19 @@ extern "C" int tq_conv2d_planes_i8(const void *act_planes, const void *wgt_plane
                                    int R, int S, int stride, int pad, float scale, int relu, float next_sf,
                                    int next_bits, int next_terms, int act_max, int wgt_max, void *stream)
 {
+    return tq_conv2d_planes_i8_enc(act_planes, wgt_planes, planes_a, planes_w, out_f32, out_codes, bias, bn_a, bn_b, residual,
+                                   N, H, W, C, Cout, R, S, stride, pad, scale, relu, next_sf, next_bits, next_terms,
+                                   TQ_ENC_HESE, act_max, wgt_max, stream);
+}
+
+extern "C" int tq_conv2d_planes_i8_enc(const void *act_planes, const void *wgt_planes, int planes_a, int planes_w,
+                                       float *out_f32, void *out_codes, const float *bias, const float *bn_a,
+                                       const float *bn_b, const float *residual, int N, int H, int W, int C, int Cout,
+                                       int R, int S, int stride, int pad, float scale, int relu, float next_sf,
+                                       int next_bits, int next_terms, int next_enc, int act_max, int wgt_max, void *stream)
+{
     int rc = check_conv_args(act_planes, wgt_planes, out_f32, out_codes, bias, bn_a, bn_b, residual, N, H, W, C, Cout, R, S,
-                             stride, pad, next_sf, next_bits, next_terms, 16);
+                             stride, pad, next_sf, next_bits, next_terms, next_enc, 16);
     if (rc != TQ_OK) return rc;
     if (planes_a < 1 || planes_a > 2 || planes_w < 1 || planes_w > 2) return fail(TQ_ERR_INVALID, "1 or 2 planes per operand");
     // int32 accumulators: |acc| <= K * act_max * wgt_max (the caller's bounds on |code|: 2^bits by construction of the
@@ -1770,6 +1795,7 @@ extern "C" int tq_conv2d_planes_i8(const void *act_planes, const void *wgt_plane
     a.bn_b = bn_b; a.residual = residual;
     a.kind = 1; a.N = N; a.H = H; a.W = W; a.C = C; a.Cout = Cout; a.R = R; a.S = S; a.stride = stride; a.pad = pad;
     a.relu = relu == 2 ? 2 : (relu ? 1 : 0); a.next_bits = out_codes ? next_bits : 1; a.next_terms = next_terms;
+    a.next_enc = next_enc;
     a.acc_groups = 1; a.planes_a = planes_a; a.planes_w = planes_w;
     a.scale = scale; a.next_sf = out_codes ? next_sf : 1.0f;
     return run_conv(a, (cudaStream_t)stream);
@@ -1935,9 +1961,10 @@ constexpr int STEM_U8 = 100;
 // max of conv columns 2q-1, 2q, 2q+1 of every conv row (fp32 [N, H/2, Wp, Cout]), the horizontal half of the pool.
 static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w2, float *out, void *out_codes,
                      const float *bn_a, const float *bn_b, int relu, int pool, float next_sf, int next_bits,
-                     int next_terms, int N, int H, int W, int Cout, void *stream, const float *mean3 = nullptr,
+                     int next_terms, int next_enc, int N, int H, int W, int Cout, void *stream, const float *mean3 = nullptr,
                      const float *std3 = nullptr)
 {
+    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
     if (!x || !x2_scratch || !w2 || !out) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (x_dtype != TQ_F32 && x_dtype != TQ_BF16 && x_dtype != TQ_F16 && x_dtype != STEM_U8)
         return fail(TQ_ERR_UNSUPPORTED, "stem conv input must be fp32, bf16, fp16 or uint8");
@@ -2023,6 +2050,7 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
     g.n_tiles = (Cout + block_n - 1) / block_n;
     g.write_f32 = 1;
     g.next_sf = out_codes ? next_sf : 1.0f; g.next_bits = out_codes ? next_bits : 1; g.next_terms = next_terms;
+    g.next_enc = next_enc;
     g.next_fastdiv = (g.next_sf >= 9.313225746154785e-10f && g.next_sf <= 1073741824.0f) ? 1 : 0;
     // program: per image plane (x_hi, and x_lo for fp32 images) ONE halo load covering the four folded filter rows; per
     // filter row R one N = 128 MMA group against the resident tile R = [w_hi (rows 0..63) ; w_lo (rows 64..127)]: columns
@@ -2088,7 +2116,7 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
 extern "C" int tq_stem_conv7x7s2_dt(const void *x, int x_dtype, void *x2_scratch, const void *w2, float *out,
                                     int N, int H, int W, int Cout, void *stream)
 {
-    return stem_impl(x, x_dtype, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 0, 1.0f, 1, 0, N, H, W, Cout, stream);
+    return stem_impl(x, x_dtype, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 0, 1.0f, 1, 0, TQ_ENC_HESE, N, H, W, Cout, stream);
 }
 
 extern "C" int tq_stem_conv7x7s2_pool(const void *x, int x_dtype, void *x2_scratch, const void *w2,
@@ -2096,30 +2124,39 @@ extern "C" int tq_stem_conv7x7s2_pool(const void *x, int x_dtype, void *x2_scrat
                                       int N, int H, int W, int Cout, float next_sf, int next_bits, int next_terms,
                                       void *stream)
 {
+    return tq_stem_conv7x7s2_pool_enc(x, x_dtype, x2_scratch, w2, bn_a, bn_b, relu, out, out_codes, N, H, W, Cout, next_sf,
+                                      next_bits, next_terms, TQ_ENC_HESE, stream);
+}
+
+extern "C" int tq_stem_conv7x7s2_pool_enc(const void *x, int x_dtype, void *x2_scratch, const void *w2,
+                                          const float *bn_a, const float *bn_b, int relu, float *out, void *out_codes,
+                                          int N, int H, int W, int Cout, float next_sf, int next_bits, int next_terms,
+                                          int next_enc, void *stream)
+{
     if (!bn_a || !bn_b) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (Cout % 8) return fail(TQ_ERR_UNSUPPORTED, "Cout must be a multiple of 8");
     if ((((uintptr_t)bn_a | (uintptr_t)bn_b | (uintptr_t)out_codes) & 15u) != 0) return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
     return stem_impl(x, x_dtype, x2_scratch, w2, out, out_codes, bn_a, bn_b, relu, 1, next_sf, next_bits, next_terms,
-                     N, H, W, Cout, stream);
+                     next_enc, N, H, W, Cout, stream);
 }
 
 extern "C" int tq_stem_conv7x7s2_u8(const void *x_u8, const float *mean3, const float *std3, void *x2_scratch, const void *w2,
                                     float *out, int N, int H, int W, int Cout, void *stream)
 {
-    return stem_impl(x_u8, STEM_U8, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 0, 1.0f, 1, 0, N, H, W, Cout, stream,
+    return stem_impl(x_u8, STEM_U8, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 0, 1.0f, 1, 0, TQ_ENC_HESE, N, H, W, Cout, stream,
                      mean3, std3);
 }
 
 extern "C" int tq_stem_conv7x7s2_rowmax(const void *x, int x_dtype, void *x2_scratch, const void *w2, float *out,
                                         int N, int H, int W, int Cout, void *stream)
 {
-    return stem_impl(x, x_dtype, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 2, 1.0f, 1, 0, N, H, W, Cout, stream);
+    return stem_impl(x, x_dtype, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 2, 1.0f, 1, 0, TQ_ENC_HESE, N, H, W, Cout, stream);
 }
 
 extern "C" int tq_stem_conv7x7s2_u8_rowmax(const void *x_u8, const float *mean3, const float *std3, void *x2_scratch,
                                            const void *w2, float *out, int N, int H, int W, int Cout, void *stream)
 {
-    return stem_impl(x_u8, STEM_U8, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 2, 1.0f, 1, 0, N, H, W, Cout, stream,
+    return stem_impl(x_u8, STEM_U8, x2_scratch, w2, out, nullptr, nullptr, nullptr, 0, 2, 1.0f, 1, 0, TQ_ENC_HESE, N, H, W, Cout, stream,
                      mean3, std3);
 }
 

@@ -22,7 +22,7 @@ struct PoolParams {
     int N, H, W, C, Ho, Wo;
     int relu;
     float next_sf;
-    int next_bits, next_terms, next_fastdiv, write_codes;
+    int next_bits, next_terms, next_enc, next_fastdiv, write_codes;
 };
 
 __global__ void __launch_bounds__(256)
@@ -33,7 +33,7 @@ bn_relu_maxpool3x3s2_kernel(const float *__restrict__ x, const float *__restrict
     extern __shared__ __half lut[];
     if (p.write_codes) {
         for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), TQ_ENC_HESE, p.next_terms);
+            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
             lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
         }
         __syncthreads();
@@ -111,7 +111,7 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
     uint64_t *full = reinterpret_cast<uint64_t *>(base + PT_STAGES * PT_STAGE_BYTES + (((size_t)(2u << p.next_bits) * 2 + 15) & ~(size_t)15));
     if (p.write_codes) {
         for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), TQ_ENC_HESE, p.next_terms);
+            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
             lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
         }
     }
@@ -217,9 +217,10 @@ namespace {
 
 // the checks and parameters both entry points share; Ho = pooled rows, Wo = pooled columns
 int pool_params(PoolParams &p, const float *x, const float *bn_a, const float *bn_b, float *out, void *out_codes, int N,
-                int H, int W, int C, int Wo, int relu, float next_sf, int next_bits, int next_terms)
+                int H, int W, int C, int Wo, int relu, float next_sf, int next_bits, int next_terms, int next_enc)
 {
     if (!x || !bn_a || !bn_b || !out) return fail(TQ_ERR_INVALID, "NULL pointer");
+    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
     if (N < 1 || H < 1 || W < 1 || C < 4 || C % 4) return fail(TQ_ERR_INVALID, "bad shape (C must be a multiple of 4)");
     if ((((uintptr_t)x | (uintptr_t)bn_a | (uintptr_t)bn_b | (uintptr_t)out | (uintptr_t)out_codes) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
@@ -232,6 +233,7 @@ int pool_params(PoolParams &p, const float *x, const float *bn_a, const float *b
     p.next_sf = out_codes ? next_sf : 1.0f;
     p.next_bits = out_codes ? next_bits : 1;
     p.next_terms = next_terms;
+    p.next_enc = next_enc;
     if (out_codes) {
         if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
         // codes are stored as fp16: |code| <= 2^bits must stay exactly representable (11-bit significand)
@@ -275,12 +277,13 @@ int launch_tiled(EncodeTiledFn enc, const float *x, const float *bn_a, const flo
 
 }  // namespace
 
-extern "C" int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, const float *bn_b, float *out,
-                                         void *out_codes, int N, int H, int W, int C, int relu,
-                                         float next_sf, int next_bits, int next_terms, void *stream)
+extern "C" int tq_bn_relu_maxpool_encode_enc(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                             void *out_codes, int N, int H, int W, int C, int relu,
+                                             float next_sf, int next_bits, int next_terms, int next_enc, void *stream)
 {
     PoolParams p;
-    int rc = pool_params(p, x, bn_a, bn_b, out, out_codes, N, H, W, C, (W + 2 - 3) / 2 + 1, relu, next_sf, next_bits, next_terms);
+    int rc = pool_params(p, x, bn_a, bn_b, out, out_codes, N, H, W, C, (W + 2 - 3) / 2 + 1, relu, next_sf, next_bits, next_terms,
+                         next_enc);
     if (rc != TQ_OK) return rc;
     // tiled TMA variant for 64-channel blocks on maps of at least one 4 x 14 tile; TQ_POOL_TILED=0 keeps the
     // one-thread-per-output kernel
@@ -300,17 +303,33 @@ extern "C" int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, cons
     return check_launch("bn_relu_maxpool3x3s2_kernel");
 }
 
-extern "C" int tq_bn_relu_maxpool_encode_rowmax(const float *x, const float *bn_a, const float *bn_b, float *out,
-                                                void *out_codes, int N, int H, int W, int C, int relu,
-                                                float next_sf, int next_bits, int next_terms, void *stream)
+extern "C" int tq_bn_relu_maxpool_encode(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                         void *out_codes, int N, int H, int W, int C, int relu,
+                                         float next_sf, int next_bits, int next_terms, void *stream)
+{
+    return tq_bn_relu_maxpool_encode_enc(x, bn_a, bn_b, out, out_codes, N, H, W, C, relu, next_sf, next_bits, next_terms,
+                                         TQ_ENC_HESE, stream);
+}
+
+extern "C" int tq_bn_relu_maxpool_encode_rowmax_enc(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                                    void *out_codes, int N, int H, int W, int C, int relu,
+                                                    float next_sf, int next_bits, int next_terms, int next_enc, void *stream)
 {
     // x: [N, H, W, C] row maxima (W = pooled columns); the vertical 3 / 2 / 1 window is all that is left
     PoolParams p;
-    int rc = pool_params(p, x, bn_a, bn_b, out, out_codes, N, H, W, C, W, relu, next_sf, next_bits, next_terms);
+    int rc = pool_params(p, x, bn_a, bn_b, out, out_codes, N, H, W, C, W, relu, next_sf, next_bits, next_terms, next_enc);
     if (rc != TQ_OK) return rc;
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
     return launch_tiled<1>(enc, x, bn_a, bn_b, out, out_codes, p, stream);
+}
+
+extern "C" int tq_bn_relu_maxpool_encode_rowmax(const float *x, const float *bn_a, const float *bn_b, float *out,
+                                                void *out_codes, int N, int H, int W, int C, int relu,
+                                                float next_sf, int next_bits, int next_terms, void *stream)
+{
+    return tq_bn_relu_maxpool_encode_rowmax_enc(x, bn_a, bn_b, out, out_codes, N, H, W, C, relu, next_sf, next_bits,
+                                                next_terms, TQ_ENC_HESE, stream);
 }
 
 

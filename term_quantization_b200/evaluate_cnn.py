@@ -24,7 +24,8 @@ def eval_model(args, model, val_loader, criterion, weight_bits, group_size, weig
                data_terms):
     tr_params = cnn_models.static_conv_layer_settings(model, weight_bits, group_size, weight_terms)
     avg_terms = compute_avg_terms(tr_params)
-    qmodel = cnn_models.convert_model(model, tr_params, data_bits, data_terms)
+    qmodel = cnn_models.convert_model(model, tr_params, data_bits, data_terms,
+                                      encoding=getattr(args, "encoding", "hese"))
     x = torch.zeros(1, 3, 224, 224, device=next(qmodel.parameters()).device)
     tmacs, params = profile_model.get_model_ops(qmodel, (x,))
     # profile ran one tracking-mode forward on zeros; restart the histograms before calibrating
@@ -78,6 +79,8 @@ def main(argv=None):
     parser.add_argument('--quick', action='store_true', help='one TR setting only')
     parser.add_argument('--engine', default='float', choices=['float', 'tcgen05', 'fused', 'auto'],
                         help='how the calibrated model runs (float = the reference path)')
+    parser.add_argument('--encoding', default='hese', choices=['hese', 'binary', 'booth'],
+                        help='term encoding of every wrapped layer (hese = the reference)')
     parser.add_argument('--out-file', default=None)
     args = parser.parse_args(argv)
     if not torch.cuda.is_available():

@@ -20,7 +20,7 @@ from .tr_layer import TRLinearLayer, TRLSTMLayer, set_tr_tracking
 NTOKENS = 33278
 
 
-def replace_lstm_layers(model, tr_params, data_bits, data_terms):
+def replace_lstm_layers(model, tr_params, data_bits, data_terms, *, encoding='hese'):
     targets = [(n, m) for n, m in model.named_modules() if isinstance(m, (nn.Linear, nn.LSTM))]
     for (name, layer), (weight_bits, group_size, weight_terms) in zip(targets, tr_params):
         cls = TRLSTMLayer if isinstance(layer, nn.LSTM) else TRLinearLayer
@@ -29,7 +29,7 @@ def replace_lstm_layers(model, tr_params, data_bits, data_terms):
         for k in keys[:-1]:
             parent = parent._modules[k]
         parent._modules[keys[-1]] = cls(layer, data_bits, data_terms, weight_bits, group_size,
-                                        weight_terms)
+                                        weight_terms, encoding=encoding)
     return model
 
 
@@ -38,8 +38,8 @@ def static_lstm_layer_settings(model, weight_bits, group_size, num_terms):
             for m in model.modules() if isinstance(m, (nn.Linear, nn.LSTM))]
 
 
-def convert_model(model, tr_params, data_bits, data_terms):
-    return replace_lstm_layers(deepcopy(model), tr_params, data_bits, data_terms)
+def convert_model(model, tr_params, data_bits, data_terms, *, encoding='hese'):
+    return replace_lstm_layers(deepcopy(model), tr_params, data_bits, data_terms, encoding=encoding)
 
 
 def repackage_hidden(h):
@@ -62,6 +62,8 @@ def main(argv=None):
         parser.add_argument(flag, nargs='+', type=int, help=what)
     parser.add_argument('--out-file', help='Output file')
     parser.add_argument('--eval-batch-size', type=int, default=10)
+    parser.add_argument('--encoding', default='hese', choices=['hese', 'binary', 'booth'],
+                        help='term encoding of every wrapped layer (hese = the reference)')
     parser.add_argument('--tokens', type=int, default=35 * 10 * 4 + 10, help='synthetic test tokens')
     args = parser.parse_args(argv)
     if not args.cuda or not torch.cuda.is_available():
@@ -95,7 +97,7 @@ def main(argv=None):
     results = {'ppls': [], 'tmacs': [], 'param_bits': []}
     for wb, wt, db, dt, gs in zip(args.wb, args.wt, args.db, args.dt, args.gs):
         tr_params = static_lstm_layer_settings(model, wb, gs, wt)
-        qmodel = convert_model(model, tr_params, db, dt)
+        qmodel = convert_model(model, tr_params, db, dt, encoding=args.encoding)
         evaluate(qmodel, test_data)                      # calibration pass
         set_tr_tracking(qmodel, False)
         loss = evaluate(qmodel, test_data)

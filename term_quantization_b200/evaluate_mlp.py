@@ -27,11 +27,11 @@ def _swap(model, name, new):
     parent._modules[keys[-1]] = new
 
 
-def replace_linear_layers(model, tr_params, data_bits, data_terms):
+def replace_linear_layers(model, tr_params, data_bits, data_terms, *, encoding='hese'):
     linears = [(n, m) for n, m in model.named_modules() if isinstance(m, nn.Linear)]
     for (name, layer), (weight_bits, group_size, weight_terms) in zip(linears, tr_params):
         _swap(model, name, TRLinearLayer(layer, data_bits, data_terms, weight_bits, group_size,
-                                         weight_terms))
+                                         weight_terms, encoding=encoding))
     return model
 
 
@@ -66,6 +66,8 @@ def main(argv=None):
     parser.add_argument('--synthetic', action='store_true', default=True)
     parser.add_argument('--samples', type=int, default=2048, help='synthetic test-set size')
     parser.add_argument('--weights', default=None, help='optional state_dict (.pt)')
+    parser.add_argument('--encoding', default='hese', choices=['hese', 'binary', 'booth'],
+                        help='term encoding of every wrapped layer (hese = the reference)')
     args = parser.parse_args(argv)
     if args.no_cuda or not torch.cuda.is_available():
         raise SystemExit("the TR op is CUDA-only (kernels/tr_cuda.cpp:12-18): no CPU path")
@@ -81,7 +83,7 @@ def main(argv=None):
     for wb, wt, db, dt, gs in zip(args.wb, args.wt, args.db, args.dt, args.gs):
         qmodel = deepcopy(model).to(device)
         tr_params = static_linear_layer_settings(qmodel, wb, gs, wt)
-        qmodel = replace_linear_layers(qmodel, tr_params, db, dt)
+        qmodel = replace_linear_layers(qmodel, tr_params, db, dt, encoding=args.encoding)
         test(args, qmodel, device, loader, pct=0.05)          # calibration pass
         set_tr_tracking(qmodel, False)
         acc = 100.0 * test(args, qmodel, device, loader)

@@ -34,8 +34,11 @@ def _bn_affine(bn):
 
 
 def _quant_key(layer):
+    """(sf, bits, terms) of a HESE quantiser, (sf, bits, terms, encoding) of any other: the `next_quant` of the fused
+    epilogues, and the key under which the executors keep the codes of one tensor per quantiser."""
     q = layer.input_quant
-    return (float(q.sf), int(q.data_bits), int(q.data_terms))
+    key = (float(q.sf), int(q.data_bits), int(q.data_terms))
+    return key if q.encoding == "hese" else key + (q.encoding,)
 
 
 class _Conv:
@@ -122,9 +125,9 @@ class FusedResNet(nn.Module):
 
     @staticmethod
     def _encode(x_nhwc, quant):
-        sf, bits, terms = quant
-        return tr_cuda.tr_codes(x_nhwc.view(1, -1, 1, 1), sf, bits, 1, terms,
-                                dtype=torch.float16).view(x_nhwc.shape)
+        sf, bits, terms = quant[:3]
+        return tr_cuda.tr_codes(x_nhwc.view(1, -1, 1, 1), sf, bits, 1, terms, dtype=torch.float16,
+                                encoding=quant[3] if len(quant) == 4 else "hese").view(x_nhwc.shape)
 
     def chain_description(self):
         """The fused chain as plain data (integer weight codes, fp32 scale, BatchNorm affine, quantiser per conv):
@@ -227,10 +230,10 @@ class FusedVGG(nn.Module):
     """Fused execution of a TQ-converted torchvision VGG (`features` = conv [-> BatchNorm] -> ReLU [-> MaxPool 2x2]
     chains; BASELINE.json configs[2]).  Every wrapped conv is one launch of the tcgen05 kernel with bias,
     BatchNorm affine and ReLU in the epilogue, emitting directly the fp16 term codes of the NEXT wrapped conv's
-    quantiser.  Max-pooling runs on those codes: for g = 1 the truncated-HESE code is a monotone non-decreasing
-    function of the (post-ReLU, non-negative) value, so maxpool(code(x)) == code(maxpool(x)) exactly and no fp32
-    activation is materialised between the first and the last conv (tests/test_oracle.py checks the monotonicity
-    exhaustively).  The first conv (never wrapped, cnn_models/__init__.py:34-36) stays on cuDNN fp32."""
+    quantiser.  Max-pooling runs on those codes: for g = 1 the truncated code of every encoding (HESE, binary, Booth) is
+    a monotone non-decreasing function of the (post-ReLU, non-negative) value, so maxpool(code(x)) == code(maxpool(x))
+    exactly and no fp32 activation is materialised between the first and the last conv (tests/test_oracle.py and
+    tests/test_encodings_host.py check the monotonicity exhaustively).  The first conv (never wrapped, cnn_models/__init__.py:34-36) stays on cuDNN fp32."""
 
     def __init__(self, model):
         super().__init__()

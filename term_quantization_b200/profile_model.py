@@ -3,7 +3,7 @@
 ops of a TR conv / linear = data_terms' * (alpha' / g) * MACs with data_terms' =
 min(data_terms, data_bits) and alpha' = min(alpha, weight_bits) when g == 1; convs are counted
 only for C_in > 3 and groups == 1 (profile_model.py:25); linear layers also count parameter
-bits -- numel * bits for g == 1, else the HESE-compressed size (device popcount reduction
+bits -- numel * bits for g == 1, else the compressed size in the layer's term encoding (device popcount reduction
 instead of the reference's per-element Python loop, tr_layer.py:57-63).  Counts land in the
 wrapped child's float32 buffer like the reference."""
 import torch
@@ -37,7 +37,7 @@ def tr_linear_ops(m, x, y):
     if m.group_size == 1:
         weight_bits = m.linear.weight.nelement() * m.weight_bits
     else:
-        weight_bits = tr_layer.compute_compressed_hese(m.linear.weight, m.w_sf, m.weight_bits)
+        weight_bits = tr_layer.compute_compressed_hese(m.linear.weight, m.w_sf, m.weight_bits, encoding=m.encoding)
     m.linear.total_params += torch.Tensor([int(weight_bits)])
 
 

@@ -17,8 +17,7 @@ _DTYPES = {torch.float32: _lib.TQ_F32, torch.float64: _lib.TQ_F64,
            torch.bfloat16: _lib.TQ_BF16, torch.float16: _lib.TQ_F16}
 _CODE_DTYPES = {torch.int8: _lib.TQ_I8, torch.int16: _lib.TQ_I16, torch.int32: _lib.TQ_I32,
                 torch.uint8: _lib.TQ_U8, torch.float16: _lib.TQ_F16C}
-_ENCODINGS = {"hese": _lib.ENC_HESE, "binary": _lib.ENC_BINARY, "booth": _lib.ENC_BOOTH,
-              0: 0, 1: 1, 2: 2}
+_ENCODINGS = {**_lib.ENCODINGS, 0: 0, 1: 1, 2: 2}
 
 
 def _check_input(input):

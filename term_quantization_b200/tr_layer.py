@@ -9,6 +9,10 @@ Same public names, constructor signatures and attributes:
     mse_profile(hist, minv, maxv, bit_width, terms)              tr_layer.py:43-54
     hese(number), compute_compressed_hese(w, sf, weight_terms)   tr_layer.py:9-41, 57-63
 
+Addition: every one of them except ``hese`` takes a keyword-only ``encoding`` ('hese', the
+reference's and the default, 'binary' or 'booth'): the term representation of a TR layer's
+weights and of its input quantiser, fixed for the layer's life.
+
 What changed underneath: every ``tr_cuda.tr`` call lands in the sm_100a kernels of
 libtq_b200.so; the tracking-mode ``torch.histc`` + add is one fused histogram pass; the
 calibration sweep (2048 launches + 2048 syncs per layer in the reference) is one fused kernel;
@@ -57,10 +61,11 @@ def hese(number):
     return out
 
 
-def mse_profile(hist, minv, maxv, bit_width, terms):
+def mse_profile(hist, minv, maxv, bit_width, terms, *, encoding="hese"):
     """Scale factor minimising the histogram-weighted squared error of g=1 term quantisation
     (tr_layer.py:43-54).  Same grid (linspace(minv, maxv, len(hist)) on the device), same 2048
     candidates, same first-minimum rule; one fused sweep on the device."""
+    enc = _lib.encoding_id(encoding)
     dev = hist.device if hist.is_cuda else torch.device("cuda")
     hist = hist.to(device=dev, dtype=torch.float32).contiguous()
     x = torch.linspace(minv, maxv, len(hist)).to(dev)
@@ -70,16 +75,18 @@ def mse_profile(hist, minv, maxv, bit_width, terms):
     errs = torch.empty(len(sfs), dtype=torch.float64, device=dev)
     argmin = torch.empty(1, dtype=torch.int32, device=dev)
     with torch.cuda.device(dev):
-        rc = _lib.lib().tq_mse_profile(hist.data_ptr(), x.data_ptr(), len(hist), sfs_d.data_ptr(),
-                                       len(sfs), int(bit_width), int(terms), errs.data_ptr(),
-                                       argmin.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        rc = _lib.lib().tq_mse_profile_enc(hist.data_ptr(), x.data_ptr(), len(hist), sfs_d.data_ptr(),
+                                           len(sfs), int(bit_width), int(terms), enc, errs.data_ptr(),
+                                           argmin.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
     _lib.check(rc)
     return sfs[int(argmin.item())]
 
 
-def compute_compressed_hese(w, sf, weight_terms):
+def compute_compressed_hese(w, sf, weight_terms, *, encoding="hese"):
     """Parameter bits of a HESE-compressed weight tensor (tr_layer.py:57-63):
-    (ceil(log2(weight_terms)) + 2) bits per surviving term."""
+    (ceil(log2(weight_terms)) + 2) bits per surviving term.  ``encoding`` counts the terms of
+    that encoding instead."""
+    enc = _lib.encoding_id(encoding)
     exp_bits = math.ceil(math.log2(weight_terms))
     bit_width = exp_bits + 2          # 1 for sign, 1 for barrier
     w = w.detach()
@@ -90,9 +97,9 @@ def compute_compressed_hese(w, sf, weight_terms):
     dt = {torch.float32: _lib.TQ_F32, torch.bfloat16: _lib.TQ_BF16}[w.dtype]
     with torch.cuda.device(w.device):
         # `w / sf` with a Python float on a CUDA tensor is w * (1/sf) inside torch
-        rc = _lib.lib().tq_hese_term_count(w.data_ptr(), dt, w.numel(), float(sf),
-                                           _lib.FLAG_RECIP_DIV, count.data_ptr(),
-                                           torch.cuda.current_stream(w.device).cuda_stream)
+        rc = _lib.lib().tq_term_count(w.data_ptr(), dt, w.numel(), float(sf), enc,
+                                      _lib.FLAG_RECIP_DIV, count.data_ptr(),
+                                      torch.cuda.current_stream(w.device).cuda_stream)
     _lib.check(rc)
     return bit_width * int(count.item())
 
@@ -136,10 +143,13 @@ def set_tr_tracking(model, tracking):
 class LinearQuantize(nn.Module):
     """Activation quantiser (tr_layer.py:78-104).  While ``tracking`` it accumulates an
     8192-bin histogram over [-50, 50] and passes the input through; afterwards it
-    term-reveals the flattened activation with g = 1 and ``data_terms`` terms per value."""
+    term-reveals the flattened activation with g = 1 and ``data_terms`` terms per value of
+    ``encoding``."""
 
-    def __init__(self, data_bits, data_terms):
+    def __init__(self, data_bits, data_terms, *, encoding="hese"):
         super().__init__()
+        _lib.encoding_id(encoding)
+        self.encoding = encoding
         self.sf = 1
         self.num_bins = 8192
         self.minv = -50
@@ -179,19 +189,22 @@ class LinearQuantize(nn.Module):
             return x
         dims = x.shape
         flat = x.contiguous().view(1, -1, 1, 1)          # tr_layer.py:97
-        flat = tr_cuda.tr(flat, self.sf, self.data_bits, 1, self.data_terms)
+        flat = tr_cuda.tr(flat, self.sf, self.data_bits, 1, self.data_terms, encoding=self.encoding)
         return flat.view(*dims)
 
     def finish_tracking(self):
-        self.sf = mse_profile(self.hist_bins, self.minv, self.maxv, self.data_bits, self.data_terms)
+        self.sf = mse_profile(self.hist_bins, self.minv, self.maxv, self.data_bits, self.data_terms,
+                              encoding=self.encoding)
         self.tracking = False
 
 
 class _TRBase(nn.Module):
-    def _setup(self, device, data_bits, data_terms, weight_bits, group_size, num_terms):
+    def _setup(self, device, data_bits, data_terms, weight_bits, group_size, num_terms, encoding):
+        _lib.encoding_id(encoding)
+        self.encoding = encoding
         self.data_bits = data_bits
         self.data_terms = data_terms
-        self.input_quant = LinearQuantize(data_bits, data_terms).to(device)
+        self.input_quant = LinearQuantize(data_bits, data_terms, encoding=encoding).to(device)
         self.group_size = group_size
         self.num_terms = num_terms
         self.weight_bits = weight_bits
@@ -201,7 +214,7 @@ class _TRBase(nn.Module):
         (tr_layer.py:117-121).  Sets self.w_sf, returns the new Parameter."""
         self.w_sf = w.abs().max().item() / 2 ** (self.weight_bits - 1)
         wq = tr_cuda.tr(w.detach().contiguous(), self.w_sf, self.weight_bits, self.group_size,
-                        self.num_terms)
+                        self.num_terms, encoding=self.encoding)
         return nn.Parameter(wq)
 
     def tracking(self, tracking):
@@ -222,10 +235,10 @@ class TRConv2dLayer(_TRBase):
     back as a channels_last fp32 tensor."""
 
     def __init__(self, conv_layer, data_bits=8, data_terms=4, weight_bits=8, group_size=1,
-                 num_terms=8):
+                 num_terms=8, *, encoding="hese"):
         super().__init__()
         self._setup(conv_layer.weight.device, data_bits, data_terms, weight_bits, group_size,
-                    num_terms)
+                    num_terms, encoding)
         conv_layer.weight = self._reveal_weight(conv_layer.weight)
         self.conv = conv_layer
         # packed operands of the tensor-core path: a NON-PERSISTENT buffer, so that .to(device) / .cuda() move it with
@@ -305,7 +318,7 @@ class TRConv2dLayer(_TRBase):
         q = self.input_quant
         x_nhwc = x.contiguous(memory_format=torch.channels_last).permute(0, 2, 3, 1)   # physical NHWC view
         codes = tr_cuda.tr_codes(x_nhwc.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms,
-                                 dtype=torch.float16).view(x_nhwc.shape)
+                                 dtype=torch.float16, encoding=q.encoding).view(x_nhwc.shape)
         sfx32 = torch.tensor(float(q.sf), dtype=torch.float32)
         scale = (sfx32 * torch.tensor(self._tc_wsf32, dtype=torch.float32)).item()   # fp32 product
         out = conv_codes.conv2d_codes(codes, self._tc_weight, c.bias, c.kernel_size, c.stride[0],
@@ -327,10 +340,10 @@ class TRLinearLayer(_TRBase):
     codes with the tcgen05 kernel (exact int32 accumulator, sf_x * w_sf and the bias in the epilogue)."""
 
     def __init__(self, linear_layer, data_bits=8, data_terms=4, weight_bits=8, group_size=1,
-                 num_terms=8):
+                 num_terms=8, *, encoding="hese"):
         super().__init__()
         self._setup(linear_layer.weight.device, data_bits, data_terms, weight_bits, group_size,
-                    num_terms)
+                    num_terms, encoding)
         linear_layer.weight = self._reveal_weight(linear_layer.weight)
         self.linear = linear_layer
         self.register_buffer("_tc_weight", None, persistent=False)
@@ -363,7 +376,8 @@ class TRLinearLayer(_TRBase):
         q = self.input_quant
         lead = x.shape[:-1]
         x2 = x.contiguous().view(-1, x.shape[-1])
-        codes = tr_cuda.tr_codes(x2.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16).view(x2.shape)
+        codes = tr_cuda.tr_codes(x2.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
+                                 encoding=q.encoding).view(x2.shape)
         scale = (torch.tensor(float(q.sf), dtype=torch.float32) * torch.tensor(self._tc_wsf32, dtype=torch.float32)).item()
         out = conv_codes.linear_codes(codes, self._tc_weight, scale, bias=self.linear.bias,
                                       out_features=self.linear.out_features, plan=self._tc_plan)
@@ -392,10 +406,10 @@ class TRLSTMLayer(_TRBase):
     evaluated step by step on that projection, and the remaining layers stay on cuDNN."""
 
     def __init__(self, lstm_layer, data_bits=8, data_terms=4, weight_bits=8, group_size=1,
-                 num_terms=8):
+                 num_terms=8, *, encoding="hese"):
         super().__init__()
         self._setup(lstm_layer.weight_ih_l0.device, data_bits, data_terms, weight_bits, group_size,
-                    num_terms)
+                    num_terms, encoding)
         lstm_layer.weight_ih_l0 = self._reveal_weight(lstm_layer.weight_ih_l0)
         self.w_sf_ih = self.w_sf                                                 # (w_sf itself ends up as hh's, like the reference)
         lstm_layer.weight_hh_l0 = self._reveal_weight(lstm_layer.weight_hh_l0)   # w_sf := hh's
@@ -430,7 +444,7 @@ class TRLSTMLayer(_TRBase):
         q = self.input_quant
         T, B, I = emb.shape
         codes = tr_cuda.tr_codes(emb.contiguous().view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms,
-                                 dtype=torch.float16).view(T * B, I)
+                                 dtype=torch.float16, encoding=q.encoding).view(T * B, I)
         scale = (torch.tensor(float(q.sf), dtype=torch.float32) * torch.tensor(self._tc_wsf32, dtype=torch.float32)).item()
         g = conv_codes.linear_codes(codes, self._tc_weight, scale, out_features=4 * self.lstm.hidden_size, plan=self._tc_plan)
         return g.view(T, B, -1)
