@@ -382,6 +382,22 @@ int tq_u8_normalize_bf16(const void *x_u8, void *y_bf16, int64_t npix, const flo
                          void *stream);
 
 /*
+ * The recurrence of one unidirectional LSTM layer (nn.LSTM, torch gate order i, f, g, o), all T steps in ONE launch of a
+ * persistent cooperative kernel (the step-wise loop tr_layer.py:174-195 runs as cuDNN calls, or as ~11 torch kernels per step):
+ *     gates = (gin[t] + bias) + h_{t-1} . w_hh^T;  c_t = sig(f) * c_{t-1} + sig(i) * tanh(g);  h_t = sig(o) * tanh(c_t)
+ *   gin  fp32 [T][B][4H], the input projection of every step (W_ih x_t, without bias)
+ *   bias fp32 [4H] (b_ih + b_hh) or NULL;  w_hh fp32 [4H][H] row-major (nn.LSTM's weight_hh_l*);  h0, c0 fp32 [B][H]
+ *   y    fp32 [T][B][H] = h_t;  hn, cn fp32 [B][H] = h_T, c_T
+ * fp32 FFMA with one fixed summation order per dot product (bit-identical from run to run), sig(x) = 1 / (1 + expf(-x)),
+ * accurate expf / tanhf.  Each CTA keeps the 4 gate rows of ceil(H / SMs) hidden units in shared memory; H is refused
+ * (TQ_ERR_UNSUPPORTED) when those rows and one hidden row exceed the device's opt-in shared memory per block (B200:
+ * H <= 1404).  All pointers 4-byte aligned, no output may alias an input; T, B, H >= 1.  The grid-wide barrier between steps
+ * relies on a cooperative launch, so the whole grid is resident by construction.
+ */
+int tq_lstm_recurrence(const float *gin, const float *bias, const float *w_hh, const float *h0, const float *c0,
+                       float *y, float *hn, float *cn, int T, int B, int H, void *stream);
+
+/*
  * Device self-test: quantises n pseudo-random (a, sf) pairs (sf in [2^-30, 2^30], a over all
  * non-negative floats and the quantiser's rounding boundaries) with the hoisted-reciprocal
  * divide and with div.rn.f32 and adds the number of disagreements to *mismatch (device).

@@ -511,3 +511,43 @@ def stem_conv_pool(x_nhwc, w2, bn, relu=True, next_quant=None, scratch=None):
             torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
     return out, codes, scratch
+
+
+def lstm_max_hidden(device=None):
+    """Largest hidden size tq_lstm_recurrence takes on `device`: each CTA keeps the 4 gate rows of ceil(H / SMs) units
+    in shared memory next to one hidden row and 2 KB of gate scratch (csrc/tq_lstm.cu, lstm_fits)."""
+    props = torch.cuda.get_device_properties(device if device is not None else torch.cuda.current_device())
+    sms, optin = props.multi_processor_count, props.shared_memory_per_block_optin
+    best = 0
+    for h in range(1, 65537):
+        if (4 * (-(-h // sms)) + 1) * h * 4 + 2048 <= optin:
+            best = h
+    return best
+
+
+def lstm_recurrence(gin, bias, w_hh, h0, c0):
+    """All T steps of one LSTM layer in one launch (tq_lstm_recurrence): gin fp32 [T, B, 4H] (W_ih x_t, torch gate order
+    i, f, g, o), bias fp32 [4H] (b_ih + b_hh) or None, w_hh fp32 [4H, H], h0 / c0 fp32 [B, H].
+    Returns (y [T, B, H], hn [B, H], cn [B, H]), fp32 with a fixed summation order."""
+    ts = [t for t in (gin, bias, w_hh, h0, c0) if t is not None]
+    if any(not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() for t in ts):
+        raise RuntimeError("lstm_recurrence expects contiguous fp32 CUDA tensors")
+    if any(t.device != gin.device for t in ts):
+        raise RuntimeError("lstm_recurrence: every tensor must be on the same device")
+    if gin.dim() != 3 or w_hh.dim() != 2:
+        raise RuntimeError("lstm_recurrence expects gin [T, B, 4H] and w_hh [4H, H]")
+    T, B, G = gin.shape
+    H = w_hh.shape[1]
+    if G != 4 * H or tuple(w_hh.shape) != (4 * H, H) or tuple(h0.shape) != (B, H) or tuple(c0.shape) != (B, H) \
+            or (bias is not None and tuple(bias.shape) != (4 * H,)):
+        raise RuntimeError(f"lstm_recurrence: shapes gin {tuple(gin.shape)}, w_hh {tuple(w_hh.shape)}, h0 {tuple(h0.shape)}, "
+                           f"c0 {tuple(c0.shape)}, bias {None if bias is None else tuple(bias.shape)} do not agree")
+    y = torch.empty((T, B, H), dtype=torch.float32, device=gin.device)
+    hn = torch.empty((B, H), dtype=torch.float32, device=gin.device)
+    cn = torch.empty((B, H), dtype=torch.float32, device=gin.device)
+    with torch.cuda.device(gin.device):
+        rc = _lib.lib().tq_lstm_recurrence(gin.data_ptr(), bias.data_ptr() if bias is not None else None, w_hh.data_ptr(),
+                                           h0.data_ptr(), c0.data_ptr(), y.data_ptr(), hn.data_ptr(), cn.data_ptr(),
+                                           T, B, H, torch.cuda.current_stream(gin.device).cuda_stream)
+    _lib.check(rc)
+    return y, hn, cn

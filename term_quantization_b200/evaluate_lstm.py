@@ -1,8 +1,11 @@
 """Wikitext-2 LSTM driver (mirror of evaluate_lstm.py:17-176): wrap nn.LSTM and the decoder
 Linear, calibrate on one pass, evaluate perplexity, count term-pair ops.
 
-Same flags (--wb --wt --db --dt --gs --out-file, model hyper-parameters).  The corpus
-(train.txt is missing, .MISSING_LARGE_BLOBS) and pretrained_models/lstm.pt are unavailable, so
+Same flags (--wb --wt --db --dt --gs --out-file, model hyper-parameters), plus --encoding and --engine:
+  float    the reference's forward (cuDNN LSTM on quantised emb / h0 / c0, fp32 decoder on the raw input)
+  tcgen05  tr_layer.use_tensor_cores: layer 0's input projection and the decoder's linear(q(x)) on term codes
+  fused    fused.FusedLSTM: the tcgen05 contractions plus one persistent recurrence kernel per layer
+The corpus (train.txt is missing, .MISSING_LARGE_BLOBS) and pretrained_models/lstm.pt are unavailable, so
 tokens are synthetic (uniform over the 33,278-word vocabulary) and weights random-init.
 `--tied/--cuda` keep the reference's inverted store_false behaviour (evaluate_lstm.py:77-82)."""
 import argparse
@@ -13,9 +16,9 @@ from copy import deepcopy
 import torch
 import torch.nn as nn
 
-from . import profile_model
+from . import fused, profile_model
 from .lstm_models.model import RNNModel
-from .tr_layer import TRLinearLayer, TRLSTMLayer, set_tr_tracking
+from .tr_layer import TRLinearLayer, TRLSTMLayer, set_tr_tracking, use_tensor_cores
 
 NTOKENS = 33278
 
@@ -64,6 +67,9 @@ def main(argv=None):
     parser.add_argument('--eval-batch-size', type=int, default=10)
     parser.add_argument('--encoding', default='hese', choices=['hese', 'binary', 'booth'],
                         help='term encoding of every wrapped layer (hese = the reference)')
+    parser.add_argument('--engine', default='float', choices=['float', 'tcgen05', 'fused'],
+                        help='float: the reference forward; tcgen05: input projection and decoder on term codes; '
+                             'fused: FusedLSTM (tcgen05 contractions, one recurrence kernel per layer)')
     parser.add_argument('--tokens', type=int, default=35 * 10 * 4 + 10, help='synthetic test tokens')
     args = parser.parse_args(argv)
     if not args.cuda or not torch.cuda.is_available():
@@ -85,7 +91,7 @@ def main(argv=None):
     def evaluate(m, source):
         m.eval()
         total = 0.
-        hidden = m.init_hidden(bsz)
+        hidden = model.init_hidden(bsz)
         with torch.no_grad():
             for i in range(0, source.size(0) - 1, args.bptt):
                 data, targets = get_batch(source, i)
@@ -100,7 +106,12 @@ def main(argv=None):
         qmodel = convert_model(model, tr_params, db, dt, encoding=args.encoding)
         evaluate(qmodel, test_data)                      # calibration pass
         set_tr_tracking(qmodel, False)
-        loss = evaluate(qmodel, test_data)
+        runner = qmodel
+        if args.engine == 'tcgen05':
+            use_tensor_cores(qmodel)
+        elif args.engine == 'fused':
+            runner = fused.FusedLSTM(qmodel)
+        loss = evaluate(runner, test_data)
         inputs = (get_batch(test_data, 0)[0], model.init_hidden(bsz))
         tmacs, param_bits = profile_model.get_model_ops(qmodel, inputs=inputs)
         ppl = math.exp(loss)

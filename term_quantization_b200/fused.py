@@ -487,3 +487,113 @@ class FusedMobileNet(nn.Module):
             capture["final"] = out
         y = out.permute(0, 3, 1, 2)
         return m.classifier(torch.flatten(nn.functional.adaptive_avg_pool2d(y, (1, 1)), 1))
+
+
+def _param_key(t):
+    return None if t is None else (t.data_ptr(), t._version, t.device)
+
+
+class FusedLSTM(nn.Module):
+    """Fused execution of a calibrated, TQ-converted RNNModel('LSTM', ...) (BASELINE.json configs[4]): an nn.Embedding
+    encoder, a TRLSTMLayer rnn and a TRLinearLayer decoder.  forward(input, hidden) -> (log_probs [T*B, ntoken], (hn, cn))
+    follows RNNModel.forward, so a bptt loop carries the hidden state across chunks unchanged.
+
+    Chain: embedding gather -> the rnn's shared quantiser on h0 / c0 -> layer 0's exact integer input projection on
+    tcgen05 (TRLSTMLayer.input_projection) -> tq_lstm_recurrence (all T steps in one persistent kernel) -> for every
+    upper layer an fp32 GEMM y . W_ih^T (torch.mm: true fp32 unless torch.backends.cuda.matmul.allow_tf32 is set; those
+    weights are not term-revealed, as in the reference) and the recurrence kernel -> the decoder's linear(q(y)) on term
+    codes (exact int32 accumulator, scale and bias in the epilogue) -> log_softmax.  Building the executor switches the rnn and decoder layers to their tensor-core paths (use_tensor_cores).
+    The recurrence is fp32 with a fixed summation order: bit-identical from run to run and under CUDA-graph replay, within
+    1e-5 of an fp64 recurrence, not bit-comparable with cuDNN or the step-wise loop of TRLSTMLayer."""
+
+    def __init__(self, model):
+        super().__init__()
+        rnn, dec = getattr(model, "rnn", None), getattr(model, "decoder", None)
+        if getattr(model, "rnn_type", None) != "LSTM" or not isinstance(rnn, tr_layer.TRLSTMLayer) \
+                or not isinstance(getattr(model, "encoder", None), nn.Embedding):
+            raise NotImplementedError("FusedLSTM expects a TQ-converted RNNModel('LSTM', ...): nn.Embedding encoder, "
+                                      "TRLSTMLayer rnn (GRU and vanilla RNN models are not supported)")
+        m = rnn.lstm
+        if type(m) is not nn.LSTM or m.bidirectional or m.batch_first or m.proj_size != 0:
+            raise NotImplementedError("FusedLSTM: unidirectional, time-major nn.LSTM without projections only "
+                                      f"(bidirectional={m.bidirectional}, batch_first={m.batch_first}, proj_size={m.proj_size})")
+        if not isinstance(dec, tr_layer.TRLinearLayer) or dec.linear.in_features != m.hidden_size:
+            raise NotImplementedError("FusedLSTM expects a TRLinearLayer decoder over the LSTM's hidden state")
+        for name, p in m.named_parameters():
+            if p.dtype != torch.float32 or not p.is_cuda:
+                raise NotImplementedError(f"FusedLSTM: fp32 CUDA parameters only ({name} is {p.dtype} on {p.device})")
+        hmax = conv_codes.lstm_max_hidden(m.weight_hh_l0.device)
+        if m.hidden_size > hmax:
+            raise NotImplementedError(f"FusedLSTM: hidden size {m.hidden_size} exceeds what the recurrence kernel keeps in "
+                                      f"shared memory on this device (H <= {hmax})")
+        if rnn.input_quant.tracking or dec.input_quant.tracking:
+            raise RuntimeError("calibrate the model (set_tr_tracking(model, False)) before fusing")
+        if model.training:
+            raise RuntimeError("FusedLSTM runs inference only: call model.eval() first")
+        dec.use_tensor_cores()                       # raises before any launch when the decoder's codes do not fit
+        rnn.use_tensor_cores()
+        self.model = model
+        self.layers = []                             # per layer: (w_ih or None for layer 0, w_hh, combined bias or None)
+        with torch.no_grad():
+            for l in range(m.num_layers):
+                bias = None
+                if m.bias:
+                    bias = (getattr(m, f"bias_ih_l{l}") + getattr(m, f"bias_hh_l{l}")).contiguous()
+                self.layers.append((None if l == 0 else getattr(m, f"weight_ih_l{l}"), getattr(m, f"weight_hh_l{l}"), bias))
+        self.dec_scale = (torch.tensor(float(dec.input_quant.sf), dtype=torch.float32)
+                          * torch.tensor(dec._tc_wsf32, dtype=torch.float32)).item()
+        self._key = self._snapshot()
+        self.train(False)
+
+    def _snapshot(self):
+        rnn, dec = self.model.rnn, self.model.decoder
+        return ([_param_key(p) for p in rnn.lstm.parameters()], _param_key(dec.linear.weight), _param_key(dec.linear.bias),
+                _param_key(self.model.encoder.weight), float(rnn.w_sf_ih), float(dec.w_sf), rnn._tc_weight, dec._tc_weight,
+                _quant_key(rnn), _quant_key(dec))
+
+    def check_fresh(self):
+        """Weights, packed operands and scale factors are snapshots: refuse stale ones (load_state_dict, in-place
+        updates, .to(device), re-calibration after fusing) and a model switched back to training or tracking."""
+        rnn, dec = self.model.rnn, self.model.decoder
+        if self.training or self.model.training:
+            raise RuntimeError("FusedLSTM runs inference only: call .eval() first")
+        if rnn.input_quant.tracking or dec.input_quant.tracking:
+            raise RuntimeError("the wrapped model is tracking (calibrating) again: finish the calibration and build the "
+                               "fused executor again")
+        key = self._snapshot()
+        if any(a is not b if isinstance(a, torch.Tensor) or isinstance(b, torch.Tensor) else a != b
+               for a, b in zip(key, self._key)):
+            raise RuntimeError("the wrapped model changed after fusing (weights, device or scale factors): "
+                               "build the fused executor again")
+
+    @torch.no_grad()
+    def forward(self, input, hidden, capture=None):
+        """input: int64 [T, B] tokens; hidden: (h0, c0) fp32 [layers, B, H].  capture: optional dict that receives 'y'
+        (the last layer's fp32 output [T, B, H]), 'codes' (the decoder's fp16 input codes [T*B, H]) and 'decoded' (the
+        decoder's fp32 output before log_softmax)."""
+        if not torch.cuda.is_current_stream_capturing():
+            self.check_fresh()
+        model = self.model
+        rnn, dec = model.rnn, model.decoder
+        emb = model.encoder(input)
+        h0, c0 = (rnn.input_quant(h) for h in hidden)                 # the shared quantiser (tr_layer.py:193-194)
+        T, B = input.shape
+        hn, cn = [], []
+        y = None
+        for l, (w_ih, w_hh, bias) in enumerate(self.layers):
+            if l == 0:
+                gin = rnn.input_projection(emb)
+            else:
+                gin = torch.mm(y.view(T * B, -1), w_ih.t()).view(T, B, -1)
+            y, h, c = conv_codes.lstm_recurrence(gin, bias, w_hh, h0[l].contiguous(), c0[l].contiguous())
+            hn.append(h)
+            cn.append(c)
+        q = dec.input_quant
+        H = y.shape[-1]
+        codes = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
+                                 encoding=q.encoding).view(T * B, H)
+        decoded = conv_codes.linear_codes(codes, dec._tc_weight, self.dec_scale, bias=dec.linear.bias,
+                                          out_features=dec.linear.out_features, plan=dec._tc_plan)
+        if capture is not None:
+            capture["y"], capture["codes"], capture["decoded"] = y, codes, decoded
+        return F.log_softmax(decoded, dim=1), (torch.stack(hn), torch.stack(cn))

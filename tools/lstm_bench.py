@@ -1,0 +1,196 @@
+"""The Wikitext-2 LSTM workload of bench_extra.py (configs[4]: 650/650, 2 layers, vocab 33,278, seq 35 x batch 80; TQ wb 8,
+g 8, alpha 12, db 8, seed 0) on its three paths, timed as CUDA-graph replays in one process, alternating:
+
+  strict   the reference forward as shipped: cuDNN LSTM on quantised emb / h0 / c0, fp32 decoder on the raw input
+  tcgen05  tr_layer.use_tensor_cores: layer-0 input projection and decoder on term codes, step-wise layer 0, cuDNN layer 1
+  fused    fused.FusedLSTM: the same contractions, every layer's recurrence one persistent kernel (tq_lstm_recurrence)
+
+Then a separate eager pass splits the fused forward into phases with CUDA events, and the recurrence kernel's FFMA rate
+is set against a DERIVED fp32 rate (SMs x 128 FMA/clk x the max SM clock nvidia-smi reports; not a measured peak).
+Writes DIR/lstm_bench.json.  Usage: python tools/lstm_bench.py --out DIR [--rounds 15] [--replays 20]"""
+import argparse
+import copy
+import json
+import os
+import statistics
+import subprocess
+import sys
+
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+from term_quantization_b200 import conv_codes, evaluate_lstm, fused, tr_cuda, tr_layer  # noqa: E402
+from term_quantization_b200.lstm_models.model import RNNModel  # noqa: E402
+
+T, B, H = 35, 80, 650
+
+
+def gpu_info():
+    q = "name,power.limit,clocks.max.sm"
+    try:
+        line = subprocess.run(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader,nounits", "-i", "0"],
+                              capture_output=True, text=True, check=True, timeout=60).stdout.strip().splitlines()[0]
+        name, power, clock = (v.strip() for v in line.split(","))
+        return {"name": name, "power_limit_w": float(power), "max_sm_clock_mhz": float(clock)}
+    except Exception as e:                                   # reported, never guessed
+        return {"error": f"nvidia-smi query failed: {e}"}
+
+
+def capture(fn):
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        for _ in range(3):
+            fn()
+    torch.cuda.current_stream().wait_stream(side)
+    torch.cuda.synchronize()
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        out = fn()
+    return graph, out
+
+
+def time_replays(graph, n):
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(n):
+        graph.replay()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / n
+
+
+def phases(f, tokens, hidden, reps):
+    """Eager fused forward split by CUDA events: the same calls FusedLSTM.forward makes, one event between phases."""
+    model = f.model
+    rnn, dec = model.rnn, model.decoder
+    names = []
+    times = {}
+
+    def run():
+        ev = [torch.cuda.Event(enable_timing=True)]
+        ev[0].record()
+        labels = []
+
+        def mark(name):
+            e = torch.cuda.Event(enable_timing=True)
+            e.record()
+            ev.append(e)
+            labels.append(name)
+        emb = model.encoder(tokens)
+        h0, c0 = (rnn.input_quant(h) for h in hidden)
+        mark("embedding + h0/c0 quantiser")
+        y = None
+        for l, (w_ih, w_hh, bias) in enumerate(f.layers):
+            if l == 0:
+                gin = rnn.input_projection(emb)
+                mark("layer 0 input projection (tcgen05, term codes)")
+            else:
+                gin = torch.mm(y.view(T * B, -1), w_ih.t()).view(T, B, -1)
+                mark(f"layer {l} input GEMM (fp32)")
+            y, _, _ = conv_codes.lstm_recurrence(gin, bias, w_hh, h0[l].contiguous(), c0[l].contiguous())
+            mark(f"layer {l} recurrence (tq_lstm_recurrence)")
+        q = dec.input_quant
+        codes = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
+                                 encoding=q.encoding).view(T * B, H)
+        decoded = conv_codes.linear_codes(codes, dec._tc_weight, f.dec_scale, bias=dec.linear.bias,
+                                          out_features=dec.linear.out_features, plan=dec._tc_plan)
+        mark("decoder: encode + linear on term codes (tcgen05)")
+        torch.log_softmax(decoded, dim=1)
+        mark("log_softmax")
+        torch.cuda.synchronize()
+        return labels, [ev[i].elapsed_time(ev[i + 1]) for i in range(len(labels))]
+
+    with torch.no_grad():
+        for _ in range(3):
+            run()
+        for _ in range(reps):
+            labels, ms = run()
+            names = labels
+            for k, v in zip(labels, ms):
+                times.setdefault(k, []).append(v)
+    return [{"phase": k, "ms_median": statistics.median(times[k]), "ms_best": min(times[k])} for k in names]
+
+
+def main(argv=None):
+    ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
+    ap.add_argument("--out", required=True, help="output directory (lstm_bench.json)")
+    ap.add_argument("--rounds", type=int, default=15, help="alternating rounds; each times every path once")
+    ap.add_argument("--replays", type=int, default=20, help="graph replays per timed sample")
+    args = ap.parse_args(argv)
+    if not torch.cuda.is_available():
+        raise SystemExit("lstm_bench needs a CUDA device: nothing is timed on the CPU")
+    os.makedirs(args.out, exist_ok=True)
+    torch.backends.cudnn.allow_tf32 = False
+    torch.backends.cuda.matmul.allow_tf32 = False
+    dev = torch.device("cuda")
+    info = gpu_info()
+    props = torch.cuda.get_device_properties(dev)
+
+    torch.manual_seed(0)
+    gen = torch.Generator(device=dev).manual_seed(0)
+    base = RNNModel('LSTM', evaluate_lstm.NTOKENS, 650, 650, 2, 0.5, True).to(dev).eval()
+    q = evaluate_lstm.convert_model(base, evaluate_lstm.static_lstm_layer_settings(base, 8, 8, 12), 8, 8)
+    tokens = torch.randint(evaluate_lstm.NTOKENS, (T, B), device=dev, generator=gen)
+    hidden = base.init_hidden(B)
+    with torch.no_grad():
+        q(tokens, hidden)
+        tr_layer.set_tr_tracking(q, False)
+        q_tc = copy.deepcopy(q)
+        tr_layer.use_tensor_cores(q_tc)
+        f = fused.FusedLSTM(copy.deepcopy(q))
+        paths = {"strict": lambda: q(tokens, hidden), "tcgen05": lambda: q_tc(tokens, hidden),
+                 "fused": lambda: f(tokens, hidden)}
+        graphs, outs, errors = {}, {}, {}
+        for name, fn in paths.items():
+            try:
+                graphs[name], outs[name] = capture(fn)
+            except Exception as e:                           # a refused capture is a result: report it
+                errors[name] = f"{type(e).__name__}: {e}"
+        samples = {k: [] for k in graphs}
+        for _ in range(args.rounds):
+            for name, g in graphs.items():
+                samples[name].append(time_replays(g, args.replays))
+        check = {}
+        if "fused" in outs and "tcgen05" in outs:
+            (lf, (hf, cf)), (lt, (ht, ct)) = outs["fused"], outs["tcgen05"]
+            check = {"hn_max_abs_diff": float((hf - ht).abs().max()), "cn_max_abs_diff": float((cf - ct).abs().max()),
+                     "log_probs_mean_abs_diff": float((lf - lt).abs().mean())}
+    per_phase = phases(f, tokens, hidden, reps=20)
+    rec = [p for p in per_phase if "recurrence" in p["phase"]]
+    fma = T * B * 4 * H * H
+    derived = None
+    if "max_sm_clock_mhz" in info:
+        derived = props.multi_processor_count * 128 * info["max_sm_clock_mhz"] * 1e6
+    recurrence = []
+    for p in rec:
+        rate = fma / (p["ms_median"] * 1e-3)
+        recurrence.append({"phase": p["phase"], "fma": fma, "ms_median": p["ms_median"], "fma_per_s": rate,
+                           "fp32_tflops": 2 * rate / 1e12,
+                           "share_of_derived_fp32_rate": rate / derived if derived else None})
+    res = {
+        "workload": "Wikitext-2-shaped LSTM 650/650 tied, 2 layers, vocab 33,278, seq 35 x batch 80, TQ wb 8 / g 8 / "
+                    "alpha 12 / db 8 (bench_extra.py configs[4]), seed 0",
+        "gpu": info, "sms": props.multi_processor_count, "shared_memory_per_block_optin": props.shared_memory_per_block_optin,
+        "lstm_max_hidden": conv_codes.lstm_max_hidden(dev),
+        "timed_as": f"CUDA-graph replays, {args.replays} per sample, {args.rounds} rounds alternating the paths; "
+                    "TF32 off",
+        "paths": {k: {"ms_best": min(v), "ms_median": statistics.median(v),
+                      "tokens_per_s_median": T * B / statistics.median(v) * 1e3} for k, v in samples.items()},
+        "capture_errors": errors,
+        "fused_vs_tcgen05": check,
+        "fused_phases_eager": per_phase,
+        "recurrence_kernel": recurrence,
+        "derived_fp32_fma_rate": {"fma_per_s": derived, "how": "SMs x 128 FP32 FMA/clk x max SM clock (derived, "
+                                                                "not a measured peak)"},
+    }
+    path = os.path.join(args.out, "lstm_bench.json")
+    with open(path, "w") as fp:
+        json.dump(res, fp, indent=1)
+    print(json.dumps(res, indent=1))
+
+
+if __name__ == "__main__":
+    main()
