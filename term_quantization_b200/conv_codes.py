@@ -38,14 +38,9 @@ def _quant_args(next_quant):
     return next_quant[0], next_quant[1], next_quant[2], enc
 
 
-def _entry(name, enc, at):
-    """The C entry point for a consumer quantiser in encoding `enc`, called with the arguments of `name`_enc: HESE goes
-    to the original entry point `name` (the encoding, argument `at`, dropped), any other encoding to the _enc twin."""
-    L = _lib.lib()
-    if enc != _lib.ENC_HESE:
-        return getattr(L, name + "_enc")
-    fn = getattr(L, name)
-    return lambda *args: fn(*args[:at], *args[at + 1:])
+def _ptr(t):
+    """Device address of an optional tensor argument (None: NULL)."""
+    return t.data_ptr() if t is not None else None
 
 
 def _relu_code(relu):
@@ -155,22 +150,21 @@ def _cached_plan(wgt, act_max, signed_act, engine):
 
 def _run_conv(act, plan, out, codes, bias, bn, residual, N, H, W, C, Cout, R, S, stride, pad, scale, relu, sf, bits,
               terms, enc, act_planes=None):
-    ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
     stream = torch.cuda.current_stream(act.device).cuda_stream
     with torch.cuda.device(act.device):
         if plan.engine == "f16":
-            rc = _entry("tq_conv2d_codes_fused", enc, 22)(
-                act.data_ptr(), plan.wgt.data_ptr(), ptr(out), ptr(codes), ptr(bias),
-                ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None, ptr(residual),
+            rc = _lib.lib().tq_conv2d_codes_fused_enc(
+                act.data_ptr(), plan.wgt.data_ptr(), _ptr(out), _ptr(codes), _ptr(bias),
+                _ptr(bn[0]) if bn else None, _ptr(bn[1]) if bn else None, _ptr(residual),
                 N, H, W, C, Cout, R, S, stride, pad, float(scale), _relu_code(relu), float(sf), int(bits),
                 int(terms), enc, int(plan.groups), stream)
         else:
             if act_planes is None:
                 pa = _planes_needed(plan.act_max)
                 act_planes, _ = codes_to_planes(act, pa)
-            rc = _entry("tq_conv2d_planes_i8", enc, 24)(
-                act_planes.data_ptr(), plan.planes.data_ptr(), act_planes.shape[0], plan.planes_w, ptr(out), ptr(codes),
-                ptr(bias), ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None, ptr(residual),
+            rc = _lib.lib().tq_conv2d_planes_i8_enc(
+                act_planes.data_ptr(), plan.planes.data_ptr(), act_planes.shape[0], plan.planes_w, _ptr(out), _ptr(codes),
+                _ptr(bias), _ptr(bn[0]) if bn else None, _ptr(bn[1]) if bn else None, _ptr(residual),
                 N, H, W, C, Cout, R, S, stride, pad, float(scale), _relu_code(relu), float(sf), int(bits), int(terms),
                 enc, int(plan.act_max), int(plan.wgt_max), stream)
     _lib.check(rc)
@@ -296,11 +290,10 @@ def depthwise3x3_codes(act, wgt, stride, scale, *, bias=None, bn=None, relu=Fals
     out = torch.empty((N, Ho, Wo, C), dtype=torch.float32, device=act.device) if want_f32 else None
     codes = torch.empty((N, Ho, Wo, C), dtype=torch.float16, device=act.device) if next_quant else None
     sf, bits, terms, enc = _quant_args(next_quant)
-    ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
     with torch.cuda.device(act.device):
-        rc = _entry("tq_depthwise3x3_codes", enc, 18)(
-            act.data_ptr(), wgt.data_ptr(), ptr(out), ptr(codes), ptr(bias), ptr(bn[0]) if bn else None,
-            ptr(bn[1]) if bn else None, N, H, W, C, stride, float(scale), _relu_code(relu), int(bool(act_unsigned)),
+        rc = _lib.lib().tq_depthwise3x3_codes_enc(
+            act.data_ptr(), wgt.data_ptr(), _ptr(out), _ptr(codes), _ptr(bias), _ptr(bn[0]) if bn else None,
+            _ptr(bn[1]) if bn else None, N, H, W, C, stride, float(scale), _relu_code(relu), int(bool(act_unsigned)),
             float(sf), int(bits), int(terms), enc, torch.cuda.current_stream(act.device).cuda_stream)
     _lib.check(rc)
     return out, codes
@@ -327,14 +320,13 @@ def first_conv3x3_fused(x_nhwc, w_packed, stride=1, bias=None, bn=None, relu=Fal
     if out is None and codes is None:
         raise RuntimeError("first_conv3x3_fused: nothing to compute (want_f32 or next_quant)")
     sf, bits, terms, enc = _quant_args(next_quant)
-    ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
     for t in (bias, bn[0] if bn else None, bn[1] if bn else None):
         if t is not None and (t.dtype != torch.float32 or t.numel() != Cout or not t.is_contiguous() or t.device != x_nhwc.device):
             raise RuntimeError("first_conv3x3_fused: bias / bn must be contiguous fp32 [Cout] tensors on the input's device")
     with torch.cuda.device(x_nhwc.device):
-        rc = _entry("tq_first_conv3x3_fused", enc, 16)(
-            x_nhwc.data_ptr(), w_packed.data_ptr(), ptr(bias), ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None,
-            ptr(out), ptr(codes), N, H, W, Cout, int(stride), _relu_code(relu), float(sf), int(bits), int(terms), enc,
+        rc = _lib.lib().tq_first_conv3x3_fused_enc(
+            x_nhwc.data_ptr(), w_packed.data_ptr(), _ptr(bias), _ptr(bn[0]) if bn else None, _ptr(bn[1]) if bn else None,
+            _ptr(out), _ptr(codes), N, H, W, Cout, int(stride), _relu_code(relu), float(sf), int(bits), int(terms), enc,
             torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
     return out, codes
@@ -365,12 +357,11 @@ def bn_act_encode(x_nhwc, bn=None, relu=False, want_f32=False, next_quant=None, 
     out = torch.empty_like(x_nhwc) if want_f32 else None
     codes = torch.empty(x_nhwc.shape, dtype=torch.float16, device=x_nhwc.device) if next_quant else None
     sf, bits, terms, enc = _quant_args(next_quant)
-    ptr = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
     with torch.cuda.device(x_nhwc.device):
         if bias is not None and (bias.dtype != torch.float32 or bias.numel() != C or not bias.is_contiguous() or bias.device != x_nhwc.device):
             raise RuntimeError("bn_act_encode: bias must be a contiguous fp32 [C] tensor on the input's device")
-        rc = _entry("tq_bn_act_encode", enc, 12)(
-            x_nhwc.data_ptr(), ptr(bias), ptr(bn[0]) if bn else None, ptr(bn[1]) if bn else None, ptr(out), ptr(codes),
+        rc = _lib.lib().tq_bn_act_encode_enc(
+            x_nhwc.data_ptr(), _ptr(bias), _ptr(bn[0]) if bn else None, _ptr(bn[1]) if bn else None, _ptr(out), _ptr(codes),
             x_nhwc.numel() // C, C, _relu_code(relu), float(sf), int(bits), int(terms), enc,
             torch.cuda.current_stream(x_nhwc.device).cuda_stream)
     _lib.check(rc)
@@ -389,7 +380,8 @@ def bn_relu_maxpool_encode(x_nhwc, bn, relu=True, next_quant=None, rowmax=False)
     out = torch.empty((N, Ho, Wo, C), dtype=torch.float32, device=x_nhwc.device)
     codes = torch.empty((N, Ho, Wo, C), dtype=torch.float16, device=x_nhwc.device) if next_quant else None
     sf, bits, terms, enc = _quant_args(next_quant)
-    fn = _entry("tq_bn_relu_maxpool_encode_rowmax" if rowmax else "tq_bn_relu_maxpool_encode", enc, 13)
+    L = _lib.lib()
+    fn = L.tq_bn_relu_maxpool_encode_rowmax_enc if rowmax else L.tq_bn_relu_maxpool_encode_enc
     with torch.cuda.device(x_nhwc.device):
         rc = fn(
             x_nhwc.data_ptr(), bn[0].data_ptr(), bn[1].data_ptr(), out.data_ptr(),
@@ -504,7 +496,7 @@ def stem_conv_pool(x_nhwc, w2, bn, relu=True, next_quant=None, scratch=None):
     codes = torch.empty((N, Hp, Wp, Cout), dtype=torch.float16, device=x_nhwc.device) if next_quant else None
     sf, bits, terms, enc = _quant_args(next_quant)
     with torch.cuda.device(x_nhwc.device):
-        rc = _entry("tq_stem_conv7x7s2_pool", enc, 16)(
+        rc = _lib.lib().tq_stem_conv7x7s2_pool_enc(
             x_nhwc.data_ptr(), _STEM_DTYPES[x_nhwc.dtype], scratch.data_ptr(), w2.data_ptr(),
             bn[0].data_ptr(), bn[1].data_ptr(), int(bool(relu)), out.data_ptr(),
             codes.data_ptr() if codes is not None else None, N, H, W, Cout, float(sf), int(bits), int(terms), enc,

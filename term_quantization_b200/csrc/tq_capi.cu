@@ -1,5 +1,5 @@
 // tq_capi.cu -- process-wide plumbing behind the C ABI (include/tq_b200.h):
-// thread-local error text, launch accounting, device properties.
+// thread-local error text, launch accounting, device properties, the fused encoders' quantiser check.
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
@@ -31,6 +31,25 @@ int check_encoding(int enc)
 {
     if (enc != TQ_ENC_HESE && enc != TQ_ENC_BINARY && enc != TQ_ENC_BOOTH)
         return fail(TQ_ERR_INVALID, "unknown term encoding %d (TQ_ENC_HESE, TQ_ENC_BINARY or TQ_ENC_BOOTH)", enc);
+    return TQ_OK;
+}
+
+int next_quant(NextQuant &q, const void *out_codes, float sf, int bits, int terms, int enc, int max_bits, bool need_fast)
+{
+    if (check_encoding(enc) != TQ_OK) return TQ_ERR_INVALID;
+    if (out_codes) {
+        if (!(sf > 0.0f) || !(sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
+        if (bits < 1 || bits > max_bits) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..%d bits", max_bits);
+        if (terms < 0) return fail(TQ_ERR_INVALID, "next_terms must be >= 0");
+        if (need_fast && !fast_div_ok(sf))
+            return fail(TQ_ERR_UNSUPPORTED, "fused encode needs 2^-30 <= next_sf <= 2^30 (got %g): encode with tq_tr_encode_codes instead", (double)sf);
+    }
+    q.write_codes = out_codes ? 1 : 0;
+    q.sf = out_codes ? sf : 1.0f;
+    q.bits = out_codes ? bits : 1;
+    q.terms = terms;
+    q.enc = enc;
+    q.fastdiv = fast_div_ok(q.sf) ? 1 : 0;
     return TQ_OK;
 }
 

@@ -36,9 +36,8 @@ struct DwParams {
     float scale;
     const float *bias, *bn_a, *bn_b;
     int relu;                   // 0 none, 1 ReLU, 2 ReLU6
-    int write_f32, write_codes;
-    float next_sf;
-    int next_bits, next_terms, next_enc, next_fastdiv;
+    int write_f32;
+    NextQuant nq;
 };
 
 // activation shared by the epilogues of this file
@@ -78,12 +77,12 @@ depthwise3x3_codes_kernel(const __grid_constant__ CUtensorMap tmIn, const int32_
     uint8_t *stage0 = base;                                                     // 2 x [in_h][in_w][64] fp16
     int32_t *sw = reinterpret_cast<int32_t *>(base + 2 * tl.stage_bytes);       // [9][C]
     __half *lut = reinterpret_cast<__half *>(sw + 9 * p.C);                     // (q, sign) -> code
-    uint64_t *full = reinterpret_cast<uint64_t *>(reinterpret_cast<uint8_t *>(lut) + (((size_t)(2u << p.next_bits) * 2 + 15) & ~(size_t)15));
+    uint64_t *full = reinterpret_cast<uint64_t *>(reinterpret_cast<uint8_t *>(lut) + code_table_bytes(p.nq.bits));
     for (int i = threadIdx.x; i < 9 * p.C; i += blockDim.x) sw[i] = wgt[i];
-    if (p.write_codes) {
-        for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
-            lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
+    if (p.nq.write_codes) {
+        for (uint32_t i = threadIdx.x; i < (2u << p.nq.bits); i += blockDim.x) {
+            const int code = elem_code(i & ((1u << p.nq.bits) - 1u), p.nq.enc, p.nq.terms);
+            lut[i] = __int2half_rn((i >> p.nq.bits) ? -code : code);
         }
     }
     if (threadIdx.x == 0) {
@@ -93,7 +92,7 @@ depthwise3x3_codes_kernel(const __grid_constant__ CUtensorMap tmIn, const int32_
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmIn) : "memory");
     }
     __syncthreads();
-    const Quant nq = make_quant(p.write_codes ? p.next_sf : 1.0f, (float)((1u << p.next_bits) - 1u));
+    const Quant nq = make_quant(p.nq);
     const int tiles_per_img = tl.tiles_h * tl.tiles_w * tl.cblocks;
     const int64_t total = (int64_t)p.N * tiles_per_img;
 
@@ -212,13 +211,13 @@ depthwise3x3_codes_kernel(const __grid_constant__ CUtensorMap tmIn, const int32_
                     reinterpret_cast<float4 *>(out_f32 + o)[0] = make_float4(tv[0], tv[1], tv[2], tv[3]);
                     reinterpret_cast<float4 *>(out_f32 + o)[1] = make_float4(tv[4], tv[5], tv[6], tv[7]);
                 }
-                if (p.write_codes) {
+                if (p.nq.write_codes) {
                     uint32_t hc[8];
 #pragma unroll
                     for (int c = 0; c < 8; ++c) {
                         const uint32_t neg = __float_as_uint(tv[c]) >> 31;
                         const uint32_t qi = quantize_f32<FAST>(tv[c], nq);
-                        hc[c] = __half_as_ushort(lut[qi | (neg << p.next_bits)]);
+                        hc[c] = __half_as_ushort(lut[qi | (neg << p.nq.bits)]);
                     }
                     *reinterpret_cast<uint4 *>(out_codes + o) =
                         make_uint4(hc[0] | (hc[1] << 16), hc[2] | (hc[3] << 16), hc[4] | (hc[5] << 16), hc[6] | (hc[7] << 16));
@@ -238,14 +237,14 @@ bn_act_encode_kernel(const float *__restrict__ x, float *__restrict__ out_f32, _
 {
     extern __shared__ __align__(128) uint8_t dw_smem[];
     __half *lut = reinterpret_cast<__half *>(dw_smem);
-    if (p.write_codes) {
-        for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
-            lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
+    if (p.nq.write_codes) {
+        for (uint32_t i = threadIdx.x; i < (2u << p.nq.bits); i += blockDim.x) {
+            const int code = elem_code(i & ((1u << p.nq.bits) - 1u), p.nq.enc, p.nq.terms);
+            lut[i] = __int2half_rn((i >> p.nq.bits) ? -code : code);
         }
         __syncthreads();
     }
-    const Quant nq = make_quant(p.write_codes ? p.next_sf : 1.0f, (float)((1u << p.next_bits) - 1u));
+    const Quant nq = make_quant(p.nq);
     const int c4n = C >> 2;
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n4; t += (int64_t)gridDim.x * blockDim.x) {
         const int c4 = (int)(t % c4n);
@@ -265,13 +264,13 @@ bn_act_encode_kernel(const float *__restrict__ x, float *__restrict__ out_f32, _
 #pragma unroll
         for (int e = 0; e < 4; ++e) tv[e] = apply_act(tv[e], p.relu);
         if (p.write_f32) reinterpret_cast<float4 *>(out_f32)[t] = make_float4(tv[0], tv[1], tv[2], tv[3]);
-        if (p.write_codes) {
+        if (p.nq.write_codes) {
             uint32_t hc[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const uint32_t neg = __float_as_uint(tv[e]) >> 31;
-                const uint32_t qi = p.next_fastdiv ? quantize_f32<true>(tv[e], nq) : quantize_f32<false>(tv[e], nq);
-                hc[e] = __half_as_ushort(lut[qi | (neg << p.next_bits)]);
+                const uint32_t qi = p.nq.fastdiv ? quantize_f32<true>(tv[e], nq) : quantize_f32<false>(tv[e], nq);
+                hc[e] = __half_as_ushort(lut[qi | (neg << p.nq.bits)]);
             }
             reinterpret_cast<uint2 *>(out_codes)[t] = make_uint2(hc[0] | (hc[1] << 16), hc[2] | (hc[3] << 16));
         }
@@ -326,9 +325,8 @@ maxpool2d_f16_kernel(const uint4 *__restrict__ x, uint4 *__restrict__ y, int N, 
 struct FirstConvParams {
     int N, H, W, Ho, Wo, stride;
     const float *bias, *bn_a, *bn_b;
-    int relu, write_f32, write_codes;
-    float next_sf;
-    int next_bits, next_terms, next_enc, next_fastdiv;
+    int relu, write_f32;
+    NextQuant nq;
 };
 
 template <int COUT, int STRIDE, bool FAST>
@@ -345,13 +343,13 @@ first_conv3x3_kernel(const float *__restrict__ x, const float *__restrict__ wgt,
     float *sin = sw + 27 * COUT;                                    // [IH][IW][3]
     __half *lut = reinterpret_cast<__half *>(sin + ((IH * IW * 3 + 3) & ~3));
     for (int i = threadIdx.x; i < 27 * COUT; i += 256) sw[i] = wgt[i];
-    if (p.write_codes) {
-        for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += 256) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
-            lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
+    if (p.nq.write_codes) {
+        for (uint32_t i = threadIdx.x; i < (2u << p.nq.bits); i += 256) {
+            const int code = elem_code(i & ((1u << p.nq.bits) - 1u), p.nq.enc, p.nq.terms);
+            lut[i] = __int2half_rn((i >> p.nq.bits) ? -code : code);
         }
     }
-    const Quant nq = make_quant(p.write_codes ? p.next_sf : 1.0f, (float)((1u << p.next_bits) - 1u));
+    const Quant nq = make_quant(p.nq);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int cg = lane % CG, pg = lane / CG;
     const int tiles_w = (p.Wo + TW - 1) / TW, tiles_h = (p.Ho + TH - 1) / TH;
@@ -419,35 +417,19 @@ first_conv3x3_kernel(const float *__restrict__ x, const float *__restrict__ wgt,
                 reinterpret_cast<float4 *>(out_f32 + o)[0] = make_float4(tv[0], tv[1], tv[2], tv[3]);
                 reinterpret_cast<float4 *>(out_f32 + o)[1] = make_float4(tv[4], tv[5], tv[6], tv[7]);
             }
-            if (p.write_codes) {
+            if (p.nq.write_codes) {
                 uint32_t hc[8];
 #pragma unroll
                 for (int c = 0; c < 8; ++c) {
                     const uint32_t neg = __float_as_uint(tv[c]) >> 31;
                     const uint32_t qi = quantize_f32<FAST>(tv[c], nq);
-                    hc[c] = __half_as_ushort(lut[qi | (neg << p.next_bits)]);
+                    hc[c] = __half_as_ushort(lut[qi | (neg << p.nq.bits)]);
                 }
                 *reinterpret_cast<uint4 *>(out_codes + o) =
                     make_uint4(hc[0] | (hc[1] << 16), hc[2] | (hc[3] << 16), hc[4] | (hc[5] << 16), hc[6] | (hc[7] << 16));
             }
         }
     }
-}
-
-static int fill_quant(DwParams &p, void *out_codes, float next_sf, int next_bits, int next_terms, int next_enc)
-{
-    p.write_codes = out_codes ? 1 : 0;
-    p.next_sf = out_codes ? next_sf : 1.0f;
-    p.next_bits = out_codes ? next_bits : 1;
-    p.next_terms = next_terms;
-    p.next_enc = next_enc;
-    if (out_codes) {
-        if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
-        // codes are stored as fp16: |code| <= 2^bits must stay exactly representable
-        if (next_bits < 1 || next_bits > 11 || next_terms < 0) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..11 bits");
-    }
-    p.next_fastdiv = (p.next_sf >= 9.313225746154785e-10f && p.next_sf <= 1073741824.0f) ? 1 : 0;
-    return TQ_OK;
 }
 
 }  // namespace tq
@@ -468,7 +450,9 @@ extern "C" int tq_depthwise3x3_codes_enc(const void *act_codes, const int32_t *w
                                          int stride, float scale, int relu, int act_unsigned, float next_sf, int next_bits,
                                          int next_terms, int next_enc, void *stream)
 {
-    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
+    DwParams p{};
+    int rc = next_quant(p.nq, out_codes, next_sf, next_bits, next_terms, next_enc, FP16_CODE_MAX_BITS, false);
+    if (rc != TQ_OK) return rc;
     if (!act_codes || !wgt_codes || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1 || C < 8 || C % 8) return fail(TQ_ERR_INVALID, "bad shape (C must be a multiple of 8)");
     if (stride != 1 && stride != 2) return fail(TQ_ERR_UNSUPPORTED, "depthwise 3x3: stride 1 or 2");
@@ -478,14 +462,11 @@ extern "C" int tq_depthwise3x3_codes_enc(const void *act_codes, const int32_t *w
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
-    DwParams p{};
     p.N = N; p.H = H; p.W = W; p.C = C; p.stride = stride;
     p.Ho = (H + 2 - 3) / stride + 1;
     p.Wo = (W + 2 - 3) / stride + 1;
     p.scale = scale; p.bias = bias; p.bn_a = bn_a; p.bn_b = bn_b; p.relu = relu;
     p.write_f32 = out_f32 ? 1 : 0;
-    int rc = fill_quant(p, out_codes, next_sf, next_bits, next_terms, next_enc);
-    if (rc != TQ_OK) return rc;
     // tile: TW a multiple of DW_PIX; small maps take small tiles (a 7x7 map in a 8x16 tile would idle 62 % of the lanes)
     DwTile tl{};
     tl.tw = p.Wo > 8 ? 16 : 8;
@@ -513,7 +494,7 @@ extern "C" int tq_depthwise3x3_codes_enc(const void *act_codes, const int32_t *w
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled(depthwise input) failed: %d", (int)r);
     }
-    const size_t smem = 128 + 2 * (size_t)tl.stage_bytes + (size_t)9 * C * 4 + (((size_t)(2u << p.next_bits) * 2 + 15) & ~(size_t)15) + 64;
+    const size_t smem = 128 + 2 * (size_t)tl.stage_bytes + (size_t)9 * C * 4 + code_table_bytes(p.nq.bits) + 64;
     if (smem > 220 * 1024) return fail(TQ_ERR_UNSUPPORTED, "depthwise conv: %d channels do not fit shared memory", C);
     const int64_t total = (int64_t)N * tl.tiles_h * tl.tiles_w * tl.cblocks;
     // persistent CTAs: as many as fit per SM by shared memory (the tile loop double-buffers its own loads)
@@ -533,7 +514,7 @@ extern "C" int tq_depthwise3x3_codes_enc(const void *act_codes, const int32_t *w
           {depthwise3x3_codes_kernel<2, 64, true, false>, depthwise3x3_codes_kernel<2, 64, true, true>}},
          {{depthwise3x3_codes_kernel<2, 32, false, false>, depthwise3x3_codes_kernel<2, 32, false, true>},
           {depthwise3x3_codes_kernel<2, 32, true, false>, depthwise3x3_codes_kernel<2, 32, true, true>}}}};
-    const int i_cb = cbsz == 32 ? 1 : 0, i_un = tl.unsigned_act, i_fast = p.next_fastdiv ? 1 : 0;
+    const int i_cb = cbsz == 32 ? 1 : 0, i_un = tl.unsigned_act, i_fast = p.nq.fastdiv;
     Kern kern = table[stride - 1][i_cb][i_un][i_fast];
     static bool attr_set[16][64] = {{false}};
     const int kidx = ((stride - 1) * 2 + i_cb) * 4 + i_un * 2 + i_fast;
@@ -561,7 +542,9 @@ extern "C" int tq_bn_act_encode_enc(const float *x, const float *bias, const flo
                                     void *out_codes, int64_t npix, int C, int relu, float next_sf, int next_bits,
                                     int next_terms, int next_enc, void *stream)
 {
-    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
+    DwParams p{};
+    const int rc = next_quant(p.nq, out_codes, next_sf, next_bits, next_terms, next_enc, FP16_CODE_MAX_BITS, false);
+    if (rc != TQ_OK) return rc;
     if (!x || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (npix < 0 || C < 4 || C % 4) return fail(TQ_ERR_INVALID, "bad shape (C must be a multiple of 4)");
     if ((bn_a == nullptr) != (bn_b == nullptr)) return fail(TQ_ERR_INVALID, "bn_a and bn_b go together");
@@ -569,15 +552,12 @@ extern "C" int tq_bn_act_encode_enc(const float *x, const float *bias, const flo
     if ((((uintptr_t)x | (uintptr_t)bias | (uintptr_t)bn_a | (uintptr_t)bn_b | (uintptr_t)out_f32 | (uintptr_t)out_codes) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
     if (npix == 0) return TQ_OK;
-    DwParams p{};
     p.C = C; p.bias = bias; p.bn_a = bn_a; p.bn_b = bn_b; p.relu = relu; p.write_f32 = out_f32 ? 1 : 0;
-    int rc = fill_quant(p, out_codes, next_sf, next_bits, next_terms, next_enc);
-    if (rc != TQ_OK) return rc;
     const int64_t n4 = npix * (C / 4);
     int64_t blocks = (n4 + 255) / 256;
     const int64_t cap = (int64_t)num_sms() * 16;
     if (blocks > cap) blocks = cap;
-    const size_t smem = out_codes ? (size_t)(2u << p.next_bits) * sizeof(__half) : 0;
+    const size_t smem = out_codes ? code_table_bytes(p.nq.bits) : 0;
     bn_act_encode_kernel<<<(int)blocks, 256, smem, (cudaStream_t)stream>>>(x, out_f32, (__half *)out_codes, n4, C, p);
     count_launch();
     return check_launch("bn_act_encode_kernel");
@@ -608,11 +588,11 @@ static int launch_first_conv(const float *x, const float *wgt, float *out_f32, v
 {
     constexpr int CGN = COUT / 8, TW = (32 / CGN) * 8, TH = 8;
     constexpr int IW = (TW - 1) * STRIDE + 3, IH = (TH - 1) * STRIDE + 3;
-    const size_t smem = (size_t)27 * COUT * 4 + (size_t)((IH * IW * 3 + 3) & ~3) * 4 + (p.write_codes ? (size_t)(2u << p.next_bits) * 2 : 0);
+    const size_t smem = (size_t)27 * COUT * 4 + (size_t)((IH * IW * 3 + 3) & ~3) * 4 + (p.nq.write_codes ? code_table_bytes(p.nq.bits) : 0);
     const int64_t tiles = (int64_t)p.N * ((p.Ho + TH - 1) / TH) * ((p.Wo + TW - 1) / TW);
     const int64_t cap = (int64_t)num_sms() * 2;
     const int grid = (int)(tiles < cap ? tiles : cap);
-    auto kern = p.next_fastdiv ? first_conv3x3_kernel<COUT, STRIDE, true> : first_conv3x3_kernel<COUT, STRIDE, false>;
+    auto kern = p.nq.fastdiv ? first_conv3x3_kernel<COUT, STRIDE, true> : first_conv3x3_kernel<COUT, STRIDE, false>;
     if (smem > 48 * 1024 && cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
         return check_launch("cudaFuncSetAttribute(first_conv3x3_kernel)");
     kern<<<grid, 256, smem, s>>>(x, wgt, out_f32, (__half *)out_codes, p);
@@ -633,7 +613,9 @@ extern "C" int tq_first_conv3x3_fused_enc(const float *x, const float *wgt, cons
                                           int stride, int relu, float next_sf, int next_bits, int next_terms, int next_enc,
                                           void *stream)
 {
-    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
+    FirstConvParams p{};
+    const int rc = next_quant(p.nq, out_codes, next_sf, next_bits, next_terms, next_enc, FP16_CODE_MAX_BITS, false);
+    if (rc != TQ_OK) return rc;
     if (!x || !wgt || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1) return fail(TQ_ERR_INVALID, "bad shape");
     if (Cout != 32 && Cout != 64) return fail(TQ_ERR_UNSUPPORTED, "first conv: Cout must be 32 or 64, got %d", Cout);
@@ -642,15 +624,9 @@ extern "C" int tq_first_conv3x3_fused_enc(const float *x, const float *wgt, cons
     if (relu < 0 || relu > 2) return fail(TQ_ERR_INVALID, "relu: 0 none, 1 ReLU, 2 ReLU6");
     if ((((uintptr_t)out_f32 | (uintptr_t)out_codes) & 15u) != 0 || (((uintptr_t)x | (uintptr_t)wgt) & 3u) != 0)
         return fail(TQ_ERR_INVALID, "outputs must be 16-byte aligned");
-    FirstConvParams p{};
     p.N = N; p.H = H; p.W = W; p.stride = stride;
     p.Ho = (H + 2 - 3) / stride + 1; p.Wo = (W + 2 - 3) / stride + 1;                // pad 1
     p.bias = bias; p.bn_a = bn_a; p.bn_b = bn_b; p.relu = relu; p.write_f32 = out_f32 ? 1 : 0;
-    DwParams q{};
-    int rc = fill_quant(q, out_codes, next_sf, next_bits, next_terms, next_enc);
-    if (rc != TQ_OK) return rc;
-    p.write_codes = q.write_codes; p.next_sf = q.next_sf; p.next_bits = q.next_bits; p.next_terms = q.next_terms;
-    p.next_enc = q.next_enc; p.next_fastdiv = q.next_fastdiv;
     cudaStream_t s = (cudaStream_t)stream;
     if (Cout == 64) return stride == 1 ? launch_first_conv<64, 1>(x, wgt, out_f32, out_codes, p, s) : launch_first_conv<64, 2>(x, wgt, out_f32, out_codes, p, s);
     return stride == 1 ? launch_first_conv<32, 1>(x, wgt, out_f32, out_codes, p, s) : launch_first_conv<32, 2>(x, wgt, out_f32, out_codes, p, s);

@@ -607,8 +607,7 @@ static int validate(const void *in, const void *out, int64_t B, int64_t C, int64
     p.alpha = alpha;
     p.enc = enc;
     p.relu = (flags & TQ_FLAG_RELU) ? 1 : 0;
-    p.fastdiv = (sf >= 9.313225746154785e-10f && sf <= 1073741824.0f) ? 1 : 0;   // [2^-30, 2^30]
-    if (flags & TQ_FLAG_EXACT_DIV) p.fastdiv = 0;
+    p.fastdiv = fast_div_ok(sf) && !(flags & TQ_FLAG_EXACT_DIV) ? 1 : 0;
     return TQ_OK;
 }
 

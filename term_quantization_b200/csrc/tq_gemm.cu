@@ -106,9 +106,8 @@ struct ConvGeom {
     // fused epilogue (all optional):  t = acc*scale (+bias) ; t = fma(t, bn_a, bn_b) ; t += residual ;
     // t = max(t, 0) ; fp32 tile out (TMA store) ; fp16 term codes of t for the next layer (TMA store)
     const float *bias, *bn_a, *bn_b, *residual;
-    int relu, relu6, write_f32, write_codes;    // relu6: additionally clamp at 6 (ReLU6 of the depthwise CNNs)
-    float next_sf;
-    int next_bits, next_terms, next_enc, next_fastdiv;
+    int relu, relu6, write_f32;                 // relu6: additionally clamp at 6 (ReLU6 of the depthwise CNNs)
+    NextQuant nq;
 };
 
 // ---- PTX wrappers ---------------------------------------------------------------------------
@@ -306,7 +305,7 @@ __device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t saddr)
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
 
-constexpr int GM_LUT_MAX_BITS = 10;             // fused next-layer encode: 2^(bits+1) fp16 entries in smem
+constexpr int GM_LUT_MAX_BITS = 10;             // fused next-layer encode: code_table_bytes(bits) in smem
 constexpr int GM_MAX_STAGES = 8;
 constexpr int GM_EPI_GROUPS = 4;                // (accumulator stage, column half)
 constexpr int GM_EPI_F32_BYTES = 16384;         // per epilogue group: [128][32] fp32 staging (output tile / residual tile)
@@ -387,10 +386,10 @@ __device__ __forceinline__ void epi_stage(float (&t)[32], const ConvGeom &g, uin
         for (int j = 0; j < 32; j += 4)
             *reinterpret_cast<float4 *>(frow + (((uint32_t)(j >> 2) ^ sw128) << 4)) = make_float4(t[j], t[j + 1], t[j + 2], t[j + 3]);
     }
-    if (g.write_codes) {
+    if (g.nq.write_codes) {
         // entry address = lut + 2 * (q | sign << bits), q = bits(t) - 0x4B000000
         const uint32_t lut_s = smem_u32(lut) - 2u * 0x4B000000u;
-        const uint32_t sign_off = 2u << g.next_bits;        // byte offset of the negative half of the table
+        const uint32_t sign_off = 2u << g.nq.bits;          // byte offset of the negative half of the table
 #pragma unroll
         for (int j = 0; j < 32; j += 8) {
             uint32_t hc[8];
@@ -481,15 +480,15 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
         if (g.write_f32) asm volatile("prefetch.tensormap [%0];" ::"l"(&tmC) : "memory");
-        if (g.write_codes) asm volatile("prefetch.tensormap [%0];" ::"l"(&tmD) : "memory");
+        if (g.nq.write_codes) asm volatile("prefetch.tensormap [%0];" ::"l"(&tmD) : "memory");
         if (g.residual) asm volatile("prefetch.tensormap [%0];" ::"l"(&tmR) : "memory");
     }
     __half *lut = reinterpret_cast<__half *>(smem + g.lut_off);
-    if (g.write_codes) {
+    if (g.nq.write_codes) {
         // (q, sign) -> fp16 term code of the consumer's quantiser, as in tr_elem_kernel
-        for (uint32_t i = threadIdx.x; i < (2u << g.next_bits); i += GM_THREADS) {
-            int code = elem_code(i & ((1u << g.next_bits) - 1u), g.next_enc, g.next_terms);
-            lut[i] = __int2half_rn((i >> g.next_bits) ? -code : code);
+        for (uint32_t i = threadIdx.x; i < (2u << g.nq.bits); i += GM_THREADS) {
+            int code = elem_code(i & ((1u << g.nq.bits) - 1u), g.nq.enc, g.nq.terms);
+            lut[i] = __int2half_rn((i >> g.nq.bits) ? -code : code);
         }
     }
     if (MODE == 4 && g.img_h1) {
@@ -939,7 +938,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         const bool store_thread = (ew == 0 && lane == 0);
         uint8_t *st_f32 = smem + g.epi_off + grp * g.epi_group_bytes;   // [128][32] fp32, 128B swizzle
         uint8_t *st_codes = st_f32 + g.epi_codes_off;                   // [128][32] fp16,  64B swizzle
-        const Quant nq = make_quant(g.write_codes ? g.next_sf : 1.0f, (float)((1u << g.next_bits) - 1u));
+        const Quant nq = make_quant(g.nq);
         const bool has_res = g.residual != nullptr;
         // With two or three accumulator stages the pairs alternate tiles and group (pair, half) takes half of the columns.
         // With ONE stage (a tile's accumulator groups fill tensor memory) consecutive completions of the same barrier
@@ -1183,14 +1182,14 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                             const uint32_t psw = (uint32_t)(pp & 7);
                             *reinterpret_cast<float4 *>(st_pool + pp * 128 + (((uint32_t)(2 * cb) ^ psw) << 4)) = make_float4(pv[0], pv[1], pv[2], pv[3]);
                             *reinterpret_cast<float4 *>(st_pool + pp * 128 + (((uint32_t)(2 * cb + 1) ^ psw) << 4)) = make_float4(pv[4], pv[5], pv[6], pv[7]);
-                            if (g.write_codes) {
+                            if (g.nq.write_codes) {
                                 uint32_t hc[8];
 #pragma unroll
                                 for (int e = 0; e < 8; ++e) {
                                     uint32_t idx;
-                                    if (RELU) idx = g.next_fastdiv ? quantize_f32_nonneg<true>(pv[e], nq) : quantize_f32_nonneg<false>(pv[e], nq);
-                                    else idx = (g.next_fastdiv ? quantize_f32<true>(pv[e], nq) : quantize_f32<false>(pv[e], nq)) |
-                                               ((__float_as_uint(pv[e]) >> 31) << g.next_bits);
+                                    if (RELU) idx = g.nq.fastdiv ? quantize_f32_nonneg<true>(pv[e], nq) : quantize_f32_nonneg<false>(pv[e], nq);
+                                    else idx = (g.nq.fastdiv ? quantize_f32<true>(pv[e], nq) : quantize_f32<false>(pv[e], nq)) |
+                                               ((__float_as_uint(pv[e]) >> 31) << g.nq.bits);
                                     hc[e] = __half_as_ushort(lut[idx]);
                                 }
                                 *reinterpret_cast<uint4 *>(st_pcodes + pp * 64 + (((uint32_t)cb ^ (uint32_t)((pp >> 1) & 3)) << 4)) =
@@ -1202,7 +1201,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                         epi_bar_sync(1 + grp);
                         if (store_thread) {
                             tma_store_4d(&tmC, st_pool, c0, tw * g.pool_q, th * g.pool_p, n0);
-                            if (g.write_codes) tma_store_4d(&tmD, st_pcodes, c0, tw * g.pool_q, th * g.pool_p, n0);
+                            if (g.nq.write_codes) tma_store_4d(&tmD, st_pcodes, c0, tw * g.pool_q, th * g.pool_p, n0);
                             bulk_commit();
                         }
                         TR_SINCE(6, tq0);
@@ -1228,7 +1227,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                 epi_bar_sync(1 + grp);
                 if (store_thread) {
                     if (g.write_f32) tma_store_4d(&tmC, st_f32, c0, w0, h0, n0);
-                    if (g.write_codes) tma_store_4d(&tmD, st_codes, c0, w0, h0, n0);
+                    if (g.nq.write_codes) tma_store_4d(&tmD, st_codes, c0, w0, h0, n0);
                     bulk_commit();
                 }
                 TR_SINCE(5, ts0);
@@ -1350,9 +1349,9 @@ static int plan_smem(ConvGeom &g, int block_n)
     // epilogue staging per group: fp32 tile only if an fp32 tile is written or a residual is read, code tile only
     // if codes are written -- what is not needed goes to the stage ring
     g.epi_codes_off = (g.write_f32 || g.residual) ? GM_EPI_F32_BYTES : 0;
-    g.epi_group_bytes = g.epi_codes_off + ((g.write_codes || g.pool == 1) ? GM_EPI_CODE_BYTES : 0);
+    g.epi_group_bytes = g.epi_codes_off + ((g.nq.write_codes || g.pool == 1) ? GM_EPI_CODE_BYTES : 0);
     const int epi_bytes = GM_EPI_GROUPS * g.epi_group_bytes;
-    const int fixed = g.ring_off + epi_bytes + (2 << GM_LUT_MAX_BITS) * 2 + 1024 /* barriers */ + 1024 /* align */;
+    const int fixed = g.ring_off + epi_bytes + (int)code_table_bytes(GM_LUT_MAX_BITS) + 1024 /* barriers */ + 1024 /* align */;
     int stages = (GM_SMEM_BUDGET - fixed) / g.stage_bytes;
     if (stages > GM_MAX_STAGES) stages = GM_MAX_STAGES;
     static const int cap = getenv("TQ_CONV_STAGES") ? atoi(getenv("TQ_CONV_STAGES")) : GM_MAX_STAGES;
@@ -1361,7 +1360,7 @@ static int plan_smem(ConvGeom &g, int block_n)
     g.stages = stages;
     g.epi_off = g.ring_off + stages * g.stage_bytes;
     g.lut_off = g.epi_off + epi_bytes;
-    g.bar_off = g.lut_off + (2 << GM_LUT_MAX_BITS) * 2;
+    g.bar_off = g.lut_off + (int)code_table_bytes(GM_LUT_MAX_BITS);
     g.smem_total = g.bar_off + 1024 + 1024;
     return TQ_OK;
 }
@@ -1470,8 +1469,9 @@ static int launch_variant(ConvVariant v, const CUtensorMap &tmA, const CUtensorM
 // as long as the caller reuses the same buffers, and any other argument tuple simply plans again.
 struct ConvArgs {
     const void *act, *wgt, *out_f32, *out_codes, *bias, *bn_a, *bn_b, *residual;
-    int kind, N, H, W, C, Cout, R, S, stride, pad, relu, next_bits, next_terms, next_enc, acc_groups, planes_a, planes_w, device;
-    float scale, next_sf;
+    int kind, N, H, W, C, Cout, R, S, stride, pad, relu, acc_groups, planes_a, planes_w, device;
+    float scale;
+    NextQuant nq;
 };
 struct ConvPlan {
     ConvArgs key;
@@ -1540,12 +1540,7 @@ static int plan_conv(const ConvArgs &a, ConvPlan &pl)
     g.relu = a.relu ? 1 : 0;
     g.relu6 = a.relu == 2 ? 1 : 0;
     g.write_f32 = a.out_f32 ? 1 : 0;
-    g.write_codes = a.out_codes ? 1 : 0;
-    g.next_sf = a.out_codes ? a.next_sf : 1.0f;
-    g.next_bits = a.out_codes ? a.next_bits : 1;
-    g.next_terms = a.next_terms;
-    g.next_enc = a.next_enc;
-    g.next_fastdiv = (g.next_sf >= 9.313225746154785e-10f && g.next_sf <= 1073741824.0f) ? 1 : 0;
+    g.nq = a.nq;
     // accumulator groups
     if (kind == 1) {
         g.n_groups = g.planes_a + g.planes_w - 1;
@@ -1690,12 +1685,14 @@ static int run_conv(ConvArgs &a, cudaStream_t s)
     return launch_variant(pl.variant, pl.tmA, pl.tmB, pl.tmC, pl.tmD, pl.tmR, pl.g, s);
 }
 
-static int check_conv_args(const void *act, const void *wgt, const void *out_f32, const void *out_codes, const void *bias,
-                           const void *bn_a, const void *bn_b, const void *residual, int N, int H, int W, int C, int Cout,
-                           int R, int S, int stride, int pad, float next_sf, int next_bits, int next_terms, int next_enc,
-                           int c_align)
+// checks the arguments and fills nq; the fused encode only has the hoisted-reciprocal divide (tq_common.cuh)
+static int check_conv_args(NextQuant &nq, const void *act, const void *wgt, const void *out_f32, const void *out_codes,
+                           const void *bias, const void *bn_a, const void *bn_b, const void *residual, int N, int H, int W,
+                           int C, int Cout, int R, int S, int stride, int pad, float next_sf, int next_bits, int next_terms,
+                           int next_enc, int c_align)
 {
-    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
+    const int rc = next_quant(nq, out_codes, next_sf, next_bits, next_terms, next_enc, GM_LUT_MAX_BITS, true);
+    if (rc != TQ_OK) return rc;
     if (!act || !wgt || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1 || C < 1 || Cout < 1 || R < 1 || S < 1 || stride < 1 || pad < 0)
         return fail(TQ_ERR_INVALID, "bad convolution geometry");
@@ -1706,14 +1703,6 @@ static int check_conv_args(const void *act, const void *wgt, const void *out_f32
     if ((((uintptr_t)act | (uintptr_t)wgt | (uintptr_t)out_f32 | (uintptr_t)out_codes | (uintptr_t)bias |
           (uintptr_t)bn_a | (uintptr_t)bn_b | (uintptr_t)residual) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
-    if (out_codes) {
-        if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
-        if (next_bits < 1 || next_bits > GM_LUT_MAX_BITS) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..%d bits", GM_LUT_MAX_BITS);
-        if (next_terms < 0) return fail(TQ_ERR_INVALID, "next_terms must be >= 0");
-        // the fused encode divides with the hoisted reciprocal (tq_common.cuh), exact for 2^-30 <= sf <= 2^30
-        if (!(next_sf >= 9.313225746154785e-10f && next_sf <= 1073741824.0f))
-            return fail(TQ_ERR_UNSUPPORTED, "fused encode needs 2^-30 <= next_sf <= 2^30 (got %g): encode with tq_tr_encode_codes instead", (double)next_sf);
-    }
     return TQ_OK;
 }
 
@@ -1737,18 +1726,17 @@ extern "C" int tq_conv2d_codes_fused_enc(const void *act, const void *wgt, float
                                          int stride, int pad, float scale, int relu, float next_sf, int next_bits,
                                          int next_terms, int next_enc, int acc_groups, void *stream)
 {
-    int rc = check_conv_args(act, wgt, out_f32, out_codes, bias, bn_a, bn_b, residual, N, H, W, C, Cout, R, S, stride, pad,
-                             next_sf, next_bits, next_terms, next_enc, 8);
-    if (rc != TQ_OK) return rc;
     ConvArgs a;
     memset(&a, 0, sizeof(a));                       // (padding bytes take part in the cache key)
+    int rc = check_conv_args(a.nq, act, wgt, out_f32, out_codes, bias, bn_a, bn_b, residual, N, H, W, C, Cout, R, S, stride, pad,
+                             next_sf, next_bits, next_terms, next_enc, 8);
+    if (rc != TQ_OK) return rc;
     a.act = act; a.wgt = wgt; a.out_f32 = out_f32; a.out_codes = out_codes; a.bias = bias; a.bn_a = bn_a; a.bn_b = bn_b;
     a.residual = residual;
     a.kind = 0; a.N = N; a.H = H; a.W = W; a.C = C; a.Cout = Cout; a.R = R; a.S = S; a.stride = stride; a.pad = pad;
-    a.relu = relu == 2 ? 2 : (relu ? 1 : 0); a.next_bits = out_codes ? next_bits : 1; a.next_terms = next_terms;
-    a.next_enc = next_enc;
+    a.relu = relu == 2 ? 2 : (relu ? 1 : 0);
     a.acc_groups = acc_groups < 1 ? 1 : acc_groups; a.planes_a = 1; a.planes_w = 1;
-    a.scale = scale; a.next_sf = out_codes ? next_sf : 1.0f;
+    a.scale = scale;
     return run_conv(a, (cudaStream_t)stream);
 }
 
@@ -1778,8 +1766,10 @@ extern "C" int tq_conv2d_planes_i8_enc(const void *act_planes, const void *wgt_p
                                        int R, int S, int stride, int pad, float scale, int relu, float next_sf,
                                        int next_bits, int next_terms, int next_enc, int act_max, int wgt_max, void *stream)
 {
-    int rc = check_conv_args(act_planes, wgt_planes, out_f32, out_codes, bias, bn_a, bn_b, residual, N, H, W, C, Cout, R, S,
-                             stride, pad, next_sf, next_bits, next_terms, next_enc, 16);
+    ConvArgs a;
+    memset(&a, 0, sizeof(a));
+    int rc = check_conv_args(a.nq, act_planes, wgt_planes, out_f32, out_codes, bias, bn_a, bn_b, residual, N, H, W, C, Cout, R,
+                             S, stride, pad, next_sf, next_bits, next_terms, next_enc, 16);
     if (rc != TQ_OK) return rc;
     if (planes_a < 1 || planes_a > 2 || planes_w < 1 || planes_w > 2) return fail(TQ_ERR_INVALID, "1 or 2 planes per operand");
     // int32 accumulators: |acc| <= K * act_max * wgt_max (the caller's bounds on |code|: 2^bits by construction of the
@@ -1789,15 +1779,12 @@ extern "C" int tq_conv2d_planes_i8_enc(const void *act_planes, const void *wgt_p
         return fail(TQ_ERR_INVALID, "act_max / wgt_max must lie in 1..%d / 1..%d for %d / %d planes", acap, wcap, planes_a, planes_w);
     if ((double)C * R * S * (double)act_max * (double)wgt_max >= 2147483648.0)
         return fail(TQ_ERR_UNSUPPORTED, "K = %d with |a| <= %d, |w| <= %d can overflow an int32 accumulator", C * R * S, act_max, wgt_max);
-    ConvArgs a;
-    memset(&a, 0, sizeof(a));
     a.act = act_planes; a.wgt = wgt_planes; a.out_f32 = out_f32; a.out_codes = out_codes; a.bias = bias; a.bn_a = bn_a;
     a.bn_b = bn_b; a.residual = residual;
     a.kind = 1; a.N = N; a.H = H; a.W = W; a.C = C; a.Cout = Cout; a.R = R; a.S = S; a.stride = stride; a.pad = pad;
-    a.relu = relu == 2 ? 2 : (relu ? 1 : 0); a.next_bits = out_codes ? next_bits : 1; a.next_terms = next_terms;
-    a.next_enc = next_enc;
+    a.relu = relu == 2 ? 2 : (relu ? 1 : 0);
     a.acc_groups = 1; a.planes_a = planes_a; a.planes_w = planes_w;
-    a.scale = scale; a.next_sf = out_codes ? next_sf : 1.0f;
+    a.scale = scale;
     return run_conv(a, (cudaStream_t)stream);
 }
 
@@ -1964,7 +1951,11 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
                      int next_terms, int next_enc, int N, int H, int W, int Cout, void *stream, const float *mean3 = nullptr,
                      const float *std3 = nullptr)
 {
-    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
+    // the quantiser is checked before the fold pass below is launched: a refused call enqueues nothing (only the pooled
+    // stem passes out_codes)
+    ConvGeom g{};
+    int rc = next_quant(g.nq, out_codes, next_sf, next_bits, next_terms, next_enc, GM_LUT_MAX_BITS, false);
+    if (rc != TQ_OK) return rc;
     if (!x || !x2_scratch || !w2 || !out) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (x_dtype != TQ_F32 && x_dtype != TQ_BF16 && x_dtype != TQ_F16 && x_dtype != STEM_U8)
         return fail(TQ_ERR_UNSUPPORTED, "stem conv input must be fp32, bf16, fp16 or uint8");
@@ -1981,11 +1972,6 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
     if (Cout < 4 || Cout % 4) return fail(TQ_ERR_UNSUPPORTED, "Cout must be a multiple of 4");
     if ((((uintptr_t)x2_scratch | (uintptr_t)w2 | (uintptr_t)out) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
-    // the pooled stem's quantiser is checked before the fold pass below is launched: a refused call enqueues nothing
-    if (pool == 1 && out_codes) {
-        if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
-        if (next_bits < 1 || next_bits > GM_LUT_MAX_BITS || next_terms < 0) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..%d bits", GM_LUT_MAX_BITS);
-    }
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
     cudaStream_t s = (cudaStream_t)stream;
@@ -2004,11 +1990,9 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
         else
             stem_prepare_kernel<__half, false><<<(int)blocks, 256, 0, s>>>((const __half *)x, (__half *)x2_scratch, N, H, W, Hs, Ws, nm);
         count_launch();
-        int rc = check_launch("stem_prepare_kernel");
-        if (rc != TQ_OK) return rc;
+        if ((rc = check_launch("stem_prepare_kernel")) != TQ_OK) return rc;
     }
 
-    ConvGeom g{};
     g.N = N; g.H = Hs; g.W = Wo; g.C = 64; g.Cout = Cout; g.R = 4; g.S = 1; g.stride = 1; g.pad = 0;
     g.Ho = Ho; g.Wo = Wo;
     g.scale = 1.0f;
@@ -2043,15 +2027,11 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
         g.a_tx_bytes = g.wbox * g.hbox * GM_BLOCK_K * 2;
         if (g.pool_p * g.pool_q > 32) return fail(TQ_ERR_UNSUPPORTED, "pooled tile too large");
         g.bn_a = bn_a; g.bn_b = bn_b; g.relu = relu ? 1 : 0;
-        g.write_codes = out_codes ? 1 : 0;
     }
     g.hw = g.wbox;
     const int block_n = Cout <= 64 ? 64 : 128;
     g.n_tiles = (Cout + block_n - 1) / block_n;
     g.write_f32 = 1;
-    g.next_sf = out_codes ? next_sf : 1.0f; g.next_bits = out_codes ? next_bits : 1; g.next_terms = next_terms;
-    g.next_enc = next_enc;
-    g.next_fastdiv = (g.next_sf >= 9.313225746154785e-10f && g.next_sf <= 1073741824.0f) ? 1 : 0;
     // program: per image plane (x_hi, and x_lo for fp32 images) ONE halo load covering the four folded filter rows; per
     // filter row R one N = 128 MMA group against the resident tile R = [w_hi (rows 0..63) ; w_lo (rows 64..127)]: columns
     // [c, c+64) of the accumulator receive x * w_hi, [c+64, c+128) x * w_lo.  Rows 0-1 and rows 2-3 accumulate apart
@@ -2067,7 +2047,6 @@ static int stem_impl(const void *x, int x_dtype, void *x2_scratch, const void *w
     }
 
     CUtensorMap tmA, tmB, tmC, tmD;
-    int rc;
     {   // overlapping windows: inner 64 elements, output column advances by one folded pixel (16 elements)
         cuuint64_t dims[4] = {64, (cuuint64_t)Wo, (cuuint64_t)Hs, (cuuint64_t)((lo_plane ? 2 : 1) * N)};
         cuuint64_t strides[3] = {32, (cuuint64_t)Ws * 32, (cuuint64_t)Hs * Ws * 32};

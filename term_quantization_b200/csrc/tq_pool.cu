@@ -21,8 +21,7 @@ namespace tq {
 struct PoolParams {
     int N, H, W, C, Ho, Wo;
     int relu;
-    float next_sf;
-    int next_bits, next_terms, next_enc, next_fastdiv, write_codes;
+    NextQuant nq;
 };
 
 __global__ void __launch_bounds__(256)
@@ -31,14 +30,14 @@ bn_relu_maxpool3x3s2_kernel(const float *__restrict__ x, const float *__restrict
                             __half *__restrict__ codes, PoolParams p)
 {
     extern __shared__ __half lut[];
-    if (p.write_codes) {
-        for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
-            lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
+    if (p.nq.write_codes) {
+        for (uint32_t i = threadIdx.x; i < (2u << p.nq.bits); i += blockDim.x) {
+            const int code = elem_code(i & ((1u << p.nq.bits) - 1u), p.nq.enc, p.nq.terms);
+            lut[i] = __int2half_rn((i >> p.nq.bits) ? -code : code);
         }
         __syncthreads();
     }
-    const Quant nq = make_quant(p.write_codes ? p.next_sf : 1.0f, (float)((1u << p.next_bits) - 1u));
+    const Quant nq = make_quant(p.nq);
     const int c4n = p.C >> 2;
     const int64_t total = (int64_t)p.N * p.Ho * p.Wo * c4n;
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
@@ -65,14 +64,14 @@ bn_relu_maxpool3x3s2_kernel(const float *__restrict__ x, const float *__restrict
         }
         if (p.relu) { m.x = fmaxf(m.x, 0.f); m.y = fmaxf(m.y, 0.f); m.z = fmaxf(m.z, 0.f); m.w = fmaxf(m.w, 0.f); }
         reinterpret_cast<float4 *>(out)[t] = m;
-        if (p.write_codes) {
+        if (p.nq.write_codes) {
             const float vv[4] = {m.x, m.y, m.z, m.w};
             uint32_t hc[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const uint32_t neg = __float_as_uint(vv[e]) >> 31;
-                const uint32_t q = p.next_fastdiv ? quantize_f32<true>(vv[e], nq) : quantize_f32<false>(vv[e], nq);
-                hc[e] = __half_as_ushort(lut[q | (neg << p.next_bits)]);
+                const uint32_t q = p.nq.fastdiv ? quantize_f32<true>(vv[e], nq) : quantize_f32<false>(vv[e], nq);
+                hc[e] = __half_as_ushort(lut[q | (neg << p.nq.bits)]);
             }
             reinterpret_cast<uint2 *>(codes)[t] = make_uint2(hc[0] | (hc[1] << 16), hc[2] | (hc[3] << 16));
         }
@@ -108,11 +107,11 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
     extern __shared__ __align__(128) uint8_t pool_smem[];
     uint8_t *base = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(pool_smem) + 127) & ~uintptr_t(127));
     __half *lut = reinterpret_cast<__half *>(base + PT_STAGES * PT_STAGE_BYTES);
-    uint64_t *full = reinterpret_cast<uint64_t *>(base + PT_STAGES * PT_STAGE_BYTES + (((size_t)(2u << p.next_bits) * 2 + 15) & ~(size_t)15));
-    if (p.write_codes) {
-        for (uint32_t i = threadIdx.x; i < (2u << p.next_bits); i += blockDim.x) {
-            const int code = elem_code(i & ((1u << p.next_bits) - 1u), p.next_enc, p.next_terms);
-            lut[i] = __int2half_rn((i >> p.next_bits) ? -code : code);
+    uint64_t *full = reinterpret_cast<uint64_t *>(base + PT_STAGES * PT_STAGE_BYTES + code_table_bytes(p.nq.bits));
+    if (p.nq.write_codes) {
+        for (uint32_t i = threadIdx.x; i < (2u << p.nq.bits); i += blockDim.x) {
+            const int code = elem_code(i & ((1u << p.nq.bits) - 1u), p.nq.enc, p.nq.terms);
+            lut[i] = __int2half_rn((i >> p.nq.bits) ? -code : code);
         }
     }
     auto s32 = [](const void *q) { return (uint32_t)__cvta_generic_to_shared(q); };
@@ -122,7 +121,7 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmIn) : "memory");
     }
     __syncthreads();
-    const Quant nq = make_quant(p.write_codes ? p.next_sf : 1.0f, (float)((1u << p.next_bits) - 1u));
+    const Quant nq = make_quant(p.nq);
     const int cblocks = (p.C + PT_CB - 1) / PT_CB, tiles_w = (p.Wo + PT_PC - 1) / PT_PC, tiles_h = (p.Ho + PT_PR - 1) / PT_PR;
     const int64_t total = (int64_t)p.N * tiles_h * tiles_w * cblocks;
     const int C4 = p.C >> 2;
@@ -192,14 +191,14 @@ bn_relu_maxpool3x3s2_tiled_kernel(const __grid_constant__ CUtensorMap tmIn, cons
             if (p.relu) { m.x = fmaxf(m.x, 0.f); m.y = fmaxf(m.y, 0.f); m.z = fmaxf(m.z, 0.f); m.w = fmaxf(m.w, 0.f); }
             const int64_t oi = (((int64_t)n * p.Ho + ho) * p.Wo + wo) * C4 + cg;
             reinterpret_cast<float4 *>(out)[oi] = m;
-            if (p.write_codes) {
+            if (p.nq.write_codes) {
                 const float vv[4] = {m.x, m.y, m.z, m.w};
                 uint32_t hc[4];
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
                     const uint32_t neg = __float_as_uint(vv[e]) >> 31;
-                    const uint32_t q = p.next_fastdiv ? quantize_f32<true>(vv[e], nq) : quantize_f32<false>(vv[e], nq);
-                    hc[e] = __half_as_ushort(lut[q | (neg << p.next_bits)]);
+                    const uint32_t q = p.nq.fastdiv ? quantize_f32<true>(vv[e], nq) : quantize_f32<false>(vv[e], nq);
+                    hc[e] = __half_as_ushort(lut[q | (neg << p.nq.bits)]);
                 }
                 reinterpret_cast<uint2 *>(codes)[oi] = make_uint2(hc[0] | (hc[1] << 16), hc[2] | (hc[3] << 16));
             }
@@ -220,26 +219,16 @@ int pool_params(PoolParams &p, const float *x, const float *bn_a, const float *b
                 int H, int W, int C, int Wo, int relu, float next_sf, int next_bits, int next_terms, int next_enc)
 {
     if (!x || !bn_a || !bn_b || !out) return fail(TQ_ERR_INVALID, "NULL pointer");
-    if (check_encoding(next_enc) != TQ_OK) return TQ_ERR_INVALID;
+    p = PoolParams{};
+    const int rc = next_quant(p.nq, out_codes, next_sf, next_bits, next_terms, next_enc, FP16_CODE_MAX_BITS, false);
+    if (rc != TQ_OK) return rc;
     if (N < 1 || H < 1 || W < 1 || C < 4 || C % 4) return fail(TQ_ERR_INVALID, "bad shape (C must be a multiple of 4)");
     if ((((uintptr_t)x | (uintptr_t)bn_a | (uintptr_t)bn_b | (uintptr_t)out | (uintptr_t)out_codes) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
-    p = PoolParams{};
     p.N = N; p.H = H; p.W = W; p.C = C;
     p.Ho = (H + 2 - 3) / 2 + 1;
     p.Wo = Wo;
     p.relu = relu ? 1 : 0;
-    p.write_codes = out_codes ? 1 : 0;
-    p.next_sf = out_codes ? next_sf : 1.0f;
-    p.next_bits = out_codes ? next_bits : 1;
-    p.next_terms = next_terms;
-    p.next_enc = next_enc;
-    if (out_codes) {
-        if (!(next_sf > 0.0f) || !(next_sf < INFINITY)) return fail(TQ_ERR_INVALID, "next_sf must be positive and finite");
-        // codes are stored as fp16: |code| <= 2^bits must stay exactly representable (11-bit significand)
-        if (next_bits < 1 || next_bits > 11 || next_terms < 0) return fail(TQ_ERR_UNSUPPORTED, "fused encode supports 1..11 bits");
-    }
-    p.next_fastdiv = (p.next_sf >= 9.313225746154785e-10f && p.next_sf <= 1073741824.0f) ? 1 : 0;
     return TQ_OK;
 }
 
@@ -258,7 +247,7 @@ int launch_tiled(EncodeTiledFn enc, const float *x, const float *bn_a, const flo
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(TQ_ERR_CUDA, "cuTensorMapEncodeTiled(pool input) failed: %d", (int)r);
-    const size_t smem_t = PT_STAGES * (size_t)T::STAGE_BYTES + (((size_t)(2u << p.next_bits) * 2 + 15) & ~(size_t)15) + 64 + 128;
+    const size_t smem_t = PT_STAGES * (size_t)T::STAGE_BYTES + code_table_bytes(p.nq.bits) + 64 + 128;
     static bool attr_done[64] = {false};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -296,7 +285,7 @@ extern "C" int tq_bn_relu_maxpool_encode_enc(const float *x, const float *bn_a, 
     int64_t blocks = (total + 255) / 256;
     const int64_t cap = (int64_t)num_sms() * 16;
     if (blocks > cap) blocks = cap;
-    const size_t smem = out_codes ? (size_t)(2u << p.next_bits) * sizeof(__half) : 0;
+    const size_t smem = out_codes ? code_table_bytes(p.nq.bits) : 0;
     bn_relu_maxpool3x3s2_kernel<<<(int)blocks, 256, smem, (cudaStream_t)stream>>>(
         x, bn_a, bn_b, out, (__half *)out_codes, p);
     count_launch();

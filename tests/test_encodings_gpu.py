@@ -40,26 +40,30 @@ def check_codes(got, want_f32, quant, what):
 
 
 # index of `next_enc` in the argument list of each _enc entry point: dropping it gives the original entry point's
-# (conv_codes sends a HESE quantiser to the original entry point, any other encoding to the _enc twin)
+# (conv_codes calls the _enc entry points for every encoding; the originals remain for C callers)
 _ENC_ARG = {"tq_conv2d_codes_fused_enc": 22, "tq_conv2d_planes_i8_enc": 24, "tq_stem_conv7x7s2_pool_enc": 16,
             "tq_bn_relu_maxpool_encode_enc": 13, "tq_bn_relu_maxpool_encode_rowmax_enc": 13,
             "tq_depthwise3x3_codes_enc": 18, "tq_bn_act_encode_enc": 12, "tq_first_conv3x3_fused_enc": 16}
 
 
-class _ViaEncEntryPoints:
-    """Stands in for libtq_b200 inside conv_codes: every original entry point is called as its _enc twin with
-    TQ_ENC_HESE."""
+class _ViaOriginalEntryPoints:
+    """Stands in for libtq_b200 inside conv_codes: every _enc entry point called with TQ_ENC_HESE goes to its original
+    entry point, the encoding dropped."""
 
     def __init__(self, L):
         self._L = L
 
     def __getattr__(self, name):
-        if name + "_enc" not in _ENC_ARG:
+        if name not in _ENC_ARG:
             return getattr(self._L, name)
-        old, fn = getattr(self._L, name), getattr(self._L, name + "_enc")
-        k = _ENC_ARG[name + "_enc"]
+        fn, old = getattr(self._L, name), getattr(self._L, name[:-len("_enc")])
+        k = _ENC_ARG[name]
         assert fn.argtypes[:k] + fn.argtypes[k + 1:] == old.argtypes and fn.argtypes[k] is ctypes.c_int, name
-        return lambda *args: fn(*args[:k], 0, *args[k:])
+
+        def call(*args):
+            assert args[k] == 0, name                    # TQ_ENC_HESE
+            return old(*args[:k], *args[k + 1:])
+        return call
 
 
 @pytest.fixture
@@ -72,13 +76,14 @@ def hese_vs_original(monkeypatch):
             return getattr(_lib, name)
 
         def lib(self):
-            return _ViaEncEntryPoints(_lib.lib())
+            return _ViaOriginalEntryPoints(_lib.lib())
 
     def run(fn):
+        new = fn()
         with monkeypatch.context() as m:
             m.setattr(conv_codes, "_lib", Shim())
-            new = fn()
-        return new, fn()
+            old = fn()
+        return new, old
     return run
 
 

@@ -1,8 +1,10 @@
 """The term encoder inside every fused epilogue, pinned to the oracle at the values where an encoder goes wrong.
 
-Each fused kernel ends with its own copy of  q = min(round_half_up(|x| / sf), 2^bits - 1) -> HESE -> keep the `terms`
-largest terms  (csrc/tq_gemm.cu: conv epilogue and one-kernel stem pool; csrc/tq_pool.cu: the pool passes;
-csrc/tq_dw.cu: depthwise, bn_act_encode, first conv).  Here the value that reaches the encoder is made equal to a set of
+Each fused kernel ends by encoding its value for the next layer's quantiser:  q = min(round_half_up(|x| / sf),
+2^bits - 1) -> HESE -> keep the `terms` largest terms, one lookup in a (q, sign) -> code table.  The quantiser, its
+checks and the table are shared (csrc/tq_common.cuh); each kernel has its own per-value loop (csrc/tq_gemm.cu: conv
+epilogue and one-kernel stem pool; csrc/tq_pool.cu: the pool passes; csrc/tq_dw.cu: depthwise, bn_act_encode, first
+conv).  Here the value that reaches the encoder is made equal to a set of
 hard values -- every rounding tie (k + 1/2) sf with its neighbours one and two ulps away, the saturation edge, zeros of
 both signs, subnormals, infinities and NaN -- and both the fp32 output and the codes must equal the CPU emulation
 (oracle/fused_emul.py, oracle/tq_oracle.c) bit for bit, across bit widths, term budgets (binding or not), scale factors
@@ -359,12 +361,12 @@ def test_rowmax_pool_against_torch(C):
 
 # ---- refusals: Python exceptions, no launch ---------------------------------------------------------------------
 
-def _refused(call, prep_launches=0):
+def _refused(call, prep_launches=0, raises=(ValueError, NotImplementedError)):
     """call raises before its kernel is launched; prep_launches: kernels the Python wrapper runs before the refusing
     C entry point (the kind::i8 engine splits the activations into planes first)."""
     from term_quantization_b200 import _lib
     n0 = _lib.launch_count()
-    with pytest.raises((ValueError, NotImplementedError)):
+    with pytest.raises(raises):
         call()
     assert _lib.launch_count() - n0 <= prep_launches
 
@@ -400,7 +402,7 @@ def test_fused_encoders_refuse_bad_quantisers():
         prep = 1 if name == "conv_i8" else 0
         for bits in (0, max_bits + 1, 12):
             _refused(lambda: call((0.5, bits, 3)), prep)
-        _refused(lambda: call((0.5, 8, -1)), prep)
+        _refused(lambda: call((0.5, 8, -1)), prep, ValueError)       # a bad argument (TQ_ERR_INVALID) everywhere
         for sf in (0.0, -1.0, float("inf"), float("nan")):
             _refused(lambda: call((sf, 8, 3)), prep)
         if name.startswith("conv_"):

@@ -354,7 +354,7 @@ def test_gather_modes_agree_at_world_size_1(resnet):
 
 # scratch-pointer argument of every stem entry point (include/tq_b200.h)
 STEM_SCRATCH_ARG = {"tq_stem_conv7x7s2": 1, "tq_stem_conv7x7s2_dt": 2, "tq_stem_conv7x7s2_rowmax": 2,
-                    "tq_stem_conv7x7s2_pool": 2, "tq_stem_conv7x7s2_u8": 3, "tq_stem_conv7x7s2_u8_rowmax": 3}
+                    "tq_stem_conv7x7s2_pool_enc": 2, "tq_stem_conv7x7s2_u8": 3, "tq_stem_conv7x7s2_u8_rowmax": 3}
 
 
 def _record_while_capturing(monkeypatch, args):
@@ -433,7 +433,7 @@ def test_captured_raw_i8_conv_keeps_its_weight_planes(monkeypatch):
     g = torch.Generator(device="cuda").manual_seed(80)
     act = torch.randint(0, 257, (2, 12, 20, 32), device="cuda", generator=g).half()
     wgt = torch.randint(-100, 101, (9, 64, 32), device="cuda", generator=g).half()
-    seen = _record_while_capturing(monkeypatch, {"tq_conv2d_planes_i8": 1})
+    seen = _record_while_capturing(monkeypatch, {"tq_conv2d_planes_i8_enc": 1})
 
     def conv():
         return conv_codes.conv2d_codes(act, wgt, None, (3, 3), 1, 1, 1.0, engine="i8")
