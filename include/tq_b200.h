@@ -398,6 +398,20 @@ int tq_lstm_recurrence(const float *gin, const float *bias, const float *w_hh, c
                        float *y, float *hn, float *cn, int T, int B, int H, void *stream);
 
 /*
+ * Per-row negative log-likelihood of a target class, read straight from the logits (one pass, no log-probability tensor):
+ *     loss[r] = logsumexp(logits[r][0:cols]) - logits[r][targets[r]]  = -log_softmax(logits[r])[targets[r]]
+ *   logits  fp32 [rows][ld] (row stride ld >= cols elements: a padded GEMM output is read in place, its pad ignored)
+ *   targets int64 [rows];  loss fp32 [rows]
+ * fp32 with accurate expf / logf and one fixed summation order per row (bit-identical from run to run and under graph
+ * replay).  Special values as torch.log_softmax + nll_loss: -inf entries add 0, a NaN or +inf in the row and an all -inf
+ * row give NaN.  A target outside [0, cols) gives a NaN loss for its row (no fault).  logits and loss 4-byte aligned,
+ * targets 8-byte aligned, rows, cols >= 1, ld >= cols, rows * ld * 4 bytes within int64; otherwise TQ_ERR_INVALID before
+ * any launch.
+ */
+int tq_log_softmax_nll(const float *logits, int64_t rows, int64_t cols, int64_t ld, const int64_t *targets, float *loss,
+                       void *stream);
+
+/*
  * Device self-test: quantises n pseudo-random (a, sf) pairs (sf in [2^-30, 2^30], a over all
  * non-negative floats and the quantiser's rounding boundaries) with the hoisted-reciprocal
  * divide and with div.rn.f32 and adds the number of disagreements to *mismatch (device).

@@ -543,3 +543,34 @@ def lstm_recurrence(gin, bias, w_hh, h0, c0):
                                            T, B, H, torch.cuda.current_stream(gin.device).cuda_stream)
     _lib.check(rc)
     return y, hn, cn
+
+
+def log_softmax_nll(logits, targets):
+    """Per-row negative log-likelihood in one read of the logits (tq_log_softmax_nll): loss[r] =
+    logsumexp(logits[r]) - logits[r, targets[r]], i.e. nll_loss(log_softmax(logits), targets, reduction='none') without
+    the log-probability tensor.  logits: fp32 CUDA [rows, cols] whose last dimension is contiguous, any row stride >= cols
+    (a column slice of a padded GEMM output is read in place); targets: int64 [rows] on the same device.  Returns fp32
+    [rows].  A target outside [0, cols) gives NaN for its row (nll_loss would raise; ignore_index is not special here)."""
+    if logits.dtype != torch.float32 or targets.dtype != torch.int64:
+        raise RuntimeError(f"log_softmax_nll expects fp32 logits and int64 targets, got {logits.dtype} and {targets.dtype}")
+    if logits.dim() != 2 or targets.dim() != 1 or targets.shape[0] != logits.shape[0]:
+        raise ValueError(f"log_softmax_nll expects logits [rows, cols] and targets [rows], got {tuple(logits.shape)} and "
+                         f"{tuple(targets.shape)}")
+    rows, cols = logits.shape
+    if rows < 1 or cols < 1:
+        raise ValueError(f"log_softmax_nll: empty logits {tuple(logits.shape)}")
+    ld = logits.stride(0) if rows > 1 else cols              # a single row's stride is arbitrary
+    if (cols > 1 and logits.stride(1) != 1) or ld < cols:
+        raise ValueError(f"log_softmax_nll expects rows of contiguous logits with a row stride >= cols, got strides "
+                         f"{logits.stride()} for {tuple(logits.shape)}")
+    if not targets.is_contiguous():
+        raise ValueError("log_softmax_nll expects contiguous targets")
+    if not logits.is_cuda or not targets.is_cuda or logits.device != targets.device:
+        raise RuntimeError(f"log_softmax_nll expects logits and targets on one CUDA device, got {logits.device} and "
+                           f"{targets.device}")
+    loss = torch.empty(rows, dtype=torch.float32, device=logits.device)
+    with torch.cuda.device(logits.device):
+        rc = _lib.lib().tq_log_softmax_nll(logits.data_ptr(), rows, cols, ld, targets.data_ptr(), loss.data_ptr(),
+                                           torch.cuda.current_stream(logits.device).cuda_stream)
+    _lib.check(rc)
+    return loss

@@ -4,7 +4,8 @@ Linear, calibrate on one pass, evaluate perplexity, count term-pair ops.
 Same flags (--wb --wt --db --dt --gs --out-file, model hyper-parameters), plus --encoding and --engine:
   float    the reference's forward (cuDNN LSTM on quantised emb / h0 / c0, fp32 decoder on the raw input)
   tcgen05  tr_layer.use_tensor_cores: layer 0's input projection and the decoder's linear(q(x)) on term codes
-  fused    fused.FusedLSTM: the tcgen05 contractions plus one persistent recurrence kernel per layer
+  fused    fused.FusedLSTM: the tcgen05 contractions plus one persistent recurrence kernel per layer; each chunk is
+           scored by FusedLSTM.nll (per-token losses summed in fp64, no [T*B, ntoken] log-probabilities)
 The corpus (train.txt is missing, .MISSING_LARGE_BLOBS) and pretrained_models/lstm.pt are unavailable, so
 tokens are synthetic (uniform over the 33,278-word vocabulary) and weights random-init.
 `--tied/--cuda` keep the reference's inverted store_false behaviour (evaluate_lstm.py:77-82)."""
@@ -95,9 +96,14 @@ def main(argv=None):
         with torch.no_grad():
             for i in range(0, source.size(0) - 1, args.bptt):
                 data, targets = get_batch(source, i)
-                output, hidden = m(data, hidden)
-                hidden = repackage_hidden(hidden)
-                total += len(data) * criterion(output, targets).item()
+                if isinstance(m, fused.FusedLSTM):
+                    # per-token losses, no log-probability tensor; sum / bsz = len(data) * the chunk's mean loss
+                    loss, hidden = m.nll(data, targets, hidden)
+                    total += loss.double().sum().item() / bsz
+                else:
+                    output, hidden = m(data, hidden)
+                    hidden = repackage_hidden(hidden)
+                    total += len(data) * criterion(output, targets).item()
         return total / (len(source) - 1)
 
     results = {'ppls': [], 'tmacs': [], 'param_bits': []}

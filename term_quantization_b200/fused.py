@@ -504,7 +504,10 @@ class FusedLSTM(nn.Module):
     weights are not term-revealed, as in the reference) and the recurrence kernel -> the decoder's linear(q(y)) on term
     codes (exact int32 accumulator, scale and bias in the epilogue) -> log_softmax.  Building the executor switches the rnn and decoder layers to their tensor-core paths (use_tensor_cores).
     The recurrence is fp32 with a fixed summation order: bit-identical from run to run and under CUDA-graph replay, within
-    1e-5 of an fp64 recurrence, not bit-comparable with cuDNN or the step-wise loop of TRLSTMLayer."""
+    1e-5 of an fp64 recurrence, not bit-comparable with cuDNN or the step-wise loop of TRLSTMLayer.
+
+    nll(input, targets, hidden) runs the same chain up to the decoder output and ends in tq_log_softmax_nll instead of
+    log_softmax: the per-token loss for perplexity, with no [T*B, ntoken] log-probability tensor."""
 
     def __init__(self, model):
         super().__init__()
@@ -542,6 +545,12 @@ class FusedLSTM(nn.Module):
                 self.layers.append((None if l == 0 else getattr(m, f"weight_ih_l{l}"), getattr(m, f"weight_hh_l{l}"), bias))
         self.dec_scale = (torch.tensor(float(dec.input_quant.sf), dtype=torch.float32)
                           * torch.tensor(dec._tc_wsf32, dtype=torch.float32)).item()
+        # the decoder bias padded to the packed weight's rows once, so that linear_codes allocates nothing next to its output
+        _, out_pad, _ = dec._tc_weight.shape
+        self.dec_bias = None
+        if dec.linear.bias is not None:
+            self.dec_bias = torch.zeros(out_pad, dtype=torch.float32, device=dec.linear.bias.device)
+            self.dec_bias[:dec.linear.out_features] = dec.linear.bias.detach()
         self._key = self._snapshot()
         self.train(False)
 
@@ -566,15 +575,11 @@ class FusedLSTM(nn.Module):
             raise RuntimeError("the wrapped model changed after fusing (weights, device or scale factors): "
                                "build the fused executor again")
 
-    @torch.no_grad()
-    def forward(self, input, hidden, capture=None):
-        """input: int64 [T, B] tokens; hidden: (h0, c0) fp32 [layers, B, H].  capture: optional dict that receives 'y'
-        (the last layer's fp32 output [T, B, H]), 'codes' (the decoder's fp16 input codes [T*B, H]) and 'decoded' (the
-        decoder's fp32 output before log_softmax)."""
-        if not torch.cuda.is_current_stream_capturing():
-            self.check_fresh()
+    def _recurrence(self, input, hidden):
+        """Embedding, the shared quantiser on h0 / c0, then every layer's input projection and recurrence kernel.
+        Returns (y [T, B, H] of the last layer, (hn, cn) [layers, B, H])."""
         model = self.model
-        rnn, dec = model.rnn, model.decoder
+        rnn = model.rnn
         emb = model.encoder(input)
         h0, c0 = (rnn.input_quant(h) for h in hidden)                 # the shared quantiser (tr_layer.py:193-194)
         T, B = input.shape
@@ -588,12 +593,48 @@ class FusedLSTM(nn.Module):
             y, h, c = conv_codes.lstm_recurrence(gin, bias, w_hh, h0[l].contiguous(), c0[l].contiguous())
             hn.append(h)
             cn.append(c)
+        return y, (torch.stack(hn), torch.stack(cn))
+
+    def _decoded(self, input, hidden):
+        """The chain forward and nll share: the recurrence, then the decoder's linear(q(y)) on term codes.  Returns
+        (decoded [T*B, ntoken] fp32, a column slice of the decoder's padded output; (hn, cn); y; the decoder's fp16 input
+        codes [T*B, H]).  The recurrence's temporaries are gone before the decoder output, the chain's largest tensor, is
+        allocated, and the codes are written at the packed weight's width so that linear_codes copies nothing."""
+        if not torch.cuda.is_current_stream_capturing():
+            self.check_fresh()
+        dec = self.model.decoder
+        y, hidden = self._recurrence(input, hidden)
+        T, B, H = y.shape
         q = dec.input_quant
-        H = y.shape[-1]
-        codes = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
-                                 encoding=q.encoding).view(T * B, H)
-        decoded = conv_codes.linear_codes(codes, dec._tc_weight, self.dec_scale, bias=dec.linear.bias,
+        codes = torch.zeros((T * B, dec._tc_weight.shape[2]), dtype=torch.float16, device=y.device)
+        codes[:, :H] = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
+                                        encoding=q.encoding).view(T * B, H)
+        decoded = conv_codes.linear_codes(codes, dec._tc_weight, self.dec_scale, bias=self.dec_bias,
                                           out_features=dec.linear.out_features, plan=dec._tc_plan)
+        return decoded, hidden, y, codes[:, :H]
+
+    @torch.no_grad()
+    def forward(self, input, hidden, capture=None):
+        """input: int64 [T, B] tokens; hidden: (h0, c0) fp32 [layers, B, H].  capture: optional dict that receives 'y'
+        (the last layer's fp32 output [T, B, H]), 'codes' (the decoder's fp16 input codes [T*B, H]) and 'decoded' (the
+        decoder's fp32 output before log_softmax)."""
+        decoded, hidden, y, codes = self._decoded(input, hidden)
         if capture is not None:
             capture["y"], capture["codes"], capture["decoded"] = y, codes, decoded
-        return F.log_softmax(decoded, dim=1), (torch.stack(hn), torch.stack(cn))
+        return F.log_softmax(decoded, dim=1), hidden
+
+    @torch.no_grad()
+    def nll(self, input, targets, hidden):
+        """Per-token negative log-likelihood of `targets` (int64 [T*B], the next tokens in forward's row order) under
+        the model: the chain of forward, then one tq_log_softmax_nll pass over the decoder's padded output.  Equals
+        nll_loss(forward(input, hidden)[0], targets, reduction='none') within the pass's fp32 bound, without
+        allocating the [T*B, ntoken] log-probabilities.  Returns (loss fp32 [T*B], (hn, cn)); a target outside
+        [0, ntoken) gives NaN for its token."""
+        T, B = input.shape
+        if targets.dtype != torch.int64 or targets.dim() != 1 or targets.shape[0] != T * B:
+            raise ValueError(f"FusedLSTM.nll expects int64 targets [T*B] = [{T * B}], got {targets.dtype} "
+                             f"{tuple(targets.shape)}")
+        if targets.device != input.device:
+            raise RuntimeError(f"FusedLSTM.nll: targets on {targets.device}, tokens on {input.device}")
+        decoded, hidden = self._decoded(input, hidden)[:2]
+        return conv_codes.log_softmax_nll(decoded, targets), hidden

@@ -7,7 +7,13 @@ g 8, alpha 12, db 8, seed 0) on its three paths, timed as CUDA-graph replays in 
 
 Then a separate eager pass splits the fused forward into phases with CUDA events, and the recurrence kernel's FFMA rate
 is set against a DERIVED fp32 rate (SMs x 128 FMA/clk x the max SM clock nvidia-smi reports; not a measured peak).
-Writes DIR/lstm_bench.json.  Usage: python tools/lstm_bench.py --out DIR [--rounds 15] [--replays 20]"""
+Writes DIR/lstm_bench.json.  Usage: python tools/lstm_bench.py --out DIR [--rounds 15] [--replays 20]
+
+--nll times the fused perplexity step instead, as alternating CUDA-graph replays of
+  forward + nll_loss   FusedLSTM.forward (log_softmax over the vocabulary) and nll_loss(reduction='none')
+  nll                  FusedLSTM.nll: the same chain, then one tq_log_softmax_nll pass over the padded decoder output
+plus the tq_log_softmax_nll kernel alone (CUDA events over many launches on the real decoder output) and its achieved
+bandwidth against the bytes it must move.  Writes DIR/lstm_nll.json."""
 import argparse
 import copy
 import json
@@ -17,6 +23,7 @@ import subprocess
 import sys
 
 import torch
+import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -93,9 +100,10 @@ def phases(f, tokens, hidden, reps):
             y, _, _ = conv_codes.lstm_recurrence(gin, bias, w_hh, h0[l].contiguous(), c0[l].contiguous())
             mark(f"layer {l} recurrence (tq_lstm_recurrence)")
         q = dec.input_quant
-        codes = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
-                                 encoding=q.encoding).view(T * B, H)
-        decoded = conv_codes.linear_codes(codes, dec._tc_weight, f.dec_scale, bias=dec.linear.bias,
+        codes = torch.zeros((T * B, dec._tc_weight.shape[2]), dtype=torch.float16, device=y.device)
+        codes[:, :H] = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
+                                        encoding=q.encoding).view(T * B, H)
+        decoded = conv_codes.linear_codes(codes, dec._tc_weight, f.dec_scale, bias=f.dec_bias,
                                           out_features=dec.linear.out_features, plan=dec._tc_plan)
         mark("decoder: encode + linear on term codes (tcgen05)")
         torch.log_softmax(decoded, dim=1)
@@ -114,11 +122,73 @@ def phases(f, tokens, hidden, reps):
     return [{"phase": k, "ms_median": statistics.median(times[k]), "ms_best": min(times[k])} for k in names]
 
 
+HBM_DATASHEET_BPS = 7.7e12          # NVIDIA HGX B200 data sheet, per GPU (not measured here)
+
+
+def nll_bench(f, tokens, hidden, targets, rounds, replays, launches=50, samples=10):
+    """The fused perplexity step with and without the vocabulary-wide log-probabilities, and the one-pass kernel alone."""
+    paths = {"forward + nll_loss": lambda: F.nll_loss(f(tokens, hidden)[0], targets, reduction="none"),
+             "nll": lambda: f.nll(tokens, targets, hidden)[0]}
+    graphs, outs = {}, {}
+    for name, fn in paths.items():
+        graphs[name], outs[name] = capture(fn)
+    samples_ms = {k: [] for k in graphs}
+    for _ in range(rounds):
+        for name, g in graphs.items():
+            samples_ms[name].append(time_replays(g, replays))
+    a, b = outs["forward + nll_loss"].double(), outs["nll"].double()
+    rel = float(((a - b).abs() / a.abs().clamp(min=1.0)).max())
+
+    cap = {}
+    f(tokens, hidden, capture=cap)
+    decoded = cap["decoded"]                                 # [T*B, V] view of the padded [T*B, Op] decoder output
+    rows, cols = decoded.shape
+    kernel, torch_pair = [], []
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for fn, acc in ((lambda: conv_codes.log_softmax_nll(decoded, targets), kernel),
+                    (lambda: F.nll_loss(torch.log_softmax(decoded, 1), targets, reduction="none"), torch_pair)):
+        for _ in range(3):
+            fn()
+        for _ in range(samples):
+            e0.record()
+            for _ in range(launches):
+                fn()
+            e1.record()
+            torch.cuda.synchronize()
+            acc.append(e0.elapsed_time(e1) / launches)
+    need = rows * cols * 4 + rows * 8 + rows * 4               # logits once, int64 targets, fp32 loss
+    k_ms = statistics.median(kernel)
+    steps = {k: {"ms_best": min(v), "ms_median": statistics.median(v),
+                 "tokens_per_s_median": T * B / statistics.median(v) * 1e3} for k, v in samples_ms.items()}
+    base, new = steps["forward + nll_loss"]["ms_median"], steps["nll"]["ms_median"]
+    return {
+        "timed_as": f"CUDA-graph replays of the whole step, {replays} per sample, {rounds} rounds alternating the two paths; "
+                    "TF32 off",
+        "paths": steps,
+        "nll_vs_forward_ms_saved_median": base - new,
+        "nll_vs_forward_speedup_median": base / new,
+        "loss_max_rel_diff_vs_forward_nll_loss": rel,
+        "kernel": {
+            "what": f"tq_log_softmax_nll on the decoder output in place ({rows} x {cols}, row stride {decoded.stride(0)}); "
+                    f"CUDA events around {launches} back-to-back launches, {samples} samples.  The {need / 1e6:.0f} MB "
+                    "read exceeds the 126 MB L2, so each launch reads mostly from HBM",
+            "ms_median": k_ms, "ms_best": min(kernel),
+            "bytes_needed": need,
+            "achieved_GBps_median": need / (k_ms * 1e-3) / 1e9,
+            "share_of_datasheet_hbm_bw": need / (k_ms * 1e-3) / HBM_DATASHEET_BPS,
+            "datasheet_hbm_bw_Bps": HBM_DATASHEET_BPS,
+        },
+        "torch_log_softmax_plus_nll_loss_same_input": {"ms_median": statistics.median(torch_pair), "ms_best": min(torch_pair),
+                                                        "how": "eager, CUDA events, same launches and samples"},
+    }
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--out", required=True, help="output directory (lstm_bench.json)")
     ap.add_argument("--rounds", type=int, default=15, help="alternating rounds; each times every path once")
     ap.add_argument("--replays", type=int, default=20, help="graph replays per timed sample")
+    ap.add_argument("--nll", action="store_true", help="time forward + nll_loss against FusedLSTM.nll (lstm_nll.json)")
     args = ap.parse_args(argv)
     if not torch.cuda.is_available():
         raise SystemExit("lstm_bench needs a CUDA device: nothing is timed on the CPU")
@@ -141,6 +211,17 @@ def main(argv=None):
         q_tc = copy.deepcopy(q)
         tr_layer.use_tensor_cores(q_tc)
         f = fused.FusedLSTM(copy.deepcopy(q))
+        if args.nll:
+            targets = torch.randint(evaluate_lstm.NTOKENS, (T * B,), device=dev, generator=gen)
+            res = {"workload": "Wikitext-2-shaped LSTM 650/650 tied, 2 layers, vocab 33,278, seq 35 x batch 80, TQ wb 8 / "
+                               "g 8 / alpha 12 / db 8 (bench_extra.py configs[4]), seed 0: one perplexity step",
+                   "gpu": info, "sms": props.multi_processor_count,
+                   **nll_bench(f, tokens, hidden, targets, args.rounds, args.replays)}
+            path = os.path.join(args.out, "lstm_nll.json")
+            with open(path, "w") as fp:
+                json.dump(res, fp, indent=1)
+            print(json.dumps(res, indent=1))
+            return
         paths = {"strict": lambda: q(tokens, hidden), "tcgen05": lambda: q_tc(tokens, hidden),
                  "fused": lambda: f(tokens, hidden)}
         graphs, outs, errors = {}, {}, {}
