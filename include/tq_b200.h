@@ -412,6 +412,36 @@ int tq_log_softmax_nll(const float *logits, int64_t rows, int64_t cols, int64_t 
                        void *stream);
 
 /*
+ * The same per-row loss straight from a linear layer on term codes, without writing its output (the language model's
+ * decoder): logits[r][c] = float(exact int32 accumulator) * scale (+ bias[c]), bit for bit the values
+ * tq_conv2d_codes_fused(_enc) / tq_conv2d_planes_i8(_enc) write for the 1 x M image (N = 1, H = 1, W = M, C = K,
+ * Cout = Op, 1x1 filter, no BatchNorm / residual / ReLU), and
+ *     loss[r] = logsumexp(logits[r][0:V]) - logits[r][targets[r]]
+ *   x_codes  fp16 [M][K] codes (K % 8 == 0) / x_planes int8 [planes_a][M][K] (K % 16 == 0)
+ *   wgt      fp16 [1][Op][K] packed weight codes / wgt_planes int8 [planes_w][1][Op][K]; Op % 4 == 0
+ *   bias     fp32 [Op] or NULL; rows [V, Op) of the weight and bias are padding, never part of any loss
+ *   targets  int64 [M];  loss fp32 [M]
+ *   workspace, workspace_bytes >= tq_linear_nll_workspace_bytes(M, Op): the caller's, per call (under stream capture
+ *   it comes from the graph's memory pool like every other buffer; the library keeps none)
+ * acc_groups, planes, act_max, wgt_max: as the conv entry points (the exactness contract above).  The decoder's
+ * epilogue keeps, per row and 32-column chunk, a running (max, sum exp(x - max)) over the live columns c < V with
+ * ex2.approx of fl(fl(x - max) * log2 e), writes one pair per row and column slice of an N tile (no fp32 tile, no codes,
+ * no TMA store) and the target logit, and a second kernel rescales the pairs to the row maximum and adds them in fp64
+ * in a fixed order.  The result is within 4e-6 * max(|ref|, 1) of an fp64 logsumexp - gather of the same logits and
+ * bit-identical from run to run, for any grid and under graph replay.  Special values and out-of-range targets as
+ * tq_log_softmax_nll (NaN, no fault).  TQ_ERR_INVALID before any launch: NULL or misaligned pointers (operands and bias
+ * 16-byte, targets 8-byte, loss 4-byte, workspace 16-byte aligned), M < 1, V < 1, V > Op, sizes that overflow int64,
+ * a workspace that is too small; TQ_ERR_UNSUPPORTED for a plan outside the streaming single-CTA conv variants.
+ */
+int64_t tq_linear_nll_workspace_bytes(int64_t M, int64_t Op);   /* -1 for M < 1, Op < 1 or sizes beyond int64 */
+int tq_linear_codes_nll(const void *x_codes, const void *wgt, int64_t M, int K, int Op, int V, float scale,
+                        const float *bias, int acc_groups, const int64_t *targets, float *loss, void *workspace,
+                        int64_t workspace_bytes, void *stream);
+int tq_linear_planes_i8_nll(const void *x_planes, const void *wgt_planes, int planes_a, int planes_w, int64_t M, int K,
+                            int Op, int V, float scale, const float *bias, int act_max, int wgt_max,
+                            const int64_t *targets, float *loss, void *workspace, int64_t workspace_bytes, void *stream);
+
+/*
  * Device self-test: quantises n pseudo-random (a, sf) pairs (sf in [2^-30, 2^30], a over all
  * non-negative floats and the quantiser's rounding boundaries) with the hoisted-reciprocal
  * divide and with div.rn.f32 and adds the number of disagreements to *mismatch (device).

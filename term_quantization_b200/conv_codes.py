@@ -265,6 +265,69 @@ def linear_codes(x_codes, wgt, scale, *, bias=None, out_features=None, plan=None
     return out if n == Op else out[:, :n]
 
 
+def linear_codes_nll(x_codes, wgt, scale, targets, *, bias=None, out_features=None, plan=None, act_max=512,
+                     signed_act=True, engine="auto"):
+    """Per-row negative log-likelihood of `targets` under the logits linear_codes(x_codes, wgt, scale, bias=bias,
+    out_features=out_features, ...) would return, without writing them (tq_linear_codes_nll / tq_linear_planes_i8_nll):
+    the decoder's epilogue reduces each row's (max, sum exp) over the first out_features columns and picks the target
+    logit, and a small kernel combines the partials.  Same operands, plan and engines as linear_codes; targets int64 [M]
+    on the same device.  Returns fp32 [M] = logsumexp(logits[r]) - logits[r, targets[r]], within 4e-6 * max(|ref|, 1)
+    of fp64 over the same logits; a target outside [0, out_features) gives NaN for its row."""
+    if x_codes.dtype != torch.float16 or wgt.dtype != torch.float16 or targets.dtype != torch.int64:
+        raise RuntimeError(f"linear_codes_nll expects fp16 codes and weights and int64 targets, got {x_codes.dtype}, "
+                           f"{wgt.dtype} and {targets.dtype}")
+    if x_codes.dim() != 2 or wgt.dim() != 3 or wgt.shape[0] != 1 or targets.dim() != 1 \
+            or targets.shape[0] != x_codes.shape[0]:
+        raise ValueError(f"linear_codes_nll expects codes [M, K], a packed weight [1, Op, Kp] and targets [M], got "
+                         f"{tuple(x_codes.shape)}, {tuple(wgt.shape)} and {tuple(targets.shape)}")
+    M, K = x_codes.shape
+    _, Op, Kp = wgt.shape
+    V = out_features if out_features is not None else Op
+    if M < 1 or K > Kp or not 1 <= V <= Op:
+        raise ValueError(f"linear_codes_nll: M = {M}, K = {K} against Kp = {Kp}, out_features = {V} against Op = {Op}: "
+                         f"need M >= 1, K <= Kp and 1 <= out_features <= Op")
+    if not targets.is_contiguous() or not wgt.is_contiguous():
+        raise ValueError("linear_codes_nll expects contiguous targets and a contiguous packed weight")
+    if bias is not None and (bias.dtype != torch.float32 or bias.dim() != 1 or bias.numel() not in (V, Op)):
+        raise ValueError(f"linear_codes_nll expects an fp32 bias of out_features or Op entries, got {bias.dtype} "
+                         f"{tuple(bias.shape)}")
+    devs = {t.device for t in (x_codes, wgt, targets) + ((bias,) if bias is not None else ())}
+    if len(devs) != 1 or not x_codes.is_cuda:
+        raise RuntimeError(f"linear_codes_nll expects every tensor on one CUDA device, got {sorted(map(str, devs))}")
+    if K != Kp or not x_codes.is_contiguous():
+        xp = torch.zeros((M, Kp), dtype=torch.float16, device=x_codes.device)
+        xp[:, :K] = x_codes
+        x_codes = xp
+    if bias is not None and bias.numel() != Op:
+        bp = torch.zeros(Op, dtype=torch.float32, device=wgt.device)
+        bp[:bias.numel()] = bias
+        bias = bp
+    elif bias is not None:
+        bias = bias.contiguous()
+    if plan is None:
+        plan = _cached_plan(wgt, act_max, signed_act, engine)
+    L = _lib.lib()
+    ws_bytes = int(L.tq_linear_nll_workspace_bytes(M, Op))
+    if ws_bytes < 0:
+        raise ValueError(f"linear_codes_nll: M = {M} rows of Op = {Op} columns overflow the workspace size")
+    workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=x_codes.device)     # per call (graph pool under capture)
+    loss = torch.empty(M, dtype=torch.float32, device=x_codes.device)
+    stream = torch.cuda.current_stream(x_codes.device).cuda_stream
+    with torch.cuda.device(x_codes.device):
+        if plan.engine == "f16":
+            rc = L.tq_linear_codes_nll(x_codes.data_ptr(), plan.wgt.data_ptr(), M, Kp, Op, V, float(scale), _ptr(bias),
+                                       int(plan.groups), targets.data_ptr(), loss.data_ptr(), workspace.data_ptr(),
+                                       ws_bytes, stream)
+        else:
+            act_planes, _ = codes_to_planes(x_codes, _planes_needed(plan.act_max))
+            rc = L.tq_linear_planes_i8_nll(act_planes.data_ptr(), plan.planes.data_ptr(), act_planes.shape[0],
+                                           plan.planes_w, M, Kp, Op, V, float(scale), _ptr(bias), int(plan.act_max),
+                                           int(plan.wgt_max), targets.data_ptr(), loss.data_ptr(), workspace.data_ptr(),
+                                           ws_bytes, stream)
+    _lib.check(rc)
+    return loss
+
+
 def pack_depthwise_weight(w, w_sf):
     """Term-revealed depthwise weight (C, 1, 3, 3) fp32 (already an integer multiple of w_sf) -> int32 [9, C] codes."""
     if w.dim() != 4 or w.shape[1] != 1 or tuple(w.shape[2:]) != (3, 3):

@@ -108,6 +108,12 @@ struct ConvGeom {
     const float *bias, *bn_a, *bn_b, *residual;
     int relu, relu6, write_f32;                 // relu6: additionally clamp at 6 (ReLU6 of the depthwise CNNs)
     NextQuant nq;
+    // loss-partials phase (epi_nll; a linear layer run as a 1 x M image, MODE 0, single CTAs, no ReLU): nll_part != NULL
+    // replaces every store by per-row (max, sum exp) partials over the columns c < nll_V and the target logit
+    const int64_t *nll_target;                  // [M] target column of each row
+    float2 *nll_part;                           // [n_tiles * nll_slices][M] (max, sum exp(x - max)) per column slice
+    float *nll_xt;                              // [M] x[r, target[r]], written by the one thread whose chunk holds it
+    int nll_V, nll_slices;                      // live columns; column slices per N tile (epilogue groups per tile)
 };
 
 // ---- PTX wrappers ---------------------------------------------------------------------------
@@ -412,6 +418,48 @@ __device__ __forceinline__ void epi_stage(float (&t)[32], const ConvGeom &g, uin
     }
 }
 
+// Loss partials (the language model's decoder): fold one 32-column chunk of a row's logits into the thread's running
+// (m, s = sum exp(x - m)) over the live columns c < V, and write x[r, target] when the target lies in the chunk.  The
+// exponential is ex2.approx of fl(fl(x - m) * log2 e): both roundings are relative to x - m, so their error, weighted by
+// each term's share of the row's sum, stays below 3u ln V (u = 2^-24; see tests/test_lstm_nll_epilogue_gpu.py).  A
+// log2 e folded into one fma with m * log2 e would add u |m| to every term of the partial, unbounded by that weighting.
+// Special values as absorb() in tq_loss.cu: -inf adds 0, NaN and +inf make s NaN.
+__device__ __forceinline__ float ex2_approx(float x)
+{
+    float r;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+    return r;
+}
+
+template <bool FULL>
+__device__ __forceinline__ void epi_nll(float (&t)[32], int c0, int V, int64_t tgt, float *xt, float &m, float &s)
+{
+    constexpr float LOG2E = 1.4426950408889634f;
+    if ((uint64_t)(tgt - c0) < 32u && tgt < V) {           // the one writer of x[r, target] (rare: a branch, no array index)
+        float v = t[0];
+#pragma unroll
+        for (int j = 1; j < 32; ++j) v = c0 + j == tgt ? t[j] : v;
+        *xt = v;
+    }
+    if (!FULL) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) t[j] = c0 + j < V ? t[j] : -INFINITY;
+    }
+    float cm = t[0];
+#pragma unroll
+    for (int j = 1; j < 32; ++j) cm = fmaxf(cm, t[j]);
+    const float mn = fmaxf(m, cm);
+    const float shift = mn == -INFINITY ? 0.0f : mn;
+#pragma unroll
+    for (int j = 0; j < 32; ++j) t[j] = ex2_approx(__fmul_rn(__fsub_rn(t[j], shift), LOG2E));
+#pragma unroll
+    for (int w = 16; w >= 1; w /= 2)
+#pragma unroll
+        for (int j = 0; j < w; ++j) t[j] = __fadd_rn(t[j], t[j + w]);
+    s = __fmaf_rn(s, ex2_approx(__fmul_rn(__fsub_rn(m, shift), LOG2E)), t[0]);
+    m = mn;
+}
+
 // MODE 0: A and B tiles stream through the stage ring.  MODE 1: all weight tiles resident in shared memory
 // (tile = filter tap, one 64-channel block), only A streams.  MODE 2 (the hi/lo stem conv): resident weights,
 // one halo load per A plane (x_hi, x_lo) covering all R filter rows, and a step table naming, per
@@ -427,7 +475,9 @@ __device__ __forceinline__ void epi_stage(float (&t)[32], const ConvGeom &g, uin
 // run-time branch would duplicate the staging code inside one kernel and cost instruction-cache misses).
 // KIND: 0 = fp16 codes, kind::f16, fp32 accumulators; 1 = s8 planes, kind::i8, s32 accumulators (MODE 0 only).
 // CG: 1 = one CTA per tile; 2 = CTA pair (MODE 4 only): the pair takes two M tiles of the same N tile, see the helpers above.
-template <int BLOCK_N, int MODE, bool RELU, int KIND, int CG = 1>
+// NLL: the loss-partials phase (epi_nll) in place of staging and stores -- its own instances, so that the registers of
+// the conv instances stay exactly as they were.
+template <int BLOCK_N, int MODE, bool RELU, int KIND, int CG = 1, bool NLL = false>
 __global__ void __launch_bounds__(GM_THREADS, 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                       const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmD,
@@ -435,6 +485,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 {
     static_assert(KIND == 0 || MODE == 0, "the s8-plane engine streams both operands (MODE 0)");
     static_assert(CG == 1 || ((MODE == 4 || MODE == 3) && KIND == 0), "the CTA pair runs the halo modes");
+    static_assert(!NLL || (MODE == 0 && CG == 1 && !RELU), "the loss phase is built for the streaming single-CTA conv");
     // MODE 2 (hi/lo stem conv): a resident weight tile stacks the hi plane (rows 0..63) on the lo plane (rows 64..127) and
     // ONE N = 128 MMA computes x * w_hi into accumulator columns [c, c + 64) and x * w_lo into [c + 64, c + 128): 64 cycles
     // instead of two N = 64 MMAs at 57 each.  The epilogue's view stays BLOCK_N = 64 output channels, four column groups.
@@ -988,9 +1039,16 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             if (carry) add_m(u_w, u_h, u_n);
             if (++acc == ACC_STAGES) { acc = 0; acc_phase ^= 1u; }
         };
+        // loss-partials phase: a 1 x M image (N = H = 1, hbox = nbox = 1), accumulator row mrow is row w0 + mrow of the
+        // linear layer
+        constexpr bool nll = NLL;
         for (int tile = tile_first; tile < total_tiles; tile += tile_step, ++it, next_tile()) {
             if (!single && (it & 1) != pair) continue;
             const int w0 = tw * g.wbox, h0 = th * g.hbox, n0 = tn * g.nbox;
+            float nll_m = -INFINITY, nll_s = 0.0f;                    // this thread's running pair over its columns of the tile
+            const int nll_r = w0 + mrow;
+            const bool nll_live = nll && mrow < g.wbox && nll_r < g.Wo;
+            const int64_t nll_t = nll_live ? __ldg(g.nll_target + nll_r) : -1;
 
             if (g.dbg_skip_epilogue) {
                 mbar_wait(&tfull_bar[acc], acc_phase);
@@ -1209,6 +1267,13 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                     }
                 }
                 TR(2, if (c0 + 32 <= g.Cout) epi_affine<true>(t, g, c0); else epi_affine<false>(t, g, c0));
+                if (nll) {                                       // no staging, no store: the partial is written per tile
+                    if (nll_live && c0 < g.nll_V) {
+                        if (c0 + 32 <= g.nll_V) epi_nll<true>(t, c0, g.nll_V, nll_t, g.nll_xt + nll_r, nll_m, nll_s);
+                        else epi_nll<false>(t, c0, g.nll_V, nll_t, g.nll_xt + nll_r, nll_m, nll_s);
+                    }
+                    continue;
+                }
                 // (b) staging: with a residual it already holds this chunk's residual tile; otherwise the previous
                 //     store of this group must have finished reading it before it is overwritten
                 TR_T0(tw0);
@@ -1231,6 +1296,10 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                     bulk_commit();
                 }
                 TR_SINCE(5, ts0);
+            }
+            if (nll_live) {                                      // slot (N tile, column slice): the same whichever CTA ran the tile
+                const int slice = single ? grp : half;
+                g.nll_part[(int64_t)(n_tile * g.nll_slices + slice) * g.Wo + nll_r] = make_float2(nll_m, nll_s);
             }
         }
 #ifdef TQ_CONV_TRACE
@@ -1365,7 +1434,7 @@ static int plan_smem(ConvGeom &g, int block_n)
     return TQ_OK;
 }
 
-template <int BLOCK_N, int MODE, int KIND = 0, int CG = 1>
+template <int BLOCK_N, int MODE, int KIND = 0, int CG = 1, bool NLL = false>
 static int launch_conv_mode(const CUtensorMap &tmA, const CUtensorMap &tmB, const CUtensorMap &tmC,
                             const CUtensorMap &tmD, const CUtensorMap &tmR, ConvGeom &g, cudaStream_t s)
 {
@@ -1375,7 +1444,8 @@ static int launch_conv_mode(const CUtensorMap &tmA, const CUtensorMap &tmB, cons
     static const int skip_tma = getenv("TQ_CONV_SKIP_TMA") ? atoi(getenv("TQ_CONV_SKIP_TMA")) : 0;
     g.dbg_skip_mma = skip_mma ? 1 : 0;
     g.dbg_skip_tma = skip_tma;
-    auto kern = g.relu ? conv_igemm_kernel<BLOCK_N, MODE, true, KIND, CG> : conv_igemm_kernel<BLOCK_N, MODE, false, KIND, CG>;
+    auto kern = NLL ? conv_igemm_kernel<BLOCK_N, MODE, false, KIND, CG, NLL>
+                    : (g.relu ? conv_igemm_kernel<BLOCK_N, MODE, true, KIND, CG> : conv_igemm_kernel<BLOCK_N, MODE, false, KIND, CG>);
     static bool attr_set[2][64] = {{false}};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1446,6 +1516,16 @@ static int pick_variant(ConvGeom &g, int block_n, int kind, bool general_prog, C
 static int launch_variant(ConvVariant v, const CUtensorMap &tmA, const CUtensorMap &tmB, const CUtensorMap &tmC,
                           const CUtensorMap &tmD, const CUtensorMap &tmR, ConvGeom &g, cudaStream_t s)
 {
+    if (g.nll_part) {                                   // the loss-partials instances (run_conv has checked the variant)
+        switch (v) {
+        case CV_64_M0: return launch_conv_mode<64, 0, 0, 1, true>(tmA, tmB, tmC, tmD, tmR, g, s);
+        case CV_128_M0: return launch_conv_mode<128, 0, 0, 1, true>(tmA, tmB, tmC, tmD, tmR, g, s);
+        case CV_256_M0: return launch_conv_mode<256, 0, 0, 1, true>(tmA, tmB, tmC, tmD, tmR, g, s);
+        case CV_I8_64: return launch_conv_mode<64, 0, 1, 1, true>(tmA, tmB, tmC, tmD, tmR, g, s);
+        case CV_I8_128: return launch_conv_mode<128, 0, 1, 1, true>(tmA, tmB, tmC, tmD, tmR, g, s);
+        default: return fail(TQ_ERR_UNSUPPORTED, "no loss-epilogue kernel variant");
+        }
+    }
     switch (v) {
     case CV_64_M0: return launch_conv_mode<64, 0>(tmA, tmB, tmC, tmD, tmR, g, s);
     case CV_64_M1: return launch_conv_mode<64, 1>(tmA, tmB, tmC, tmD, tmR, g, s);
@@ -1472,6 +1552,7 @@ struct ConvArgs {
     int kind, N, H, W, C, Cout, R, S, stride, pad, relu, acc_groups, planes_a, planes_w, device;
     float scale;
     NextQuant nq;
+    int nll;                                    // loss-partials phase (its per-call pointers are not part of the plan)
 };
 struct ConvPlan {
     ConvArgs key;
@@ -1559,7 +1640,7 @@ static int plan_conv(const ConvArgs &a, ConvPlan &pl)
     // small layers: every weight tile stays resident in shared memory and the K loop is a table of A loads
     const int taps = R * S * g.kc_blocks;
     static const bool no_prog = getenv("TQ_CONV_NO_PROG") != nullptr;
-    if (kind == 0 && g.n_groups == 1 && !no_prog && Cout <= 64 && taps <= 12) {
+    if (kind == 0 && g.n_groups == 1 && !no_prog && !a.nll && Cout <= 64 && taps <= 12) {   // (the loss phase is MODE 0)
         g.prog_steps = taps;
         g.nb_tiles = taps;
         // stride-1 filters wider than 1x1 on maps big enough to fill the tile: one halo load per tile
@@ -1658,7 +1739,16 @@ static int plan_conv(const ConvArgs &a, ConvPlan &pl)
     return TQ_OK;
 }
 
-static int run_conv(ConvArgs &a, cudaStream_t s)
+// the per-call outputs of the loss-partials phase
+struct NllOut {
+    const int64_t *target;
+    float2 *part;
+    float *xt;
+    int V;
+    int slices, slots;                          // set by run_conv from the plan: slices per N tile, slices of all tiles
+};
+
+static int run_conv(ConvArgs &a, cudaStream_t s, NllOut *nll = nullptr)
 {
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1682,6 +1772,22 @@ static int run_conv(ConvArgs &a, cudaStream_t s)
             ++g_plan_count;
         }
     }
+    if (nll) {
+        // the phase is built into the MODE 0 single-CTA variants; column slices per N tile = epilogue groups sharing a tile
+        // (two with two or three accumulator stages, four when one stage fills tensor memory, as in the kernel)
+        int block_n;
+        switch (pl.variant) {
+        case CV_64_M0: case CV_I8_64: block_n = 64; break;
+        case CV_128_M0: case CV_I8_128: block_n = 128; break;
+        case CV_256_M0: block_n = 256; break;
+        default: return fail(TQ_ERR_UNSUPPORTED, "the loss epilogue runs on the streaming single-CTA conv variants only");
+        }
+        const int acc_cols = pl.g.n_groups * block_n;
+        nll->slices = 2 * acc_cols > 512 ? 4 : 2;
+        nll->slots = pl.g.n_tiles * nll->slices;
+        pl.g.nll_target = nll->target; pl.g.nll_part = nll->part; pl.g.nll_xt = nll->xt;
+        pl.g.nll_V = nll->V; pl.g.nll_slices = nll->slices;
+    }
     return launch_variant(pl.variant, pl.tmA, pl.tmB, pl.tmC, pl.tmD, pl.tmR, pl.g, s);
 }
 
@@ -1689,11 +1795,11 @@ static int run_conv(ConvArgs &a, cudaStream_t s)
 static int check_conv_args(NextQuant &nq, const void *act, const void *wgt, const void *out_f32, const void *out_codes,
                            const void *bias, const void *bn_a, const void *bn_b, const void *residual, int N, int H, int W,
                            int C, int Cout, int R, int S, int stride, int pad, float next_sf, int next_bits, int next_terms,
-                           int next_enc, int c_align)
+                           int next_enc, int c_align, bool nll = false)
 {
     const int rc = next_quant(nq, out_codes, next_sf, next_bits, next_terms, next_enc, GM_LUT_MAX_BITS, true);
     if (rc != TQ_OK) return rc;
-    if (!act || !wgt || (!out_f32 && !out_codes)) return fail(TQ_ERR_INVALID, "NULL pointer");
+    if (!act || !wgt || (!out_f32 && !out_codes && !nll)) return fail(TQ_ERR_INVALID, "NULL pointer");
     if (N < 1 || H < 1 || W < 1 || C < 1 || Cout < 1 || R < 1 || S < 1 || stride < 1 || pad < 0)
         return fail(TQ_ERR_INVALID, "bad convolution geometry");
     if (C % c_align != 0) return fail(TQ_ERR_UNSUPPORTED, "input channels must be a multiple of %d (16-byte TMA rows), got %d", c_align, C);
@@ -1704,6 +1810,49 @@ static int check_conv_args(NextQuant &nq, const void *act, const void *wgt, cons
           (uintptr_t)bn_a | (uintptr_t)bn_b | (uintptr_t)residual) & 15u) != 0)
         return fail(TQ_ERR_INVALID, "pointers must be 16-byte aligned");
     return TQ_OK;
+}
+
+// ---- the linear layer's loss epilogue (tq_linear_codes_nll / tq_linear_planes_i8_nll) ------------------------------------
+// Workspace: x[r, target[r]] as fp32 [M] (rounded up to 16 bytes), then the (max, sum) partials as float2 [slots][M],
+// slot = N tile * slices + column slice.  Sized for four slots per 128 columns, the most any plan uses, so that the
+// caller needs to know nothing of the plan.
+int nll_combine(const float2 *part, const float *xt, const int64_t *target, float *loss, int M, int slots, int V,
+                cudaStream_t s);                                  // tq_loss.cu
+
+static int64_t nll_xt_bytes(int64_t M) { return (M * 4 + 15) & ~(int64_t)15; }
+
+static int64_t nll_workspace_bytes(int64_t M, int64_t Op)
+{
+    if (M < 1 || Op < 1 || M > INT32_MAX || Op > INT32_MAX) return -1;
+    const int64_t slots = 4 * ((Op + 127) / 128);
+    if (M > (INT64_MAX - 64) / 8 / slots) return -1;
+    return nll_xt_bytes(M) + slots * M * 8;
+}
+
+static int linear_nll(ConvArgs &a, int64_t M, int K, int Op, int V, const int64_t *targets, float *loss, void *workspace,
+                      int64_t workspace_bytes, cudaStream_t s)
+{
+    if (!targets || !loss || !workspace) return fail(TQ_ERR_INVALID, "NULL pointer");
+    if (((uintptr_t)targets & 7u) || ((uintptr_t)loss & 3u) || ((uintptr_t)workspace & 15u))
+        return fail(TQ_ERR_INVALID, "targets must be 8-byte, loss 4-byte and the workspace 16-byte aligned");
+    if (M < 1 || K < 1 || Op < 1 || V < 1 || V > Op)
+        return fail(TQ_ERR_INVALID, "M = %lld, K = %d, Op = %d, V = %d: need M, K >= 1 and 1 <= V <= Op", (long long)M, K, Op, V);
+    const int64_t need = nll_workspace_bytes(M, Op);
+    if (need < 0 || M * (int64_t)K > INT64_MAX / 2 || M * (int64_t)Op > INT64_MAX / 4)
+        return fail(TQ_ERR_INVALID, "M = %lld rows of K = %d / Op = %d columns overflow the sizes", (long long)M, K, Op);
+    if (workspace_bytes < need)
+        return fail(TQ_ERR_INVALID, "workspace of %lld bytes, %lld needed (tq_linear_nll_workspace_bytes)",
+                    (long long)workspace_bytes, (long long)need);
+    a.nll = 1;
+    NllOut o;
+    o.target = targets;
+    o.xt = static_cast<float *>(workspace);
+    o.part = reinterpret_cast<float2 *>(static_cast<uint8_t *>(workspace) + nll_xt_bytes(M));
+    o.V = V;
+    o.slices = o.slots = 0;
+    const int rc = run_conv(a, s, &o);
+    if (rc != TQ_OK) return rc;
+    return nll_combine(o.part, o.xt, targets, loss, (int)M, o.slots, V, s);
 }
 
 }  // namespace tq
@@ -1786,6 +1935,52 @@ extern "C" int tq_conv2d_planes_i8_enc(const void *act_planes, const void *wgt_p
     a.acc_groups = 1; a.planes_a = planes_a; a.planes_w = planes_w;
     a.scale = scale;
     return run_conv(a, (cudaStream_t)stream);
+}
+
+extern "C" int64_t tq_linear_nll_workspace_bytes(int64_t M, int64_t Op)
+{
+    return nll_workspace_bytes(M, Op);
+}
+
+extern "C" int tq_linear_codes_nll(const void *x_codes, const void *wgt, int64_t M, int K, int Op, int V, float scale,
+                                   const float *bias, int acc_groups, const int64_t *targets, float *loss, void *workspace,
+                                   int64_t workspace_bytes, void *stream)
+{
+    ConvArgs a;
+    memset(&a, 0, sizeof(a));
+    if (M < 1 || M > INT32_MAX) return fail(TQ_ERR_INVALID, "M = %lld rows: need 1 <= M <= 2^31 - 1", (long long)M);
+    int rc = check_conv_args(a.nq, x_codes, wgt, nullptr, nullptr, bias, nullptr, nullptr, nullptr, 1, 1, (int)M, K, Op, 1, 1,
+                             1, 0, 1.0f, 1, 0, TQ_ENC_HESE, 8, true);
+    if (rc != TQ_OK) return rc;
+    a.act = x_codes; a.wgt = wgt; a.bias = bias;
+    a.kind = 0; a.N = 1; a.H = 1; a.W = (int)M; a.C = K; a.Cout = Op; a.R = 1; a.S = 1; a.stride = 1; a.pad = 0;
+    a.acc_groups = acc_groups < 1 ? 1 : acc_groups; a.planes_a = 1; a.planes_w = 1;
+    a.scale = scale;
+    return linear_nll(a, M, K, Op, V, targets, loss, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int tq_linear_planes_i8_nll(const void *x_planes, const void *wgt_planes, int planes_a, int planes_w, int64_t M,
+                                       int K, int Op, int V, float scale, const float *bias, int act_max, int wgt_max,
+                                       const int64_t *targets, float *loss, void *workspace, int64_t workspace_bytes,
+                                       void *stream)
+{
+    ConvArgs a;
+    memset(&a, 0, sizeof(a));
+    if (M < 1 || M > INT32_MAX) return fail(TQ_ERR_INVALID, "M = %lld rows: need 1 <= M <= 2^31 - 1", (long long)M);
+    int rc = check_conv_args(a.nq, x_planes, wgt_planes, nullptr, nullptr, bias, nullptr, nullptr, nullptr, 1, 1, (int)M, K, Op,
+                             1, 1, 1, 0, 1.0f, 1, 0, TQ_ENC_HESE, 16, true);
+    if (rc != TQ_OK) return rc;
+    if (planes_a < 1 || planes_a > 2 || planes_w < 1 || planes_w > 2) return fail(TQ_ERR_INVALID, "1 or 2 planes per operand");
+    const int acap = planes_a == 2 ? 2047 : 127, wcap = planes_w == 2 ? 2047 : 127;
+    if (act_max < 1 || act_max > acap || wgt_max < 1 || wgt_max > wcap)
+        return fail(TQ_ERR_INVALID, "act_max / wgt_max must lie in 1..%d / 1..%d for %d / %d planes", acap, wcap, planes_a, planes_w);
+    if ((double)K * (double)act_max * (double)wgt_max >= 2147483648.0)
+        return fail(TQ_ERR_UNSUPPORTED, "K = %d with |a| <= %d, |w| <= %d can overflow an int32 accumulator", K, act_max, wgt_max);
+    a.act = x_planes; a.wgt = wgt_planes; a.bias = bias;
+    a.kind = 1; a.N = 1; a.H = 1; a.W = (int)M; a.C = K; a.Cout = Op; a.R = 1; a.S = 1; a.stride = 1; a.pad = 0;
+    a.acc_groups = 1; a.planes_a = planes_a; a.planes_w = planes_w;
+    a.scale = scale;
+    return linear_nll(a, M, K, Op, V, targets, loss, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // ---- operand planes and the static accumulator bound ------------------------------------------------

@@ -159,7 +159,65 @@ __global__ void __launch_bounds__(NLL_THREADS, 2) log_softmax_nll_kernel(const N
     }
 }
 
+// ---- combine of the decoder's loss partials (tq_linear_codes_nll / tq_linear_planes_i8_nll, tq_gemm.cu) ----------------
+// The conv epilogue leaves, per row r, `slots` (max m_p, sum s_p of exp(x - m_p)) partials at part[p * M + r] and the
+// target logit at xt[r].  A CTA takes 32 rows: warp w reads slots w, w + 8, ... of all 32 rows (lane = row, coalesced),
+// the row maximum M is taken exactly, every s_p is rescaled to it and summed in fp64, in a fixed order (per warp by
+// slot, then the eight warps in a tree), so the result is bit-identical for any grid and under graph replay.  fp64
+// makes the combine's own error negligible (~2^-53 per step): the loss error is that of the epilogue's fp32 partials.
+constexpr int CMB_ROWS = 32, CMB_WARPS = 8;
+
+__global__ void __launch_bounds__(CMB_ROWS * CMB_WARPS)
+nll_combine_kernel(const float2 *__restrict__ part, const float *__restrict__ xt, const int64_t *__restrict__ target,
+                   float *__restrict__ loss, int M, int slots, int V)
+{
+    __shared__ float sm[CMB_WARPS][CMB_ROWS];
+    __shared__ double ss[CMB_WARPS][CMB_ROWS];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int r = blockIdx.x * CMB_ROWS + lane;
+    const bool live = r < M;
+    float m = -INFINITY;
+    if (live)
+        for (int p = warp; p < slots; p += CMB_WARPS) m = fmaxf(m, __ldg(&part[(int64_t)p * M + r].x));
+    sm[warp][lane] = m;
+    __syncthreads();
+    float Mx = sm[0][lane];
+#pragma unroll
+    for (int w = 1; w < CMB_WARPS; ++w) Mx = fmaxf(Mx, sm[w][lane]);
+    const double shift = Mx == -INFINITY ? 0.0 : (double)Mx;  // all -inf: every s_p is 0 (exp(-inf) = 0, not NaN)
+    double S = 0.0;
+    if (live)
+        for (int p = warp; p < slots; p += CMB_WARPS) {
+            const float2 q = __ldg(&part[(int64_t)p * M + r]);
+            S += (double)q.y * exp((double)q.x - shift);    // exact difference; a NaN s_p makes S NaN
+        }
+    ss[warp][lane] = S;
+    __syncthreads();
+    if (warp == 0 && live) {
+        double w8[CMB_WARPS];
+#pragma unroll
+        for (int w = 0; w < CMB_WARPS; ++w) w8[w] = ss[w][lane];
+#pragma unroll
+        for (int w = CMB_WARPS / 2; w >= 1; w /= 2)
+#pragma unroll
+            for (int j = 0; j < w; ++j) w8[j] = w8[j] + w8[j + w];
+        const int64_t t = target[r];
+        // M = -inf: every logit -inf; M = +inf: inf - inf; a target outside [0, V) has no logit (its slot is stale)
+        loss[r] = (isfinite(Mx) && t >= 0 && t < V) ? (float)(((double)Mx - (double)xt[r]) + log(w8[0])) : NAN;
+    }
+}
+
 }  // namespace
+
+int nll_combine(const float2 *part, const float *xt, const int64_t *target, float *loss, int M, int slots, int V,
+                cudaStream_t s)
+{
+    nll_combine_kernel<<<(unsigned)((M + CMB_ROWS - 1) / CMB_ROWS), CMB_ROWS * CMB_WARPS, 0, s>>>(part, xt, target, loss, M,
+                                                                                                 slots, V);
+    count_launch();
+    return check_launch("nll_combine_kernel");
+}
+
 }  // namespace tq
 
 using namespace tq;

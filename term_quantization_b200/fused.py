@@ -506,8 +506,9 @@ class FusedLSTM(nn.Module):
     The recurrence is fp32 with a fixed summation order: bit-identical from run to run and under CUDA-graph replay, within
     1e-5 of an fp64 recurrence, not bit-comparable with cuDNN or the step-wise loop of TRLSTMLayer.
 
-    nll(input, targets, hidden) runs the same chain up to the decoder output and ends in tq_log_softmax_nll instead of
-    log_softmax: the per-token loss for perplexity, with no [T*B, ntoken] log-probability tensor."""
+    nll(input, targets, hidden) runs the same chain up to the decoder's input codes and ends in the decoder with the loss
+    epilogue (conv_codes.linear_codes_nll): the per-token loss for perplexity, with neither the [T*B, ntoken] logits nor
+    the log-probabilities ever written."""
 
     def __init__(self, model):
         super().__init__()
@@ -580,26 +581,25 @@ class FusedLSTM(nn.Module):
         Returns (y [T, B, H] of the last layer, (hn, cn) [layers, B, H])."""
         model = self.model
         rnn = model.rnn
-        emb = model.encoder(input)
         h0, c0 = (rnn.input_quant(h) for h in hidden)                 # the shared quantiser (tr_layer.py:193-194)
         T, B = input.shape
         hn, cn = [], []
         y = None
         for l, (w_ih, w_hh, bias) in enumerate(self.layers):
             if l == 0:
-                gin = rnn.input_projection(emb)
+                gin = rnn.input_projection(model.encoder(input))       # (the embedding is freed with the projection)
             else:
                 gin = torch.mm(y.view(T * B, -1), w_ih.t()).view(T, B, -1)
             y, h, c = conv_codes.lstm_recurrence(gin, bias, w_hh, h0[l].contiguous(), c0[l].contiguous())
+            del gin                                                     # before the next layer's projection is allocated
             hn.append(h)
             cn.append(c)
         return y, (torch.stack(hn), torch.stack(cn))
 
-    def _decoded(self, input, hidden):
-        """The chain forward and nll share: the recurrence, then the decoder's linear(q(y)) on term codes.  Returns
-        (decoded [T*B, ntoken] fp32, a column slice of the decoder's padded output; (hn, cn); y; the decoder's fp16 input
-        codes [T*B, H]).  The recurrence's temporaries are gone before the decoder output, the chain's largest tensor, is
-        allocated, and the codes are written at the packed weight's width so that linear_codes copies nothing."""
+    def _decoder_codes(self, input, hidden):
+        """The chain forward and nll share: the recurrence, then the decoder's input quantiser.  Returns (the decoder's
+        fp16 input codes [T*B, Kp] at the packed weight's width, so that the decoder copies nothing; (hn, cn); y).  The
+        recurrence's temporaries are gone before the decoder runs."""
         if not torch.cuda.is_current_stream_capturing():
             self.check_fresh()
         dec = self.model.decoder
@@ -609,9 +609,16 @@ class FusedLSTM(nn.Module):
         codes = torch.zeros((T * B, dec._tc_weight.shape[2]), dtype=torch.float16, device=y.device)
         codes[:, :H] = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
                                         encoding=q.encoding).view(T * B, H)
+        return codes, hidden, y
+
+    def _decoded(self, input, hidden):
+        """_decoder_codes, then the decoder's linear(q(y)) on term codes.  Returns (decoded [T*B, ntoken] fp32, a column
+        slice of the decoder's padded output; (hn, cn); y; the decoder's fp16 input codes [T*B, H])."""
+        codes, hidden, y = self._decoder_codes(input, hidden)
+        dec = self.model.decoder
         decoded = conv_codes.linear_codes(codes, dec._tc_weight, self.dec_scale, bias=self.dec_bias,
                                           out_features=dec.linear.out_features, plan=dec._tc_plan)
-        return decoded, hidden, y, codes[:, :H]
+        return decoded, hidden, y, codes[:, :y.shape[2]]
 
     @torch.no_grad()
     def forward(self, input, hidden, capture=None):
@@ -626,15 +633,19 @@ class FusedLSTM(nn.Module):
     @torch.no_grad()
     def nll(self, input, targets, hidden):
         """Per-token negative log-likelihood of `targets` (int64 [T*B], the next tokens in forward's row order) under
-        the model: the chain of forward, then one tq_log_softmax_nll pass over the decoder's padded output.  Equals
-        nll_loss(forward(input, hidden)[0], targets, reduction='none') within the pass's fp32 bound, without
-        allocating the [T*B, ntoken] log-probabilities.  Returns (loss fp32 [T*B], (hn, cn)); a target outside
-        [0, ntoken) gives NaN for its token."""
+        the model: the chain of forward up to the decoder's input codes, then the decoder with the loss epilogue
+        (conv_codes.linear_codes_nll), which reduces each row of logits inside the decoder and never writes them.
+        Equals nll_loss(forward(input, hidden)[0], targets, reduction='none') within 4e-6 * max(|ref|, 1) of fp64 over
+        the decoder output, without allocating any [T*B, ntoken] tensor.  Returns (loss fp32 [T*B], (hn, cn)); a target
+        outside [0, ntoken) gives NaN for its token."""
         T, B = input.shape
         if targets.dtype != torch.int64 or targets.dim() != 1 or targets.shape[0] != T * B:
             raise ValueError(f"FusedLSTM.nll expects int64 targets [T*B] = [{T * B}], got {targets.dtype} "
                              f"{tuple(targets.shape)}")
         if targets.device != input.device:
             raise RuntimeError(f"FusedLSTM.nll: targets on {targets.device}, tokens on {input.device}")
-        decoded, hidden = self._decoded(input, hidden)[:2]
-        return conv_codes.log_softmax_nll(decoded, targets), hidden
+        codes, hidden, _ = self._decoder_codes(input, hidden)
+        dec = self.model.decoder
+        loss = conv_codes.linear_codes_nll(codes, dec._tc_weight, self.dec_scale, targets, bias=self.dec_bias,
+                                           out_features=dec.linear.out_features, plan=dec._tc_plan)
+        return loss, hidden

@@ -10,12 +10,14 @@ is set against a DERIVED fp32 rate (SMs x 128 FMA/clk x the max SM clock nvidia-
 Writes DIR/lstm_bench.json.  Usage: python tools/lstm_bench.py --out DIR [--rounds 15] [--replays 20]
 
 --nll times the fused perplexity step instead, as alternating CUDA-graph replays of
-  forward + nll_loss   FusedLSTM.forward (log_softmax over the vocabulary) and nll_loss(reduction='none')
-  nll                  FusedLSTM.nll: the same chain, then one tq_log_softmax_nll pass over the padded decoder output
-plus the tq_log_softmax_nll kernel alone (CUDA events over many launches on the real decoder output) and its achieved
-bandwidth against the bytes it must move.  Writes DIR/lstm_nll.json."""
+  forward + nll_loss                FusedLSTM.forward (log_softmax over the vocabulary) and nll_loss(reduction='none')
+  decoder output + log_softmax_nll  the chain up to the padded decoder output, then one tq_log_softmax_nll pass over it
+  nll                               FusedLSTM.nll: the decoder's loss epilogue, no [T*B, V] tensor written at all
+with the peak memory of each, plus the decoder with its loss epilogue against the decoder followed by
+tq_log_softmax_nll (CUDA events over many calls).  Writes DIR/lstm_nll_epilogue.json."""
 import argparse
 import copy
+import gc
 import json
 import os
 import statistics
@@ -122,12 +124,42 @@ def phases(f, tokens, hidden, reps):
     return [{"phase": k, "ms_median": statistics.median(times[k]), "ms_best": min(times[k])} for k in names]
 
 
-HBM_DATASHEET_BPS = 7.7e12          # NVIDIA HGX B200 data sheet, per GPU (not measured here)
+def _events(fn, launches, samples):
+    """Median and best ms per call of fn over `samples` windows of `launches` back-to-back calls (CUDA events)."""
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(3):
+        fn()
+    acc = []
+    for _ in range(samples):
+        e0.record()
+        for _ in range(launches):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        acc.append(e0.elapsed_time(e1) / launches)
+    return {"ms_median": statistics.median(acc), "ms_best": min(acc), "ms_spread": max(acc) - min(acc)}
+
+
+def peak_rise(fn):
+    """Bytes the caching allocator's peak rises above what is allocated before an eager call of fn."""
+    gc.collect()
+    torch.cuda.synchronize()
+    torch.cuda.empty_cache()
+    torch.cuda.reset_peak_memory_stats()
+    base = torch.cuda.memory_allocated()
+    out = fn()
+    torch.cuda.synchronize()
+    rise = torch.cuda.max_memory_allocated() - base
+    del out
+    return rise
 
 
 def nll_bench(f, tokens, hidden, targets, rounds, replays, launches=50, samples=10):
-    """The fused perplexity step with and without the vocabulary-wide log-probabilities, and the one-pass kernel alone."""
+    """The fused perplexity step three ways, and the decoder with its loss epilogue against the decoder + one-pass loss."""
+    dec = f.model.decoder
+    V = dec.linear.out_features
     paths = {"forward + nll_loss": lambda: F.nll_loss(f(tokens, hidden)[0], targets, reduction="none"),
+             "decoder output + log_softmax_nll": lambda: conv_codes.log_softmax_nll(f._decoded(tokens, hidden)[0], targets),
              "nll": lambda: f.nll(tokens, targets, hidden)[0]}
     graphs, outs = {}, {}
     for name, fn in paths.items():
@@ -136,50 +168,46 @@ def nll_bench(f, tokens, hidden, targets, rounds, replays, launches=50, samples=
     for _ in range(rounds):
         for name, g in graphs.items():
             samples_ms[name].append(time_replays(g, replays))
-    a, b = outs["forward + nll_loss"].double(), outs["nll"].double()
-    rel = float(((a - b).abs() / a.abs().clamp(min=1.0)).max())
+    ref = outs["forward + nll_loss"].double()
+    rel = {k: float(((outs[k].double() - ref).abs() / ref.abs().clamp(min=1.0)).max()) for k in outs}
+    peaks = {k: peak_rise(fn) for k, fn in paths.items()}
 
-    cap = {}
-    f(tokens, hidden, capture=cap)
-    decoded = cap["decoded"]                                 # [T*B, V] view of the padded [T*B, Op] decoder output
-    rows, cols = decoded.shape
-    kernel, torch_pair = [], []
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for fn, acc in ((lambda: conv_codes.log_softmax_nll(decoded, targets), kernel),
-                    (lambda: F.nll_loss(torch.log_softmax(decoded, 1), targets, reduction="none"), torch_pair)):
-        for _ in range(3):
-            fn()
-        for _ in range(samples):
-            e0.record()
-            for _ in range(launches):
-                fn()
-            e1.record()
-            torch.cuda.synchronize()
-            acc.append(e0.elapsed_time(e1) / launches)
-    need = rows * cols * 4 + rows * 8 + rows * 4               # logits once, int64 targets, fp32 loss
-    k_ms = statistics.median(kernel)
-    steps = {k: {"ms_best": min(v), "ms_median": statistics.median(v),
-                 "tokens_per_s_median": T * B / statistics.median(v) * 1e3} for k, v in samples_ms.items()}
-    base, new = steps["forward + nll_loss"]["ms_median"], steps["nll"]["ms_median"]
+    codes = f._decoder_codes(tokens, hidden)[0]              # the decoder's fp16 input codes [T*B, Kp]
+    plan, w, scale, bias = dec._tc_plan, dec._tc_weight, f.dec_scale, f.dec_bias
+    kernels = {
+        "decoder + loss epilogue (linear_codes_nll)":
+            lambda: conv_codes.linear_codes_nll(codes, w, scale, targets, bias=bias, out_features=V, plan=plan),
+        "decoder (linear_codes) + tq_log_softmax_nll":
+            lambda: conv_codes.log_softmax_nll(conv_codes.linear_codes(codes, w, scale, bias=bias, out_features=V,
+                                                                       plan=plan), targets),
+        "decoder alone (linear_codes)": lambda: conv_codes.linear_codes(codes, w, scale, bias=bias, out_features=V,
+                                                                        plan=plan),
+    }
+    k_times = {}
+    for _ in range(2):                                        # alternating, twice: the spread between windows is reported
+        for k, fn in kernels.items():
+            k_times.setdefault(k, []).append(_events(fn, launches, samples))
+    k_res = {k: {"ms_median": statistics.median(r["ms_median"] for r in v), "ms_best": min(r["ms_best"] for r in v),
+                 "ms_spread": max(max(r["ms_median"] for r in v) - min(r["ms_median"] for r in v),
+                                  max(r["ms_spread"] for r in v))} for k, v in k_times.items()}
+    steps = {k: {"ms_best": min(v), "ms_median": statistics.median(v), "ms_spread": max(v) - min(v),
+                 "tokens_per_s_median": T * B / statistics.median(v) * 1e3,
+                 "peak_memory_rise_bytes": peaks[k], "loss_max_rel_diff_vs_forward_nll_loss": rel[k]}
+             for k, v in samples_ms.items()}
+    r05, new = steps["decoder output + log_softmax_nll"]["ms_median"], steps["nll"]["ms_median"]
     return {
-        "timed_as": f"CUDA-graph replays of the whole step, {replays} per sample, {rounds} rounds alternating the two paths; "
-                    "TF32 off",
+        "timed_as": f"CUDA-graph replays of the whole step, {replays} per sample, {rounds} rounds alternating the three "
+                    "paths; TF32 off.  Peak memory: eager call, rise of max_memory_allocated above the allocation before it",
         "paths": steps,
-        "nll_vs_forward_ms_saved_median": base - new,
-        "nll_vs_forward_speedup_median": base / new,
-        "loss_max_rel_diff_vs_forward_nll_loss": rel,
-        "kernel": {
-            "what": f"tq_log_softmax_nll on the decoder output in place ({rows} x {cols}, row stride {decoded.stride(0)}); "
-                    f"CUDA events around {launches} back-to-back launches, {samples} samples.  The {need / 1e6:.0f} MB "
-                    "read exceeds the 126 MB L2, so each launch reads mostly from HBM",
-            "ms_median": k_ms, "ms_best": min(kernel),
-            "bytes_needed": need,
-            "achieved_GBps_median": need / (k_ms * 1e-3) / 1e9,
-            "share_of_datasheet_hbm_bw": need / (k_ms * 1e-3) / HBM_DATASHEET_BPS,
-            "datasheet_hbm_bw_Bps": HBM_DATASHEET_BPS,
+        "nll_vs_r05_path_ms_saved_median": r05 - new,
+        "nll_vs_r05_path_speedup_median": r05 / new,
+        "logits_bytes": T * B * V * 4,
+        "decoder_kernels": {
+            "how": f"eager, CUDA events around {launches} back-to-back calls, {samples} samples, two alternating passes; "
+                   f"{T * B} x {V} logits from K = {codes.shape[1]} codes on the '{plan.engine}' engine "
+                   f"({plan.groups} K chunk(s)); ms_spread: the widest gap between samples or passes",
+            **k_res,
         },
-        "torch_log_softmax_plus_nll_loss_same_input": {"ms_median": statistics.median(torch_pair), "ms_best": min(torch_pair),
-                                                        "how": "eager, CUDA events, same launches and samples"},
     }
 
 
@@ -188,7 +216,7 @@ def main(argv=None):
     ap.add_argument("--out", required=True, help="output directory (lstm_bench.json)")
     ap.add_argument("--rounds", type=int, default=15, help="alternating rounds; each times every path once")
     ap.add_argument("--replays", type=int, default=20, help="graph replays per timed sample")
-    ap.add_argument("--nll", action="store_true", help="time forward + nll_loss against FusedLSTM.nll (lstm_nll.json)")
+    ap.add_argument("--nll", action="store_true", help="time the three perplexity paths (lstm_nll_epilogue.json)")
     args = ap.parse_args(argv)
     if not torch.cuda.is_available():
         raise SystemExit("lstm_bench needs a CUDA device: nothing is timed on the CPU")
@@ -217,7 +245,7 @@ def main(argv=None):
                                "g 8 / alpha 12 / db 8 (bench_extra.py configs[4]), seed 0: one perplexity step",
                    "gpu": info, "sms": props.multi_processor_count,
                    **nll_bench(f, tokens, hidden, targets, args.rounds, args.replays)}
-            path = os.path.join(args.out, "lstm_nll.json")
+            path = os.path.join(args.out, "lstm_nll_epilogue.json")
             with open(path, "w") as fp:
                 json.dump(res, fp, indent=1)
             print(json.dumps(res, indent=1))
