@@ -398,6 +398,28 @@ int tq_lstm_recurrence(const float *gin, const float *bias, const float *w_hh, c
                        float *y, float *hn, float *cn, int T, int B, int H, void *stream);
 
 /*
+ * The same persistent recurrence for the other cells of nn.GRU / nn.RNN (one unidirectional layer, torch's gate order
+ * and formulas), the same kernel template, numerics, layout and refusals as tq_lstm_recurrence:
+ *   GRU (gates r, z, n):  gin fp32 [T][B][3H] = W_ih x_t + b_ih;  b_hh fp32 [3H] or NULL;  w_hh fp32 [3H][H]
+ *       r = sig(gin_r + b_hr + W_hr h),  z = sig(gin_z + b_hz + W_hz h),  n = tanh(gin_n + r * (W_hn h + b_hn)),
+ *       h_t = n + z * (h_{t-1} - n)
+ *   RNN:  gin fp32 [T][B][H] = W_ih x_t;  bias fp32 [H] (b_ih + b_hh) or NULL;  w_hh fp32 [H][H]
+ *       h_t = act(gin + bias + W_hh h),  act = relu ? ReLU (a NaN stays NaN, as torch.relu) : tanh
+ *   h0 fp32 [B][H];  y fp32 [T][B][H] = h_t;  hn fp32 [B][H] = h_T
+ * Each CTA keeps the G gate rows (G = 3 / 1) of ceil(H / SMs) units in shared memory, so the bound on H grows as G
+ * shrinks (B200: GRU H <= 1628, RNN H <= 2812).  TQ_ERR_INVALID for NULL or misaligned pointers, T, B or H below 1 and
+ * B * G * H above 2^31 - 1; TQ_ERR_UNSUPPORTED (the message names the largest H) above the bound; all before any launch.
+ */
+int tq_gru_recurrence(const float *gin, const float *b_hh, const float *w_hh, const float *h0, float *y, float *hn,
+                      int T, int B, int H, void *stream);
+int tq_rnn_recurrence(const float *gin, const float *bias, const float *w_hh, const float *h0, float *y, float *hn,
+                      int T, int B, int H, int relu, void *stream);
+
+/* Largest H the recurrence of a cell with `gates` gate rows per unit (4 LSTM, 3 GRU, 1 RNN) takes on the current
+ * device; -1 (TQ_ERR_INVALID / TQ_ERR_CUDA in tq_last_error) for another gate count or an unreadable device. */
+int tq_recurrence_max_hidden(int gates);
+
+/*
  * Per-row negative log-likelihood of a target class, read straight from the logits (one pass, no log-probability tensor):
  *     loss[r] = logsumexp(logits[r][0:cols]) - logits[r][targets[r]]  = -log_softmax(logits[r])[targets[r]]
  *   logits  fp32 [rows][ld] (row stride ld >= cols elements: a padded GEMM output is read in place, its pad ignored)

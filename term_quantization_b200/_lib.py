@@ -65,6 +65,9 @@ SYMBOLS = {
     "tq_bn_relu_maxpool_encode_rowmax": (_i, [_p] * 5 + [_i] * 5 + [_f, _i, _i, _p]),
     "tq_bn_relu_maxpool_encode_rowmax_enc": (_i, [_p] * 5 + [_i] * 5 + [_f, _i, _i, _i, _p]),
     "tq_lstm_recurrence": (_i, [_p] * 8 + [_i, _i, _i, _p]),
+    "tq_gru_recurrence": (_i, [_p] * 6 + [_i, _i, _i, _p]),
+    "tq_rnn_recurrence": (_i, [_p] * 6 + [_i, _i, _i, _i, _p]),
+    "tq_recurrence_max_hidden": (_i, [_i]),
     "tq_log_softmax_nll": (_i, [_p, _i64, _i64, _i64, _p, _p, _p]),
     "tq_linear_nll_workspace_bytes": (_i64, [_i64, _i64]),
     "tq_linear_codes_nll": (_i, [_p, _p, _i64, _i, _i, _i, _f, _p, _i, _p, _p, _p, _i64, _p]),

@@ -568,35 +568,53 @@ def stem_conv_pool(x_nhwc, w2, bn, relu=True, next_quant=None, scratch=None):
     return out, codes, scratch
 
 
+# gate rows per hidden unit of each RNNModel cell: the recurrence kernel keeps this many rows of W_hh per unit
+RECURRENCE_GATES = {"LSTM": 4, "GRU": 3, "RNN_TANH": 1, "RNN_RELU": 1}
+
+
+def recurrence_max_hidden(cell, device=None):
+    """Largest hidden size the recurrence kernel of `cell` ('LSTM', 'GRU', 'RNN_TANH' or 'RNN_RELU') takes on `device`:
+    each CTA keeps the gate rows of ceil(H / SMs) units in shared memory next to one hidden row and 2 KB of gate
+    scratch.  The library computes it (tq_recurrence_max_hidden), the same number its refusals name."""
+    if cell not in RECURRENCE_GATES:
+        raise ValueError(f"unknown recurrent cell {cell!r}: expected one of {', '.join(RECURRENCE_GATES)}")
+    with torch.cuda.device(device if device is not None else torch.cuda.current_device()):
+        n = _lib.lib().tq_recurrence_max_hidden(RECURRENCE_GATES[cell])
+    if n < 0:
+        raise _lib.TQError(f"tq_b200: {_lib.lib().tq_last_error().decode('utf-8', 'replace')}")
+    return n
+
+
 def lstm_max_hidden(device=None):
-    """Largest hidden size tq_lstm_recurrence takes on `device`: each CTA keeps the 4 gate rows of ceil(H / SMs) units
-    in shared memory next to one hidden row and 2 KB of gate scratch (csrc/tq_lstm.cu, lstm_fits)."""
-    props = torch.cuda.get_device_properties(device if device is not None else torch.cuda.current_device())
-    sms, optin = props.multi_processor_count, props.shared_memory_per_block_optin
-    best = 0
-    for h in range(1, 65537):
-        if (4 * (-(-h // sms)) + 1) * h * 4 + 2048 <= optin:
-            best = h
-    return best
+    """Largest hidden size tq_lstm_recurrence takes on `device` (recurrence_max_hidden('LSTM'))."""
+    return recurrence_max_hidden("LSTM", device)
+
+
+def _recurrence_shapes(name, gates, gin, bias, w_hh, h0, c0=None):
+    """The checks every recurrence wrapper makes before the library is reached; returns (T, B, H)."""
+    ts = [t for t in (gin, bias, w_hh, h0, c0) if t is not None]
+    if any(not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() for t in ts):
+        raise RuntimeError(f"{name} expects contiguous fp32 CUDA tensors")
+    if any(t.device != gin.device for t in ts):
+        raise RuntimeError(f"{name}: every tensor must be on the same device")
+    gh = f"{gates}H" if gates > 1 else "H"
+    if gin.dim() != 3 or w_hh.dim() != 2:
+        raise RuntimeError(f"{name} expects gin [T, B, {gh}] and w_hh [{gh}, H]")
+    T, B, G = gin.shape
+    H = w_hh.shape[1]
+    if G != gates * H or tuple(w_hh.shape) != (gates * H, H) or tuple(h0.shape) != (B, H) \
+            or (c0 is not None and tuple(c0.shape) != (B, H)) or (bias is not None and tuple(bias.shape) != (gates * H,)):
+        raise RuntimeError(f"{name}: shapes gin {tuple(gin.shape)}, w_hh {tuple(w_hh.shape)}, h0 {tuple(h0.shape)}, "
+                           + (f"c0 {tuple(c0.shape)}, " if c0 is not None else "")
+                           + f"bias {None if bias is None else tuple(bias.shape)} do not agree")
+    return T, B, H
 
 
 def lstm_recurrence(gin, bias, w_hh, h0, c0):
     """All T steps of one LSTM layer in one launch (tq_lstm_recurrence): gin fp32 [T, B, 4H] (W_ih x_t, torch gate order
     i, f, g, o), bias fp32 [4H] (b_ih + b_hh) or None, w_hh fp32 [4H, H], h0 / c0 fp32 [B, H].
     Returns (y [T, B, H], hn [B, H], cn [B, H]), fp32 with a fixed summation order."""
-    ts = [t for t in (gin, bias, w_hh, h0, c0) if t is not None]
-    if any(not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() for t in ts):
-        raise RuntimeError("lstm_recurrence expects contiguous fp32 CUDA tensors")
-    if any(t.device != gin.device for t in ts):
-        raise RuntimeError("lstm_recurrence: every tensor must be on the same device")
-    if gin.dim() != 3 or w_hh.dim() != 2:
-        raise RuntimeError("lstm_recurrence expects gin [T, B, 4H] and w_hh [4H, H]")
-    T, B, G = gin.shape
-    H = w_hh.shape[1]
-    if G != 4 * H or tuple(w_hh.shape) != (4 * H, H) or tuple(h0.shape) != (B, H) or tuple(c0.shape) != (B, H) \
-            or (bias is not None and tuple(bias.shape) != (4 * H,)):
-        raise RuntimeError(f"lstm_recurrence: shapes gin {tuple(gin.shape)}, w_hh {tuple(w_hh.shape)}, h0 {tuple(h0.shape)}, "
-                           f"c0 {tuple(c0.shape)}, bias {None if bias is None else tuple(bias.shape)} do not agree")
+    T, B, H = _recurrence_shapes("lstm_recurrence", 4, gin, bias, w_hh, h0, c0)
     y = torch.empty((T, B, H), dtype=torch.float32, device=gin.device)
     hn = torch.empty((B, H), dtype=torch.float32, device=gin.device)
     cn = torch.empty((B, H), dtype=torch.float32, device=gin.device)
@@ -606,6 +624,40 @@ def lstm_recurrence(gin, bias, w_hh, h0, c0):
                                            T, B, H, torch.cuda.current_stream(gin.device).cuda_stream)
     _lib.check(rc)
     return y, hn, cn
+
+
+def gru_recurrence(gin, b_hh, w_hh, h0):
+    """All T steps of one GRU layer in one launch (tq_gru_recurrence): gin fp32 [T, B, 3H] (W_ih x_t + b_ih, torch gate
+    order r, z, n), b_hh fp32 [3H] or None, w_hh fp32 [3H, H], h0 fp32 [B, H].  b_hn stays inside the reset gate's
+    product: n = tanh(gin_n + r * (W_hn h + b_hn)).  Returns (y [T, B, H], hn [B, H]), fp32 with a fixed summation
+    order."""
+    T, B, H = _recurrence_shapes("gru_recurrence", 3, gin, b_hh, w_hh, h0)
+    y = torch.empty((T, B, H), dtype=torch.float32, device=gin.device)
+    hn = torch.empty((B, H), dtype=torch.float32, device=gin.device)
+    with torch.cuda.device(gin.device):
+        rc = _lib.lib().tq_gru_recurrence(gin.data_ptr(), b_hh.data_ptr() if b_hh is not None else None, w_hh.data_ptr(),
+                                          h0.data_ptr(), y.data_ptr(), hn.data_ptr(), T, B, H,
+                                          torch.cuda.current_stream(gin.device).cuda_stream)
+    _lib.check(rc)
+    return y, hn
+
+
+def rnn_recurrence(gin, bias, w_hh, h0, nonlinearity):
+    """All T steps of one vanilla RNN layer in one launch (tq_rnn_recurrence): h_t = act(gin[t] + bias + W_hh h_{t-1})
+    with gin fp32 [T, B, H] (W_ih x_t), bias fp32 [H] (b_ih + b_hh) or None, w_hh fp32 [H, H], h0 fp32 [B, H] and
+    nonlinearity 'tanh' or 'relu' (a NaN stays NaN, as torch.relu).  Returns (y [T, B, H], hn [B, H]), fp32 with a
+    fixed summation order."""
+    if nonlinearity not in ("tanh", "relu"):
+        raise ValueError(f"rnn_recurrence: nonlinearity {nonlinearity!r} is neither 'tanh' nor 'relu'")
+    T, B, H = _recurrence_shapes("rnn_recurrence", 1, gin, bias, w_hh, h0)
+    y = torch.empty((T, B, H), dtype=torch.float32, device=gin.device)
+    hn = torch.empty((B, H), dtype=torch.float32, device=gin.device)
+    with torch.cuda.device(gin.device):
+        rc = _lib.lib().tq_rnn_recurrence(gin.data_ptr(), bias.data_ptr() if bias is not None else None, w_hh.data_ptr(),
+                                          h0.data_ptr(), y.data_ptr(), hn.data_ptr(), T, B, H,
+                                          int(nonlinearity == "relu"), torch.cuda.current_stream(gin.device).cuda_stream)
+    _lib.check(rc)
+    return y, hn
 
 
 def log_softmax_nll(logits, targets):

@@ -4,8 +4,10 @@ Linear, calibrate on one pass, evaluate perplexity, count term-pair ops.
 Same flags (--wb --wt --db --dt --gs --out-file, model hyper-parameters), plus --encoding and --engine:
   float    the reference's forward (cuDNN LSTM on quantised emb / h0 / c0, fp32 decoder on the raw input)
   tcgen05  tr_layer.use_tensor_cores: layer 0's input projection and the decoder's linear(q(x)) on term codes
-  fused    fused.FusedLSTM: the tcgen05 contractions plus one persistent recurrence kernel per layer; each chunk is
-           scored by FusedLSTM.nll (per-token losses summed in fp64, no [T*B, ntoken] log-probabilities)
+  fused    fused.FusedLSTM (--model LSTM) or fused.FusedRNN (GRU, RNN_TANH, RNN_RELU): the tcgen05 contractions plus
+           one persistent recurrence kernel per layer; each chunk is scored by the executor's nll (per-token losses
+           summed in fp64, no [T*B, ntoken] log-probabilities)
+For GRU and RNN models only the decoder is a TR layer (only nn.Linear and nn.LSTM are wrapped), as in the reference.
 The corpus (train.txt is missing, .MISSING_LARGE_BLOBS) and pretrained_models/lstm.pt are unavailable, so
 tokens are synthetic (uniform over the 33,278-word vocabulary) and weights random-init.
 `--tied/--cuda` keep the reference's inverted store_false behaviour (evaluate_lstm.py:77-82)."""
@@ -70,7 +72,7 @@ def main(argv=None):
                         help='term encoding of every wrapped layer (hese = the reference)')
     parser.add_argument('--engine', default='float', choices=['float', 'tcgen05', 'fused'],
                         help='float: the reference forward; tcgen05: input projection and decoder on term codes; '
-                             'fused: FusedLSTM (tcgen05 contractions, one recurrence kernel per layer)')
+                             'fused: FusedLSTM / FusedRNN (tcgen05 contractions, one recurrence kernel per layer)')
     parser.add_argument('--tokens', type=int, default=35 * 10 * 4 + 10, help='synthetic test tokens')
     args = parser.parse_args(argv)
     if not args.cuda or not torch.cuda.is_available():
@@ -96,7 +98,7 @@ def main(argv=None):
         with torch.no_grad():
             for i in range(0, source.size(0) - 1, args.bptt):
                 data, targets = get_batch(source, i)
-                if isinstance(m, fused.FusedLSTM):
+                if isinstance(m, (fused.FusedLSTM, fused.FusedRNN)):
                     # per-token losses, no log-probability tensor; sum / bsz = len(data) * the chunk's mean loss
                     loss, hidden = m.nll(data, targets, hidden)
                     total += loss.double().sum().item() / bsz
@@ -116,7 +118,7 @@ def main(argv=None):
         if args.engine == 'tcgen05':
             use_tensor_cores(qmodel)
         elif args.engine == 'fused':
-            runner = fused.FusedLSTM(qmodel)
+            runner = fused.FusedLSTM(qmodel) if args.model == 'LSTM' else fused.FusedRNN(qmodel)
         loss = evaluate(runner, test_data)
         inputs = (get_batch(test_data, 0)[0], model.init_hidden(bsz))
         tmacs, param_bits = profile_model.get_model_ops(qmodel, inputs=inputs)

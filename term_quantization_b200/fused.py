@@ -493,7 +493,99 @@ def _param_key(t):
     return None if t is None else (t.data_ptr(), t._version, t.device)
 
 
-class FusedLSTM(nn.Module):
+class _FusedLanguageModel(nn.Module):
+    """What FusedLSTM and FusedRNN share: the TRLinearLayer decoder on term codes (its input codes, linear_codes for
+    forward, linear_codes_nll for nll, the padded bias and scale), the staleness checks, and forward / nll around the
+    cell-specific _recurrence(input, hidden) -> (y [T, B, H] of the last layer, hidden state out).  A subclass
+    switches the decoder to its tensor-core path (use_tensor_cores) before it calls _init_decoder and sets _key."""
+
+    def _init_decoder(self):
+        dec = self.model.decoder
+        self.dec_scale = (torch.tensor(float(dec.input_quant.sf), dtype=torch.float32)
+                          * torch.tensor(dec._tc_wsf32, dtype=torch.float32)).item()
+        # the decoder bias padded to the packed weight's rows once, so that linear_codes allocates nothing next to its output
+        _, out_pad, _ = dec._tc_weight.shape
+        self.dec_bias = None
+        if dec.linear.bias is not None:
+            self.dec_bias = torch.zeros(out_pad, dtype=torch.float32, device=dec.linear.bias.device)
+            self.dec_bias[:dec.linear.out_features] = dec.linear.bias.detach()
+
+    def _decoder_snapshot(self):
+        dec = self.model.decoder
+        return [_param_key(dec.linear.weight), _param_key(dec.linear.bias), float(dec.w_sf), dec._tc_weight,
+                _quant_key(dec)]
+
+    def check_fresh(self):
+        """Weights, packed operands and scale factors are snapshots: refuse stale ones (load_state_dict, in-place
+        updates, .to(device), re-calibration after fusing) and a model switched back to training or tracking."""
+        if self.training or self.model.training:
+            raise RuntimeError(f"{type(self).__name__} runs inference only: call .eval() first")
+        if any(q.tracking for q in self._quantisers()):
+            raise RuntimeError("the wrapped model is tracking (calibrating) again: finish the calibration and build the "
+                               "fused executor again")
+        key = self._snapshot()
+        if any(a is not b if isinstance(a, torch.Tensor) or isinstance(b, torch.Tensor) else a != b
+               for a, b in zip(key, self._key)):
+            raise RuntimeError("the wrapped model changed after fusing (weights, device or scale factors): "
+                               "build the fused executor again")
+
+    def _decoder_codes(self, input, hidden):
+        """The chain forward and nll share: the recurrence, then the decoder's input quantiser.  Returns (the decoder's
+        fp16 input codes [T*B, Kp] at the packed weight's width, so that the decoder copies nothing; the hidden state
+        out; y).  The recurrence's temporaries are gone before the decoder runs."""
+        if not torch.cuda.is_current_stream_capturing():
+            self.check_fresh()
+        dec = self.model.decoder
+        y, hidden = self._recurrence(input, hidden)
+        T, B, H = y.shape
+        q = dec.input_quant
+        codes = torch.zeros((T * B, dec._tc_weight.shape[2]), dtype=torch.float16, device=y.device)
+        codes[:, :H] = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
+                                        encoding=q.encoding).view(T * B, H)
+        return codes, hidden, y
+
+    def _decoded(self, input, hidden):
+        """_decoder_codes, then the decoder's linear(q(y)) on term codes.  Returns (decoded [T*B, ntoken] fp32, a column
+        slice of the decoder's padded output; the hidden state out; y; the decoder's fp16 input codes [T*B, H])."""
+        codes, hidden, y = self._decoder_codes(input, hidden)
+        dec = self.model.decoder
+        decoded = conv_codes.linear_codes(codes, dec._tc_weight, self.dec_scale, bias=self.dec_bias,
+                                          out_features=dec.linear.out_features, plan=dec._tc_plan)
+        return decoded, hidden, y, codes[:, :y.shape[2]]
+
+    @torch.no_grad()
+    def forward(self, input, hidden, capture=None):
+        """input: int64 [T, B] tokens; hidden: the hidden state RNNModel.forward takes.  capture: optional dict that
+        receives 'y' (the last layer's fp32 output [T, B, H]), 'codes' (the decoder's fp16 input codes [T*B, H]) and
+        'decoded' (the decoder's fp32 output before log_softmax)."""
+        decoded, hidden, y, codes = self._decoded(input, hidden)
+        if capture is not None:
+            capture["y"], capture["codes"], capture["decoded"] = y, codes, decoded
+        return F.log_softmax(decoded, dim=1), hidden
+
+    @torch.no_grad()
+    def nll(self, input, targets, hidden):
+        """Per-token negative log-likelihood of `targets` (int64 [T*B], the next tokens in forward's row order) under
+        the model: the chain of forward up to the decoder's input codes, then the decoder with the loss epilogue
+        (conv_codes.linear_codes_nll), which reduces each row of logits inside the decoder and never writes them.
+        Equals nll_loss(forward(input, hidden)[0], targets, reduction='none') within 4e-6 * max(|ref|, 1) of fp64 over
+        the decoder output, without allocating any [T*B, ntoken] tensor.  Returns (loss fp32 [T*B], the hidden state
+        out); a target outside [0, ntoken) gives NaN for its token."""
+        T, B = input.shape
+        name = type(self).__name__
+        if targets.dtype != torch.int64 or targets.dim() != 1 or targets.shape[0] != T * B:
+            raise ValueError(f"{name}.nll expects int64 targets [T*B] = [{T * B}], got {targets.dtype} "
+                             f"{tuple(targets.shape)}")
+        if targets.device != input.device:
+            raise RuntimeError(f"{name}.nll: targets on {targets.device}, tokens on {input.device}")
+        codes, hidden, _ = self._decoder_codes(input, hidden)
+        dec = self.model.decoder
+        loss = conv_codes.linear_codes_nll(codes, dec._tc_weight, self.dec_scale, targets, bias=self.dec_bias,
+                                           out_features=dec.linear.out_features, plan=dec._tc_plan)
+        return loss, hidden
+
+
+class FusedLSTM(_FusedLanguageModel):
     """Fused execution of a calibrated, TQ-converted RNNModel('LSTM', ...) (BASELINE.json configs[4]): an nn.Embedding
     encoder, a TRLSTMLayer rnn and a TRLinearLayer decoder.  forward(input, hidden) -> (log_probs [T*B, ntoken], (hn, cn))
     follows RNNModel.forward, so a bptt loop carries the hidden state across chunks unchanged.
@@ -516,7 +608,7 @@ class FusedLSTM(nn.Module):
         if getattr(model, "rnn_type", None) != "LSTM" or not isinstance(rnn, tr_layer.TRLSTMLayer) \
                 or not isinstance(getattr(model, "encoder", None), nn.Embedding):
             raise NotImplementedError("FusedLSTM expects a TQ-converted RNNModel('LSTM', ...): nn.Embedding encoder, "
-                                      "TRLSTMLayer rnn (GRU and vanilla RNN models are not supported)")
+                                      "TRLSTMLayer rnn (GRU and vanilla RNN models run on FusedRNN)")
         m = rnn.lstm
         if type(m) is not nn.LSTM or m.bidirectional or m.batch_first or m.proj_size != 0:
             raise NotImplementedError("FusedLSTM: unidirectional, time-major nn.LSTM without projections only "
@@ -544,37 +636,17 @@ class FusedLSTM(nn.Module):
                 if m.bias:
                     bias = (getattr(m, f"bias_ih_l{l}") + getattr(m, f"bias_hh_l{l}")).contiguous()
                 self.layers.append((None if l == 0 else getattr(m, f"weight_ih_l{l}"), getattr(m, f"weight_hh_l{l}"), bias))
-        self.dec_scale = (torch.tensor(float(dec.input_quant.sf), dtype=torch.float32)
-                          * torch.tensor(dec._tc_wsf32, dtype=torch.float32)).item()
-        # the decoder bias padded to the packed weight's rows once, so that linear_codes allocates nothing next to its output
-        _, out_pad, _ = dec._tc_weight.shape
-        self.dec_bias = None
-        if dec.linear.bias is not None:
-            self.dec_bias = torch.zeros(out_pad, dtype=torch.float32, device=dec.linear.bias.device)
-            self.dec_bias[:dec.linear.out_features] = dec.linear.bias.detach()
+        self._init_decoder()
         self._key = self._snapshot()
         self.train(False)
 
-    def _snapshot(self):
-        rnn, dec = self.model.rnn, self.model.decoder
-        return ([_param_key(p) for p in rnn.lstm.parameters()], _param_key(dec.linear.weight), _param_key(dec.linear.bias),
-                _param_key(self.model.encoder.weight), float(rnn.w_sf_ih), float(dec.w_sf), rnn._tc_weight, dec._tc_weight,
-                _quant_key(rnn), _quant_key(dec))
+    def _quantisers(self):
+        return self.model.rnn.input_quant, self.model.decoder.input_quant
 
-    def check_fresh(self):
-        """Weights, packed operands and scale factors are snapshots: refuse stale ones (load_state_dict, in-place
-        updates, .to(device), re-calibration after fusing) and a model switched back to training or tracking."""
-        rnn, dec = self.model.rnn, self.model.decoder
-        if self.training or self.model.training:
-            raise RuntimeError("FusedLSTM runs inference only: call .eval() first")
-        if rnn.input_quant.tracking or dec.input_quant.tracking:
-            raise RuntimeError("the wrapped model is tracking (calibrating) again: finish the calibration and build the "
-                               "fused executor again")
-        key = self._snapshot()
-        if any(a is not b if isinstance(a, torch.Tensor) or isinstance(b, torch.Tensor) else a != b
-               for a, b in zip(key, self._key)):
-            raise RuntimeError("the wrapped model changed after fusing (weights, device or scale factors): "
-                               "build the fused executor again")
+    def _snapshot(self):
+        rnn = self.model.rnn
+        return [[_param_key(p) for p in rnn.lstm.parameters()], _param_key(self.model.encoder.weight), float(rnn.w_sf_ih),
+                rnn._tc_weight, _quant_key(rnn)] + self._decoder_snapshot()
 
     def _recurrence(self, input, hidden):
         """Embedding, the shared quantiser on h0 / c0, then every layer's input projection and recurrence kernel.
@@ -596,56 +668,91 @@ class FusedLSTM(nn.Module):
             cn.append(c)
         return y, (torch.stack(hn), torch.stack(cn))
 
-    def _decoder_codes(self, input, hidden):
-        """The chain forward and nll share: the recurrence, then the decoder's input quantiser.  Returns (the decoder's
-        fp16 input codes [T*B, Kp] at the packed weight's width, so that the decoder copies nothing; (hn, cn); y).  The
-        recurrence's temporaries are gone before the decoder runs."""
-        if not torch.cuda.is_current_stream_capturing():
-            self.check_fresh()
-        dec = self.model.decoder
-        y, hidden = self._recurrence(input, hidden)
-        T, B, H = y.shape
-        q = dec.input_quant
-        codes = torch.zeros((T * B, dec._tc_weight.shape[2]), dtype=torch.float16, device=y.device)
-        codes[:, :H] = tr_cuda.tr_codes(y.view(1, -1, 1, 1), q.sf, q.data_bits, 1, q.data_terms, dtype=torch.float16,
-                                        encoding=q.encoding).view(T * B, H)
-        return codes, hidden, y
 
-    def _decoded(self, input, hidden):
-        """_decoder_codes, then the decoder's linear(q(y)) on term codes.  Returns (decoded [T*B, ntoken] fp32, a column
-        slice of the decoder's padded output; (hn, cn); y; the decoder's fp16 input codes [T*B, H])."""
-        codes, hidden, y = self._decoder_codes(input, hidden)
-        dec = self.model.decoder
-        decoded = conv_codes.linear_codes(codes, dec._tc_weight, self.dec_scale, bias=self.dec_bias,
-                                          out_features=dec.linear.out_features, plan=dec._tc_plan)
-        return decoded, hidden, y, codes[:, :y.shape[2]]
+class FusedRNN(_FusedLanguageModel):
+    """Fused execution of a calibrated, TQ-converted RNNModel('GRU' | 'RNN_TANH' | 'RNN_RELU', ...): an nn.Embedding
+    encoder, an nn.GRU / nn.RNN rnn and a TRLinearLayer decoder.  forward(input, hidden) -> (log_probs [T*B, ntoken], hn)
+    follows RNNModel.forward with its single hidden tensor [layers, B, H].
 
-    @torch.no_grad()
-    def forward(self, input, hidden, capture=None):
-        """input: int64 [T, B] tokens; hidden: (h0, c0) fp32 [layers, B, H].  capture: optional dict that receives 'y'
-        (the last layer's fp32 output [T, B, H]), 'codes' (the decoder's fp16 input codes [T*B, H]) and 'decoded' (the
-        decoder's fp32 output before log_softmax)."""
-        decoded, hidden, y, codes = self._decoded(input, hidden)
-        if capture is not None:
-            capture["y"], capture["codes"], capture["decoded"] = y, codes, decoded
-        return F.log_softmax(decoded, dim=1), hidden
+    As in the reference, only the decoder is a TR layer: the recurrent weights are not term-revealed and h0 is not
+    quantised.  Chain: embedding gather -> per layer an fp32 GEMM x . W_ih^T (+ b_ih for the GRU; torch.mm / addmm, true
+    fp32 unless torch.backends.cuda.matmul.allow_tf32 is set) and the recurrence kernel (conv_codes.gru_recurrence /
+    rnn_recurrence: all T steps in one persistent launch) -> the decoder's linear(q(y)) on term codes -> log_softmax, or
+    the decoder's loss epilogue for nll, exactly as FusedLSTM.  The recurrence is fp32 with a fixed summation order:
+    bit-identical from run to run and under CUDA-graph replay, within 1e-5 of an fp64 recurrence, not bit-comparable
+    with cuDNN."""
 
-    @torch.no_grad()
-    def nll(self, input, targets, hidden):
-        """Per-token negative log-likelihood of `targets` (int64 [T*B], the next tokens in forward's row order) under
-        the model: the chain of forward up to the decoder's input codes, then the decoder with the loss epilogue
-        (conv_codes.linear_codes_nll), which reduces each row of logits inside the decoder and never writes them.
-        Equals nll_loss(forward(input, hidden)[0], targets, reduction='none') within 4e-6 * max(|ref|, 1) of fp64 over
-        the decoder output, without allocating any [T*B, ntoken] tensor.  Returns (loss fp32 [T*B], (hn, cn)); a target
-        outside [0, ntoken) gives NaN for its token."""
+    def __init__(self, model):
+        super().__init__()
+        kind = getattr(model, "rnn_type", None)
+        rnn, dec = getattr(model, "rnn", None), getattr(model, "decoder", None)
+        if kind == "LSTM":
+            raise NotImplementedError("FusedRNN runs GRU and vanilla RNN models: use FusedLSTM for RNNModel('LSTM', ...)")
+        cls = {"GRU": nn.GRU, "RNN_TANH": nn.RNN, "RNN_RELU": nn.RNN}.get(kind)
+        if cls is None or type(rnn) is not cls or not isinstance(getattr(model, "encoder", None), nn.Embedding):
+            raise NotImplementedError("FusedRNN expects a TQ-converted RNNModel('GRU' | 'RNN_TANH' | 'RNN_RELU', ...): "
+                                      "nn.Embedding encoder, nn.GRU / nn.RNN rnn")
+        self.nonlinearity = None if kind == "GRU" else kind.split("_")[1].lower()
+        if cls is nn.RNN and rnn.nonlinearity != self.nonlinearity:
+            raise NotImplementedError(f"FusedRNN: an {kind} model with a {rnn.nonlinearity} nn.RNN")
+        if rnn.bidirectional or rnn.batch_first:
+            raise NotImplementedError("FusedRNN: unidirectional, time-major recurrences only "
+                                      f"(bidirectional={rnn.bidirectional}, batch_first={rnn.batch_first})")
+        if not isinstance(dec, tr_layer.TRLinearLayer) or dec.linear.in_features != rnn.hidden_size:
+            raise NotImplementedError(f"FusedRNN expects a TRLinearLayer decoder over the {kind}'s hidden state")
+        for name, p in rnn.named_parameters():
+            if p.dtype != torch.float32 or not p.is_cuda:
+                raise NotImplementedError(f"FusedRNN: fp32 CUDA parameters only ({name} is {p.dtype} on {p.device})")
+        hmax = conv_codes.recurrence_max_hidden(kind, rnn.weight_hh_l0.device)
+        if rnn.hidden_size > hmax:
+            raise NotImplementedError(f"FusedRNN: hidden size {rnn.hidden_size} exceeds what the {kind} recurrence kernel "
+                                      f"keeps in shared memory on this device (H <= {hmax})")
+        if dec.input_quant.tracking:
+            raise RuntimeError("calibrate the model (set_tr_tracking(model, False)) before fusing")
+        if model.training:
+            raise RuntimeError("FusedRNN runs inference only: call model.eval() first")
+        dec.use_tensor_cores()                       # raises before any launch when the decoder's codes do not fit
+        self.model = model
+        self.cell = kind
+        # per layer: (w_ih, the bias folded into the input GEMM or None, w_hh, the kernel's bias or None).  The GRU's
+        # b_hn multiplies with the reset gate, so b_ih goes into the GEMM and b_hh to the kernel; an RNN adds both.
+        self.layers = []
+        with torch.no_grad():
+            for l in range(rnn.num_layers):
+                w_ih, w_hh = getattr(rnn, f"weight_ih_l{l}"), getattr(rnn, f"weight_hh_l{l}")
+                b_gemm = b_rec = None
+                if rnn.bias:
+                    b_ih, b_hh = getattr(rnn, f"bias_ih_l{l}"), getattr(rnn, f"bias_hh_l{l}")
+                    if kind == "GRU":
+                        b_gemm, b_rec = b_ih, b_hh
+                    else:
+                        b_rec = (b_ih + b_hh).contiguous()
+                self.layers.append((w_ih, b_gemm, w_hh, b_rec))
+        self._init_decoder()
+        self._key = self._snapshot()
+        self.train(False)
+
+    def _quantisers(self):
+        return (self.model.decoder.input_quant,)
+
+    def _snapshot(self):
+        return [[_param_key(p) for p in self.model.rnn.parameters()],
+                _param_key(self.model.encoder.weight)] + self._decoder_snapshot()
+
+    def _recurrence(self, input, hidden):
+        """Embedding, then every layer's input GEMM and recurrence kernel.  Returns (y [T, B, H] of the last layer,
+        hn [layers, B, H])."""
         T, B = input.shape
-        if targets.dtype != torch.int64 or targets.dim() != 1 or targets.shape[0] != T * B:
-            raise ValueError(f"FusedLSTM.nll expects int64 targets [T*B] = [{T * B}], got {targets.dtype} "
-                             f"{tuple(targets.shape)}")
-        if targets.device != input.device:
-            raise RuntimeError(f"FusedLSTM.nll: targets on {targets.device}, tokens on {input.device}")
-        codes, hidden, _ = self._decoder_codes(input, hidden)
-        dec = self.model.decoder
-        loss = conv_codes.linear_codes_nll(codes, dec._tc_weight, self.dec_scale, targets, bias=self.dec_bias,
-                                           out_features=dec.linear.out_features, plan=dec._tc_plan)
-        return loss, hidden
+        y = self.model.encoder(input)
+        hn = []
+        for l, (w_ih, b_gemm, w_hh, b_rec) in enumerate(self.layers):
+            x = y.view(T * B, -1)
+            gin = (torch.mm(x, w_ih.t()) if b_gemm is None else torch.addmm(b_gemm, x, w_ih.t())).view(T, B, -1)
+            del x, y                                                    # the layer input, before the kernel's output
+            if self.nonlinearity is None:
+                y, h = conv_codes.gru_recurrence(gin, b_rec, w_hh, hidden[l].contiguous())
+            else:
+                y, h = conv_codes.rnn_recurrence(gin, b_rec, w_hh, hidden[l].contiguous(), self.nonlinearity)
+            del gin                                                     # before the next layer's GEMM is allocated
+            hn.append(h)
+        return y, torch.stack(hn)

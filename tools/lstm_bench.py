@@ -14,7 +14,14 @@ Writes DIR/lstm_bench.json.  Usage: python tools/lstm_bench.py --out DIR [--roun
   decoder output + log_softmax_nll  the chain up to the padded decoder output, then one tq_log_softmax_nll pass over it
   nll                               FusedLSTM.nll: the decoder's loss epilogue, no [T*B, V] tensor written at all
 with the peak memory of each, plus the decoder with its loss epilogue against the decoder followed by
-tq_log_softmax_nll (CUDA events over many calls).  Writes DIR/lstm_nll_epilogue.json."""
+tq_log_softmax_nll (CUDA events over many calls).  Writes DIR/lstm_nll_epilogue.json.
+
+--model GRU RNN_TANH RNN_RELU times the same workload with each of those cells (only the decoder is a TR layer, as in
+the reference), one perplexity step as alternating CUDA-graph replays of
+  tcgen05  cuDNN recurrence + the decoder on term codes + log_softmax + nll_loss(reduction='none')
+  nll      FusedRNN.nll: the recurrence kernel per layer, the decoder's loss epilogue
+with the peak memory of each, and every layer's recurrence launch on its own (CUDA events) with its FFMA rate against
+the derived fp32 rate.  Writes DIR/rnn_bench.json."""
 import argparse
 import copy
 import gc
@@ -211,12 +218,75 @@ def nll_bench(f, tokens, hidden, targets, rounds, replays, launches=50, samples=
     }
 
 
+def derived_fp32_rate(info, props):
+    """SMs x 128 FP32 FMA/clk x the max SM clock nvidia-smi reports (derived, not a measured peak); None without it."""
+    return props.multi_processor_count * 128 * info["max_sm_clock_mhz"] * 1e6 if "max_sm_clock_mhz" in info else None
+
+
+def rnn_bench(cell, dev, rounds, replays, derived, launches=20, samples=10):
+    """One cell's perplexity step on both paths, and its recurrence launches alone."""
+    torch.manual_seed(0)
+    gen = torch.Generator(device=dev).manual_seed(0)
+    base = RNNModel(cell, evaluate_lstm.NTOKENS, 650, 650, 2, 0.5, True).to(dev).eval()
+    q = evaluate_lstm.convert_model(base, evaluate_lstm.static_lstm_layer_settings(base, 8, 8, 12), 8, 8)
+    tokens = torch.randint(evaluate_lstm.NTOKENS, (T, B), device=dev, generator=gen)
+    targets = torch.randint(evaluate_lstm.NTOKENS, (T * B,), device=dev, generator=gen)
+    hidden = base.init_hidden(B)
+    with torch.no_grad():
+        q(tokens, hidden)
+        tr_layer.set_tr_tracking(q, False)
+        q_tc = copy.deepcopy(q)
+        tr_layer.use_tensor_cores(q_tc)
+        f = fused.FusedRNN(copy.deepcopy(q))
+        paths = {"tcgen05": lambda: F.nll_loss(q_tc(tokens, hidden)[0], targets, reduction="none"),
+                 "nll": lambda: f.nll(tokens, targets, hidden)[0]}
+        graphs, outs = {}, {}
+        for name, fn in paths.items():
+            graphs[name], outs[name] = capture(fn)
+        samples_ms = {k: [] for k in graphs}
+        for _ in range(rounds):
+            for name, g in graphs.items():
+                samples_ms[name].append(time_replays(g, replays))
+        ref = outs["tcgen05"].double()
+        rel = float(((outs["nll"].double() - ref).abs() / ref.abs().clamp(min=1.0)).max())
+        peaks = {k: peak_rise(fn) for k, fn in paths.items()}
+
+        # every layer's recurrence alone, on the input projection the executor computes for it
+        G = conv_codes.RECURRENCE_GATES[cell]
+        fma = T * B * G * H * H
+        y = f.model.encoder(tokens)
+        recurrence = []
+        for l, (w_ih, b_gemm, w_hh, b_rec) in enumerate(f.layers):
+            x = y.view(T * B, -1)
+            gin = (torch.mm(x, w_ih.t()) if b_gemm is None else torch.addmm(b_gemm, x, w_ih.t())).view(T, B, -1)
+            h0 = hidden[l].contiguous()
+            if cell == "GRU":
+                run = lambda gin=gin, b=b_rec, w=w_hh, h0=h0: conv_codes.gru_recurrence(gin, b, w, h0)  # noqa: E731
+            else:
+                run = lambda gin=gin, b=b_rec, w=w_hh, h0=h0: conv_codes.rnn_recurrence(  # noqa: E731
+                    gin, b, w, h0, f.nonlinearity)
+            t = _events(run, launches, samples)
+            rate = fma / (t["ms_median"] * 1e-3)
+            recurrence.append({"layer": l, "fma": fma, **t, "fma_per_s": rate, "fp32_tflops": 2 * rate / 1e12,
+                               "share_of_derived_fp32_rate": rate / derived if derived else None})
+            y = run()[0]
+    steps = {k: {"ms_best": min(v), "ms_median": statistics.median(v), "ms_spread": max(v) - min(v),
+                 "tokens_per_s_median": T * B / statistics.median(v) * 1e3, "peak_memory_rise_bytes": peaks[k]}
+             for k, v in samples_ms.items()}
+    return {"paths": steps, "nll_vs_tcgen05_speedup_median": steps["tcgen05"]["ms_median"] / steps["nll"]["ms_median"],
+            "loss_max_rel_diff_nll_vs_tcgen05": rel, "max_hidden": conv_codes.recurrence_max_hidden(cell, dev),
+            "recurrence_kernel": {"how": f"eager, CUDA events around {launches} back-to-back launches, {samples} samples",
+                                  "layers": recurrence}}
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--out", required=True, help="output directory (lstm_bench.json)")
     ap.add_argument("--rounds", type=int, default=15, help="alternating rounds; each times every path once")
     ap.add_argument("--replays", type=int, default=20, help="graph replays per timed sample")
     ap.add_argument("--nll", action="store_true", help="time the three perplexity paths (lstm_nll_epilogue.json)")
+    ap.add_argument("--model", nargs="+", choices=["GRU", "RNN_TANH", "RNN_RELU"],
+                    help="time these cells' perplexity step instead (rnn_bench.json)")
     args = ap.parse_args(argv)
     if not torch.cuda.is_available():
         raise SystemExit("lstm_bench needs a CUDA device: nothing is timed on the CPU")
@@ -226,6 +296,22 @@ def main(argv=None):
     dev = torch.device("cuda")
     info = gpu_info()
     props = torch.cuda.get_device_properties(dev)
+    if args.model:
+        derived = derived_fp32_rate(info, props)
+        res = {"workload": "Wikitext-2-shaped RNNModel 650/650 tied, 2 layers, vocab 33,278, seq 35 x batch 80, only the "
+                           "decoder TQ (wb 8 / g 8 / alpha 12 / db 8), seed 0: one perplexity step",
+               "gpu": info, "sms": props.multi_processor_count,
+               "timed_as": f"CUDA-graph replays of the whole step, {args.replays} per sample, {args.rounds} rounds "
+                           "alternating the two paths; TF32 off.  Peak memory: eager call, rise of max_memory_allocated "
+                           "above the allocation before it",
+               "derived_fp32_fma_rate": {"fma_per_s": derived, "how": "SMs x 128 FP32 FMA/clk x max SM clock (derived, "
+                                                                      "not a measured peak)"},
+               "cells": {cell: rnn_bench(cell, dev, args.rounds, args.replays, derived) for cell in args.model}}
+        path = os.path.join(args.out, "rnn_bench.json")
+        with open(path, "w") as fp:
+            json.dump(res, fp, indent=1)
+        print(json.dumps(res, indent=1))
+        return
 
     torch.manual_seed(0)
     gen = torch.Generator(device=dev).manual_seed(0)
@@ -270,9 +356,7 @@ def main(argv=None):
     per_phase = phases(f, tokens, hidden, reps=20)
     rec = [p for p in per_phase if "recurrence" in p["phase"]]
     fma = T * B * 4 * H * H
-    derived = None
-    if "max_sm_clock_mhz" in info:
-        derived = props.multi_processor_count * 128 * info["max_sm_clock_mhz"] * 1e6
+    derived = derived_fp32_rate(info, props)
     recurrence = []
     for p in rec:
         rate = fma / (p["ms_median"] * 1e-3)
