@@ -1486,6 +1486,14 @@ static int launch_conv_mode(const CUtensorMap &tmA, const CUtensorMap &tmB, cons
     }
 }
 
+// A halo tiling is taken only when its buffers leave room for a ring of two stages beside the epilogue staging: seven
+// halo rows of 128 pixels (a 7x7 filter on a map about 128 pixels wide) or a 3-row halo beside nine resident weight tiles
+// and fp32 + code staging do not, and the plan the halo would replace stays
+static bool smem_fits(ConvGeom h, int block_n)
+{
+    return plan_smem(h, block_n) == TQ_OK;
+}
+
 // which kernel instance runs a planned conv
 enum ConvVariant { CV_NONE = 0, CV_64_M0, CV_64_M1, CV_64_M2, CV_64_M3, CV_64_M3_PAIR, CV_128_M0, CV_128_M4, CV_128_M4_PAIR, CV_256_M0, CV_I8_64, CV_I8_128 };
 
@@ -1656,9 +1664,8 @@ static int plan_conv(const ConvArgs &a, ConvPlan &pl)
             // 0.740 -> 0.621 ms)
             static const int slack = getenv("TQ_CONV_HALO_SLACK") ? atoi(getenv("TQ_CONV_HALO_SLACK")) : 16;
             if (pick_box_halo(h) && (long)h.m_tiles * 100 <= (long)g.m_tiles * (100 + slack)) {
-                g = h;
-                g.halo = 1;
-                g.halo_baseoff = halo_baseoff ? 1 : 0;
+                h.halo = 1;
+                h.halo_baseoff = halo_baseoff ? 1 : 0;
                 // CTA pairs (opt-in, TQ_CONV_PAIR3=1): N = 64 MMAs are bound by shared-memory operand reads (A 4 KB + B 2 KB per
                 // 32-cycle MMA); with half of every weight tile per CTA it is 4 + 1 KB.  Measured: the 56x56 64 -> 64 layer with
                 // an fp32-only epilogue 0.0756 -> 0.0569 ms (1040 TFLOP/s), but NO change inside ResNet-18 / VGG-16, where
@@ -1666,7 +1673,8 @@ static int plan_conv(const ConvArgs &a, ConvPlan &pl)
                 // them -- so single CTAs stay the default.
                 static const int pair3_env = getenv("TQ_CONV_PAIR3") ? atoi(getenv("TQ_CONV_PAIR3")) : 0;
                 static const int pair_env3 = getenv("TQ_CONV_PAIR") ? atoi(getenv("TQ_CONV_PAIR")) : 1;
-                if (pair3_env && pair_env3 && !g.halo_baseoff && Cout % 16 == 0 && ((g.m_tiles + 1) / 2) * g.n_tiles >= num_sms() / 2) g.pair = 1;
+                if (pair3_env && pair_env3 && !h.halo_baseoff && Cout % 16 == 0 && ((h.m_tiles + 1) / 2) * h.n_tiles >= num_sms() / 2) h.pair = 1;
+                if (smem_fits(h, block_n)) g = h;
             }
         }
     }
@@ -1683,26 +1691,28 @@ static int plan_conv(const ConvArgs &a, ConvPlan &pl)
     if (kind == 0 && !no_halo4 && !no_packed && g.prog_steps == 0 && !g.halo && block_n == 128 && stride == 1 && R == 3 && S == 3 &&
         pad == 1 && N >= 2 && 2 * (W + 1) * (H + 1) <= 128) {
         const int per = (W + 1) * (H + 1);
-        g.wbox = W; g.hbox = H; g.nbox = 128 / per < N ? 128 / per : N;
-        g.hw = W + 1; g.img_h1 = H + 1;
-        g.tiles_w = g.tiles_h = 1; g.tiles_n = (N + g.nbox - 1) / g.nbox; g.m_tiles = g.tiles_n;
-        g.a_tx_bytes = g.nbox * per * GM_ROW_BYTES;
-        g.step_w = g.wbox; g.step_h = g.hbox;
-        g.halo = 1;
+        ConvGeom h = g;
+        h.wbox = W; h.hbox = H; h.nbox = 128 / per < N ? 128 / per : N;
+        h.hw = W + 1; h.img_h1 = H + 1;
+        h.tiles_w = h.tiles_h = 1; h.tiles_n = (N + h.nbox - 1) / h.nbox; h.m_tiles = h.tiles_n;
+        h.a_tx_bytes = h.nbox * per * GM_ROW_BYTES;
+        h.step_w = h.wbox; h.step_h = h.hbox;
+        h.halo = 1;
         static const int pair_env = getenv("TQ_CONV_PAIR") ? atoi(getenv("TQ_CONV_PAIR")) : 1;
-        if (pair_env && ((g.m_tiles + 1) / 2) * g.n_tiles >= num_sms() / 2) g.pair = 1;
+        if (pair_env && ((h.m_tiles + 1) / 2) * h.n_tiles >= num_sms() / 2) h.pair = 1;
+        if (smem_fits(h, block_n)) g = h;
     }
     if (kind == 0 && !no_halo4 && g.prog_steps == 0 && !g.halo && block_n == 128 && stride == 1 && R * S > 1) {
         ConvGeom h = g;
         static const int slack4 = getenv("TQ_CONV_HALO_SLACK") ? atoi(getenv("TQ_CONV_HALO_SLACK")) : 16;
         if (pick_box_halo(h) && (long)h.m_tiles * 100 <= (long)g.m_tiles * (100 + slack4)) {
             h.step_w = h.wbox; h.step_h = h.hbox;
-            g = h;
-            g.halo = 1;
+            h.halo = 1;
             // CTA pairs (cta_group::2) when there are enough tiles to keep every pair busy: per CTA half the weight
             // traffic from L2 and 6 KB instead of 8 KB of operand reads per MMA.  TQ_CONV_PAIR=0 keeps single CTAs.
             static const int pair_env = getenv("TQ_CONV_PAIR") ? atoi(getenv("TQ_CONV_PAIR")) : 1;
-            if (pair_env && ((g.m_tiles + 1) / 2) * g.n_tiles >= num_sms() / 2) g.pair = 1;
+            if (pair_env && ((h.m_tiles + 1) / 2) * h.n_tiles >= num_sms() / 2) h.pair = 1;
+            if (smem_fits(h, block_n)) g = h;
         }
     }
     const CUtensorMapDataType op_dt = kind == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;

@@ -74,6 +74,12 @@ def test_conv_codes_exact_accumulators(case):
         assert torch.equal(out2, want2), engine
 
 
+def _fma(t, a, b):
+    """fmaf(t, a[c], b[c]) over the channel axis, correctly rounded once (tq_oracle.fma_channels), on t's device."""
+    from oracle import tq_oracle as O
+    return torch.from_numpy(O.fma_channels(t.cpu().numpy(), a.cpu().numpy(), b.cpu().numpy())).to(t.device)
+
+
 def _exact(act, wgt, k, stride, pad):
     Cout, C = wgt.shape[1], wgt.shape[2]
     w_oihw = wgt.view(k, k, Cout, C).permute(2, 3, 0, 1).double()
@@ -144,7 +150,7 @@ def test_k_chunk_accumulators_exact_beyond_2_24(case, amp, groups):
         a = torch.rand(Cout, device="cuda", generator=g) + 0.5
         b = torch.randn(Cout, device="cuda", generator=g)
         res = torch.randn(want.shape, device="cuda", generator=g)
-        t = torch.relu(((want.float() * scale).double() * a.double() + b.double()).float() + res)
+        t = torch.relu(_fma(want.float() * scale, a, b) + res)
         nq = (max(float(t.max()), 1e-3) / 512, 9, 3)
         o2, codes = conv_codes.conv2d_codes_fused(act.half().contiguous(), wh, (k, k), stride, pad, scale, bn=(a, b), residual=res,
                                                   relu=True, next_quant=nq, plan=plan)
@@ -174,7 +180,7 @@ def test_i8_plane_engine_plane_counts():
             scale = np.float32(1.7e-6)
             a = torch.rand(Cout, device="cuda", generator=g) + 0.5
             b = torch.randn(Cout, device="cuda", generator=g)
-            t = torch.relu((want.float() * scale).double() * a.double() + b.double()).float()
+            t = torch.relu(_fma(want.float() * scale, a, b))
             nq = (max(float(t.max()), 1e-3) / 512, 9, 3)
             out, codes = conv_codes.conv2d_codes_fused(act.half().contiguous(), wh, (k, k), stride, pad, scale, bn=(a, b),
                                                        relu=True, next_quant=nq, plan=plan)
@@ -228,7 +234,7 @@ def test_conv_fused_epilogue(case):
     b = torch.randn(Cout, device="cuda", generator=g)
     res = torch.randn(acc.shape, device="cuda", generator=g)
     t0 = acc * scale
-    t1 = (t0.double() * a.double() + b.double()).float()          # fma(t, a, b), one rounding
+    t1 = _fma(t0, a, b)                                           # fmaf(t, a, b), one rounding
     t2 = t1 + res
     t3 = torch.relu(t2)
     nq = (float(t3.max()) / 512, 9, 3)
@@ -261,7 +267,7 @@ def test_bn_relu_maxpool_encode():
         x = torch.randn(N, H, W, C, device="cuda", generator=g) * 2
         a = torch.randn(C, device="cuda", generator=g)            # negative slopes included
         b = torch.randn(C, device="cuda", generator=g)
-        y = (x.double() * a.double() + b.double()).float()        # fma, one rounding
+        y = _fma(x, a, b)                                         # fmaf, one rounding
         want = F.max_pool2d(torch.relu(y).permute(0, 3, 1, 2), 3, 2, 1).permute(0, 2, 3, 1).contiguous()
         nq = (float(want.max()) / 512, 9, 3)
         out, codes = conv_codes.bn_relu_maxpool_encode(x, (a, b), relu=True, next_quant=nq)
