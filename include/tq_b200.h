@@ -389,10 +389,13 @@ int tq_u8_normalize_bf16(const void *x_u8, void *y_bf16, int64_t npix, const flo
  *   bias fp32 [4H] (b_ih + b_hh) or NULL;  w_hh fp32 [4H][H] row-major (nn.LSTM's weight_hh_l*);  h0, c0 fp32 [B][H]
  *   y    fp32 [T][B][H] = h_t;  hn, cn fp32 [B][H] = h_T, c_T
  * fp32 FFMA with one fixed summation order per dot product (bit-identical from run to run), sig(x) = 1 / (1 + expf(-x)),
- * accurate expf / tanhf.  Each CTA keeps the 4 gate rows of ceil(H / SMs) hidden units in shared memory; H is refused
- * (TQ_ERR_UNSUPPORTED) when those rows and one hidden row exceed the device's opt-in shared memory per block (B200:
- * H <= 1404).  All pointers 4-byte aligned, no output may alias an input; T, B, H >= 1.  The grid-wide barrier between steps
- * relies on a cooperative launch, so the whole grid is resident by construction.
+ * accurate expf / tanhf.  Each CTA keeps the 4 gate rows of U = ceil(H / SMs) hidden units on chip: in shared memory
+ * while they fit next to one hidden row (B200: H <= 1404), above that as many units as fit in the SM's tensor memory
+ * (4 * floor(512 / (4 * ceil(H / 32))) per CTA) and the rest in shared memory.  H is refused (TQ_ERR_UNSUPPORTED) when
+ * the rows TMEM does not hold and one hidden row exceed the device's opt-in shared memory per block (B200: H <= 2048).
+ * Results do not depend on where a row lives.  All pointers 4-byte aligned, no output may alias an input;
+ * T, B, H >= 1.  The grid-wide barrier between steps relies on a cooperative launch, so the whole grid is resident by
+ * construction.
  */
 int tq_lstm_recurrence(const float *gin, const float *bias, const float *w_hh, const float *h0, const float *c0,
                        float *y, float *hn, float *cn, int T, int B, int H, void *stream);
@@ -406,8 +409,9 @@ int tq_lstm_recurrence(const float *gin, const float *bias, const float *w_hh, c
  *   RNN:  gin fp32 [T][B][H] = W_ih x_t;  bias fp32 [H] (b_ih + b_hh) or NULL;  w_hh fp32 [H][H]
  *       h_t = act(gin + bias + W_hh h),  act = relu ? ReLU (a NaN stays NaN, as torch.relu) : tanh
  *   h0 fp32 [B][H];  y fp32 [T][B][H] = h_t;  hn fp32 [B][H] = h_T
- * Each CTA keeps the G gate rows (G = 3 / 1) of ceil(H / SMs) units in shared memory, so the bound on H grows as G
- * shrinks (B200: GRU H <= 1628, RNN H <= 2812).  TQ_ERR_INVALID for NULL or misaligned pointers, T, B or H below 1 and
+ * Each CTA keeps the G gate rows (G = 3 / 1) of ceil(H / SMs) units in shared memory and tensor memory, so the bound
+ * on H grows as G shrinks (B200: GRU H <= 2304, RNN H <= 4096; shared memory alone up to GRU 1628, RNN 2812).
+ * TQ_ERR_INVALID for NULL or misaligned pointers, T, B or H below 1 and
  * B * G * H above 2^31 - 1; TQ_ERR_UNSUPPORTED (the message names the largest H) above the bound; all before any launch.
  */
 int tq_gru_recurrence(const float *gin, const float *b_hh, const float *w_hh, const float *h0, float *y, float *hn,

@@ -574,8 +574,10 @@ RECURRENCE_GATES = {"LSTM": 4, "GRU": 3, "RNN_TANH": 1, "RNN_RELU": 1}
 
 def recurrence_max_hidden(cell, device=None):
     """Largest hidden size the recurrence kernel of `cell` ('LSTM', 'GRU', 'RNN_TANH' or 'RNN_RELU') takes on `device`:
-    each CTA keeps the gate rows of ceil(H / SMs) units in shared memory next to one hidden row and 2 KB of gate
-    scratch.  The library computes it (tq_recurrence_max_hidden), the same number its refusals name."""
+    each CTA keeps the gate rows of ceil(H / SMs) units on chip, as many units as fit in the SM's tensor memory
+    (4 * floor(512 / (gates * ceil(H / 32))) once shared memory alone is not enough) and the rest in shared memory next
+    to one hidden row and 2 KB of gate scratch (B200: LSTM 2048, GRU 2304, RNN 4096).  The library computes it
+    (tq_recurrence_max_hidden), the same number its refusals name."""
     if cell not in RECURRENCE_GATES:
         raise ValueError(f"unknown recurrent cell {cell!r}: expected one of {', '.join(RECURRENCE_GATES)}")
     with torch.cuda.device(device if device is not None else torch.cuda.current_device()):

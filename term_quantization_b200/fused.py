@@ -621,7 +621,7 @@ class FusedLSTM(_FusedLanguageModel):
         hmax = conv_codes.lstm_max_hidden(m.weight_hh_l0.device)
         if m.hidden_size > hmax:
             raise NotImplementedError(f"FusedLSTM: hidden size {m.hidden_size} exceeds what the recurrence kernel keeps in "
-                                      f"shared memory on this device (H <= {hmax})")
+                                      f"shared and tensor memory on this device (H <= {hmax})")
         if rnn.input_quant.tracking or dec.input_quant.tracking:
             raise RuntimeError("calibrate the model (set_tr_tracking(model, False)) before fusing")
         if model.training:
@@ -706,7 +706,7 @@ class FusedRNN(_FusedLanguageModel):
         hmax = conv_codes.recurrence_max_hidden(kind, rnn.weight_hh_l0.device)
         if rnn.hidden_size > hmax:
             raise NotImplementedError(f"FusedRNN: hidden size {rnn.hidden_size} exceeds what the {kind} recurrence kernel "
-                                      f"keeps in shared memory on this device (H <= {hmax})")
+                                      f"keeps in shared and tensor memory on this device (H <= {hmax})")
         if dec.input_quant.tracking:
             raise RuntimeError("calibrate the model (set_tr_tracking(model, False)) before fusing")
         if model.training:

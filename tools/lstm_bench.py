@@ -21,7 +21,12 @@ the reference), one perplexity step as alternating CUDA-graph replays of
   tcgen05  cuDNN recurrence + the decoder on term codes + log_softmax + nll_loss(reduction='none')
   nll      FusedRNN.nll: the recurrence kernel per layer, the decoder's loss epilogue
 with the peak memory of each, and every layer's recurrence launch on its own (CUDA events) with its FFMA rate against
-the derived fp32 rate.  Writes DIR/rnn_bench.json."""
+the derived fp32 rate.  --model LSTM does the same for the LSTM (layer-0 input projection and decoder TR layers, as in
+the default workload; FusedLSTM.nll) with the eager per-phase split of the fused forward in place of the launches alone.
+Writes DIR/rnn_bench.json.
+
+--emsize / --nhid (default 650 / 650, tied) size the model of every mode, e.g. --emsize 1500 --nhid 1500 --model LSTM
+for the word-language-model example's large configuration, whose recurrence keeps part of W_hh in tensor memory."""
 import argparse
 import copy
 import gc
@@ -41,6 +46,7 @@ from term_quantization_b200 import conv_codes, evaluate_lstm, fused, tr_cuda, tr
 from term_quantization_b200.lstm_models.model import RNNModel  # noqa: E402
 
 T, B, H = 35, 80, 650
+EMSIZE = 650
 
 
 def gpu_info():
@@ -227,7 +233,7 @@ def rnn_bench(cell, dev, rounds, replays, derived, launches=20, samples=10):
     """One cell's perplexity step on both paths, and its recurrence launches alone."""
     torch.manual_seed(0)
     gen = torch.Generator(device=dev).manual_seed(0)
-    base = RNNModel(cell, evaluate_lstm.NTOKENS, 650, 650, 2, 0.5, True).to(dev).eval()
+    base = RNNModel(cell, evaluate_lstm.NTOKENS, EMSIZE, H, 2, 0.5, True).to(dev).eval()
     q = evaluate_lstm.convert_model(base, evaluate_lstm.static_lstm_layer_settings(base, 8, 8, 12), 8, 8)
     tokens = torch.randint(evaluate_lstm.NTOKENS, (T, B), device=dev, generator=gen)
     targets = torch.randint(evaluate_lstm.NTOKENS, (T * B,), device=dev, generator=gen)
@@ -237,7 +243,7 @@ def rnn_bench(cell, dev, rounds, replays, derived, launches=20, samples=10):
         tr_layer.set_tr_tracking(q, False)
         q_tc = copy.deepcopy(q)
         tr_layer.use_tensor_cores(q_tc)
-        f = fused.FusedRNN(copy.deepcopy(q))
+        f = (fused.FusedLSTM if cell == "LSTM" else fused.FusedRNN)(copy.deepcopy(q))
         paths = {"tcgen05": lambda: F.nll_loss(q_tc(tokens, hidden)[0], targets, reduction="none"),
                  "nll": lambda: f.nll(tokens, targets, hidden)[0]}
         graphs, outs = {}, {}
@@ -251,12 +257,20 @@ def rnn_bench(cell, dev, rounds, replays, derived, launches=20, samples=10):
         rel = float(((outs["nll"].double() - ref).abs() / ref.abs().clamp(min=1.0)).max())
         peaks = {k: peak_rise(fn) for k, fn in paths.items()}
 
-        # every layer's recurrence alone, on the input projection the executor computes for it
         G = conv_codes.RECURRENCE_GATES[cell]
         fma = T * B * G * H * H
-        y = f.model.encoder(tokens)
         recurrence = []
-        for l, (w_ih, b_gemm, w_hh, b_rec) in enumerate(f.layers):
+        if cell == "LSTM":                                    # its phases, the recurrence launches among them
+            per_phase = phases(f, tokens, hidden, reps=samples)
+            for p in per_phase:
+                if "recurrence" in p["phase"]:
+                    rate = fma / (p["ms_median"] * 1e-3)
+                    recurrence.append({"phase": p["phase"], "fma": fma, "ms_median": p["ms_median"], "fma_per_s": rate,
+                                       "fp32_tflops": 2 * rate / 1e12,
+                                       "share_of_derived_fp32_rate": rate / derived if derived else None})
+        # every layer's recurrence alone, on the input projection the executor computes for it
+        y = f.model.encoder(tokens)
+        for l, (w_ih, b_gemm, w_hh, b_rec) in enumerate(f.layers if cell != "LSTM" else []):
             x = y.view(T * B, -1)
             gin = (torch.mm(x, w_ih.t()) if b_gemm is None else torch.addmm(b_gemm, x, w_ih.t())).view(T, B, -1)
             h0 = hidden[l].contiguous()
@@ -273,10 +287,14 @@ def rnn_bench(cell, dev, rounds, replays, derived, launches=20, samples=10):
     steps = {k: {"ms_best": min(v), "ms_median": statistics.median(v), "ms_spread": max(v) - min(v),
                  "tokens_per_s_median": T * B / statistics.median(v) * 1e3, "peak_memory_rise_bytes": peaks[k]}
              for k, v in samples_ms.items()}
-    return {"paths": steps, "nll_vs_tcgen05_speedup_median": steps["tcgen05"]["ms_median"] / steps["nll"]["ms_median"],
-            "loss_max_rel_diff_nll_vs_tcgen05": rel, "max_hidden": conv_codes.recurrence_max_hidden(cell, dev),
-            "recurrence_kernel": {"how": f"eager, CUDA events around {launches} back-to-back launches, {samples} samples",
-                                  "layers": recurrence}}
+    res = {"paths": steps, "nll_vs_tcgen05_speedup_median": steps["tcgen05"]["ms_median"] / steps["nll"]["ms_median"],
+           "loss_max_rel_diff_nll_vs_tcgen05": rel, "max_hidden": conv_codes.recurrence_max_hidden(cell, dev),
+           "recurrence_kernel": {"how": f"eager, CUDA events around {launches} back-to-back launches, {samples} samples"
+                                 if cell != "LSTM" else f"eager fused forward split by CUDA events, {samples} passes",
+                                 "layers": recurrence}}
+    if cell == "LSTM":
+        res["fused_phases_eager"] = per_phase
+    return res
 
 
 def main(argv=None):
@@ -285,9 +303,13 @@ def main(argv=None):
     ap.add_argument("--rounds", type=int, default=15, help="alternating rounds; each times every path once")
     ap.add_argument("--replays", type=int, default=20, help="graph replays per timed sample")
     ap.add_argument("--nll", action="store_true", help="time the three perplexity paths (lstm_nll_epilogue.json)")
-    ap.add_argument("--model", nargs="+", choices=["GRU", "RNN_TANH", "RNN_RELU"],
+    ap.add_argument("--model", nargs="+", choices=["LSTM", "GRU", "RNN_TANH", "RNN_RELU"],
                     help="time these cells' perplexity step instead (rnn_bench.json)")
+    ap.add_argument("--emsize", type=int, default=650, help="embedding size")
+    ap.add_argument("--nhid", type=int, default=650, help="hidden units per layer (tied decoder: equal to --emsize)")
     args = ap.parse_args(argv)
+    global H, EMSIZE
+    H, EMSIZE = args.nhid, args.emsize
     if not torch.cuda.is_available():
         raise SystemExit("lstm_bench needs a CUDA device: nothing is timed on the CPU")
     os.makedirs(args.out, exist_ok=True)
@@ -298,8 +320,9 @@ def main(argv=None):
     props = torch.cuda.get_device_properties(dev)
     if args.model:
         derived = derived_fp32_rate(info, props)
-        res = {"workload": "Wikitext-2-shaped RNNModel 650/650 tied, 2 layers, vocab 33,278, seq 35 x batch 80, only the "
-                           "decoder TQ (wb 8 / g 8 / alpha 12 / db 8), seed 0: one perplexity step",
+        res = {"workload": f"Wikitext-2-shaped RNNModel {EMSIZE}/{H} tied, 2 layers, vocab 33,278, seq {T} x batch {B}, "
+                           "only the decoder TQ (LSTM: also the layer-0 input projection; wb 8 / g 8 / alpha 12 / db 8), "
+                           "seed 0: one perplexity step",
                "gpu": info, "sms": props.multi_processor_count,
                "timed_as": f"CUDA-graph replays of the whole step, {args.replays} per sample, {args.rounds} rounds "
                            "alternating the two paths; TF32 off.  Peak memory: eager call, rise of max_memory_allocated "
@@ -315,7 +338,7 @@ def main(argv=None):
 
     torch.manual_seed(0)
     gen = torch.Generator(device=dev).manual_seed(0)
-    base = RNNModel('LSTM', evaluate_lstm.NTOKENS, 650, 650, 2, 0.5, True).to(dev).eval()
+    base = RNNModel('LSTM', evaluate_lstm.NTOKENS, EMSIZE, H, 2, 0.5, True).to(dev).eval()
     q = evaluate_lstm.convert_model(base, evaluate_lstm.static_lstm_layer_settings(base, 8, 8, 12), 8, 8)
     tokens = torch.randint(evaluate_lstm.NTOKENS, (T, B), device=dev, generator=gen)
     hidden = base.init_hidden(B)
@@ -327,7 +350,7 @@ def main(argv=None):
         f = fused.FusedLSTM(copy.deepcopy(q))
         if args.nll:
             targets = torch.randint(evaluate_lstm.NTOKENS, (T * B,), device=dev, generator=gen)
-            res = {"workload": "Wikitext-2-shaped LSTM 650/650 tied, 2 layers, vocab 33,278, seq 35 x batch 80, TQ wb 8 / "
+            res = {"workload": f"Wikitext-2-shaped LSTM {EMSIZE}/{H} tied, 2 layers, vocab 33,278, seq 35 x batch 80, TQ wb 8 / "
                                "g 8 / alpha 12 / db 8 (bench_extra.py configs[4]), seed 0: one perplexity step",
                    "gpu": info, "sms": props.multi_processor_count,
                    **nll_bench(f, tokens, hidden, targets, args.rounds, args.replays)}
@@ -364,7 +387,7 @@ def main(argv=None):
                            "fp32_tflops": 2 * rate / 1e12,
                            "share_of_derived_fp32_rate": rate / derived if derived else None})
     res = {
-        "workload": "Wikitext-2-shaped LSTM 650/650 tied, 2 layers, vocab 33,278, seq 35 x batch 80, TQ wb 8 / g 8 / "
+        "workload": f"Wikitext-2-shaped LSTM {EMSIZE}/{H} tied, 2 layers, vocab 33,278, seq 35 x batch 80, TQ wb 8 / g 8 / "
                     "alpha 12 / db 8 (bench_extra.py configs[4]), seed 0",
         "gpu": info, "sms": props.multi_processor_count, "shared_memory_per_block_optin": props.shared_memory_per_block_optin,
         "lstm_max_hidden": conv_codes.lstm_max_hidden(dev),
