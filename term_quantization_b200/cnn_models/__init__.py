@@ -12,6 +12,8 @@ from copy import deepcopy
 
 import torch.nn as nn
 from torchvision.models import alexnet, mobilenet_v2, resnet18, vgg16_bn  # noqa: F401
+# deeper ResNets beyond the reference's list: BasicBlock resnet34 and the Bottleneck networks (fused.FusedResNet runs all)
+from torchvision.models import resnet34, resnet50, resnet101, resnet152, wide_resnet50_2  # noqa: F401
 
 from .. import _lib
 from ..tr_layer import TRConv2dLayer
@@ -27,6 +29,11 @@ except ImportError:  # pragma: no cover
 
 def model_names():
     return ['alexnet', 'vgg16_bn', 'resnet18', 'efficientnet_b0', 'mobilenet_v2']
+
+
+def resnet_names():
+    """The ResNets exported here besides the reference's resnet18 (evaluate_cnn -a takes them too)."""
+    return ['resnet34', 'resnet50', 'resnet101', 'resnet152', 'wide_resnet50_2']
 
 
 def efficientnet_b0(pretrained=True):

@@ -43,7 +43,7 @@ def select_engine(qmodel, engine):
     """How the calibrated model runs the validation pass.
     'float'   -- the reference's path: TR kernels + cuDNN fp32 conv on dequantised tensors (tr_layer.py:124-126);
     'tcgen05' -- every supported wrapped conv on integer term codes with the tcgen05 kernel, module tree unchanged;
-    'fused'   -- the fused executor of the architecture (fused.FusedResNet for BasicBlock ResNets, fused.FusedVGG,
+    'fused'   -- the fused executor of the architecture (fused.FusedResNet for ResNets (BasicBlock or Bottleneck), fused.FusedVGG,
                  fused.FusedMobileNet): BN / residual / ReLU(6) / next encode in the conv epilogue, depthwise convs code
                  to code;
     'auto'    -- 'fused' where the topology allows it, else 'tcgen05'.
@@ -69,7 +69,7 @@ def main(argv=None):
     parser = argparse.ArgumentParser(description='TQ CNN evaluation')
     parser.add_argument('val_dir', nargs='?', default=None,
                         help='dataset root holding imagenet/val (evaluate_cnn.py:50); synthetic images when absent')
-    parser.add_argument('-a', '--arch', default='resnet18', choices=cnn_models.model_names())
+    parser.add_argument('-a', '--arch', default='resnet18', choices=cnn_models.model_names() + cnn_models.resnet_names())
     parser.add_argument('-j', '--workers', default=0, type=int)
     parser.add_argument('-b', '--batch-size', default=256, type=int)
     parser.add_argument('-p', '--print-freq', default=10, type=int)

@@ -1,4 +1,4 @@
-"""Fused execution of a TQ-converted ResNet (torchvision BasicBlock topology).
+"""Fused execution of a TQ-converted ResNet (torchvision BasicBlock or Bottleneck topology).
 
 The reference runs, per wrapped conv: TR encode -> cuDNN conv -> BatchNorm -> ReLU (-> add) as
 separate passes over fp32 activations (tr_layer.py:124-126 inside torchvision's BasicBlock).
@@ -81,7 +81,15 @@ class _Conv:
 
 
 class FusedResNet(nn.Module):
-    """Wraps a calibrated, TQ-converted torchvision ResNet built from BasicBlocks."""
+    """Wraps a calibrated, TQ-converted torchvision ResNet built from BasicBlocks (resnet18 / 34) or Bottlenecks
+    (resnet50 / 101 / 152, wide_resnet50_2 / 101_2: any base_width, groups 1, no dilation).
+
+    Per BasicBlock: conv1 (BN + ReLU, emits conv2's codes) and conv2 (BN + identity + ReLU, writes the fp32 block
+    output and the next block's codes).  Per Bottleneck (stride on the 3x3 conv, torchvision v1.5): conv1 1x1 and
+    conv2 3x3/s codes to codes with BN + ReLU, conv3 1x1 with BN + identity + ReLU writing the fp32 block output and
+    the next block's codes.  The downsample (1x1/s conv + BN) goes from codes to the fp32 identity.  A ResNeXt
+    (grouped conv2), a dilated stage or a downsample that is not a wrapped conv is refused with NotImplementedError
+    before anything is launched."""
 
     def __init__(self, model, stem="tcgen05", engine="auto"):
         """engine: how each conv's exact accumulator is obtained ('auto' | 'f16' | 'i8', conv_codes.plan_weight).
@@ -93,20 +101,33 @@ class FusedResNet(nn.Module):
         if stem not in ("tcgen05", "tcgen05_pool", "cudnn"):
             raise ValueError("stem must be 'tcgen05', 'tcgen05_pool' or 'cudnn'")
         self.stem_mode = stem
-        self.model = model.to(memory_format=torch.channels_last).eval()
-        self.blocks = []
+        # the whole topology is checked before any _Conv is built: packing and planning a weight launches kernels
+        plan = []                                     # per block: ([(conv, bn) of the body], (conv, bn) of the downsample | None)
         for stage in (model.layer1, model.layer2, model.layer3, model.layer4):
             for blk in stage:
-                if not (isinstance(blk.conv1, tr_layer.TRConv2dLayer) and isinstance(blk.conv2, tr_layer.TRConv2dLayer)
-                        and hasattr(blk, "bn2") and not hasattr(blk, "conv3")):
-                    raise NotImplementedError("FusedResNet expects TQ-converted BasicBlocks")
+                if hasattr(blk, "conv3") and hasattr(blk, "bn3"):
+                    body = [(blk.conv1, blk.bn1), (blk.conv2, blk.bn2), (blk.conv3, blk.bn3)]
+                elif hasattr(blk, "conv2") and hasattr(blk, "bn2"):
+                    body = [(blk.conv1, blk.bn1), (blk.conv2, blk.bn2)]
+                else:
+                    raise NotImplementedError("FusedResNet expects TQ-converted BasicBlocks or Bottlenecks")
+                if not all(isinstance(c, tr_layer.TRConv2dLayer) for c, _ in body):
+                    raise NotImplementedError("FusedResNet expects TQ-converted BasicBlocks or Bottlenecks")
                 down = None
                 if blk.downsample is not None:
                     if not isinstance(blk.downsample[0], tr_layer.TRConv2dLayer):
                         raise NotImplementedError("downsample conv must be a TRConv2dLayer")
-                    down = _Conv(blk.downsample[0], blk.downsample[1], engine=engine)
-                # every conv input of a BasicBlock chain is the output of a ReLU (block input / conv1 output)
-                self.blocks.append((_Conv(blk.conv1, blk.bn1, engine=engine), _Conv(blk.conv2, blk.bn2, engine=engine), down))
+                    down = (blk.downsample[0], blk.downsample[1])
+                for c, _ in body + ([down] if down else []):
+                    why = c.tensor_core_blocker()     # ResNeXt: 'grouped/depthwise conv'; dilated stages: 'dilated conv'
+                    if why is not None:
+                        raise NotImplementedError(f"fused path: {why}")
+                plan.append((body, down))
+        self.model = model.to(memory_format=torch.channels_last).eval()
+        # every conv input of a BasicBlock or Bottleneck chain is the output of a ReLU (block input / the body convs'
+        # outputs), so every _Conv takes the one-sided (post_relu) bound
+        self.blocks = [tuple(_Conv(c, bn, engine=engine) for c, bn in body)
+                       + ((_Conv(*down, engine=engine) if down else None),) for body, down in plan]
         mp = model.maxpool
         self.fuse_stem = (isinstance(mp, nn.MaxPool2d) and mp.kernel_size in (3, (3, 3)) and mp.stride in (2, (2, 2))
                           and mp.padding in (1, (1, 1)) and mp.dilation in (1, (1, 1)) and not mp.ceil_mode
@@ -130,8 +151,10 @@ class FusedResNet(nn.Module):
                                 encoding=quant[3] if len(quant) == 4 else "hese").view(x_nhwc.shape)
 
     def chain_description(self):
-        """The fused chain as plain data (integer weight codes, fp32 scale, BatchNorm affine, quantiser per conv):
-        what oracle/fused_emul.run_resnet_chain needs to reproduce the block outputs bit for bit on a CPU."""
+        """The fused chain as plain data (integer weight codes, fp32 scale, BatchNorm affine, quantiser per conv), one
+        (conv1, conv2, down) tuple per BasicBlock and one (conv1, conv2, conv3, down) tuple per Bottleneck (down: None
+        without a downsample): what a CPU emulation needs to reproduce the block outputs bit for bit
+        (oracle/fused_emul.run_resnet_chain for BasicBlocks)."""
         def d(c):
             if c is None:
                 return None
@@ -139,7 +162,7 @@ class FusedResNet(nn.Module):
                     "scale": c.scale, "bias": None if c.bias is None else c.bias.detach().float().cpu().numpy(),
                     "bn": None if c.bn is None else (c.bn[0].cpu().numpy(), c.bn[1].cpu().numpy()),
                     "quant": c.quant, "engine": c.plan.engine, "groups": c.plan.groups}
-        return [(d(c1), d(c2), d(down)) for c1, c2, down in self.blocks]
+        return [tuple(d(c) for c in blk) for blk in self.blocks]
 
     @torch.no_grad()
     def forward_u8(self, x_u8_nhwc, mean, std):
@@ -196,15 +219,18 @@ class FusedResNet(nn.Module):
             codes = {}
         if capture is not None:
             capture["stem"] = cur
-        for i, (c1, c2, down) in enumerate(self.blocks):
+        for i, (*body, down) in enumerate(self.blocks):
             def get(q):
                 if q not in codes:
                     codes[q] = self._encode(cur, q)
                 return codes[q]
             identity = cur if down is None else down(get(down.quant), want_f32=True)[0]
-            _, mid = c1(get(c1.quant), relu=True, want_f32=False, next_quant=c2.quant)
+            # conv1 (and a Bottleneck's conv2): codes to the next body conv's codes, BN + ReLU in the epilogue
+            mid = get(body[0].quant)
+            for c, c_next in zip(body[:-1], body[1:]):
+                _, mid = c(mid, relu=True, want_f32=False, next_quant=c_next.quant)
             nxt = self.blocks[i + 1][0].quant if i + 1 < len(self.blocks) else None
-            cur, out_codes = c2(mid, residual=identity, relu=True, want_f32=True, next_quant=nxt)
+            cur, out_codes = body[-1](mid, residual=identity, relu=True, want_f32=True, next_quant=nxt)
             codes = {nxt: out_codes} if nxt is not None else {}
         if capture is not None:
             capture["final"] = cur
